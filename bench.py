@@ -2,6 +2,7 @@
 """bench.py -- throughput of the batched KilobotsEnv.step hot path on B200.
 
     python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference] [--workload c2|c2p|c3|c5|c1]
+                    [--dump-outputs DIR]
 
 A "step" is one `KilobotsEnv.step` (10 physics sub-steps of 0.1 s, gym_kilobots/envs/kilobots_env.py:161-215)
 for EVERY environment of the batch.  Default workload (BASELINE.json configs[1]): 4096 envs x 15
@@ -13,6 +14,10 @@ One JSON line on stdout (rank 0).  `value` = kilobot-steps/s with all inputs res
 `e2e` = the same metric through KilobotsVecEnv.step with HOST numpy buffers (pinned staging,
 H2D + D2H inside the timed region).  `--impl reference` times the CPU oracle (oracle/, a Box2D
 restatement -- pybox2d itself is not installable here) on all host cores on a bounded sample.
+
+Scenes and actions are seeded, so the same arguments give the same inputs on every run.  `--dump-outputs DIR` writes
+what the last of the K timed steps returned (observations, reward, done, status) as DIR/<name>.npy, so that two
+builds can be compared output for output.
 """
 import argparse
 import json
@@ -158,8 +163,27 @@ def measured_peaks():
     return {"hbm_gbs": 6650.0}, "fallback (B200_PROFILING.md)"
 
 
-def time_oracle(workload, sample_envs, steps, warmup, threads):
-    """CPU oracle on the host cores: kilobot-steps/s on a bounded sample of the workload."""
+DUMP_MAX_BYTES = 64 * 10 ** 6
+
+
+def dump_outputs(out_dir, outputs):
+    """Write the outputs of one env-step as out_dir/<name>.npy (float32, or float64 where the step returns float64).
+    When they exceed DUMP_MAX_BYTES, the same fixed, seeded sample of envs is kept from every array."""
+    outputs = {k: v.astype(np.float64 if v.dtype == np.float64 else np.float32) for k, v in outputs.items()}
+    E = len(outputs["reward"])
+    per_env = sum(v.nbytes for v in outputs.values()) // E
+    keep = (DUMP_MAX_BYTES - 4096 * len(outputs)) // per_env   # 4 KB per file for the .npy header
+    if keep < E:
+        envs = np.sort(np.random.default_rng(0).choice(E, keep, replace=False))
+        outputs = {k: v[envs] for k, v in outputs.items()}
+    os.makedirs(out_dir, exist_ok=True)
+    for k, v in outputs.items():
+        np.save(os.path.join(out_dir, k + ".npy"), v)
+
+
+def time_oracle(workload, sample_envs, steps, warmup, threads, dump_dir=None):
+    """CPU oracle on the host cores: kilobot-steps/s on a bounded sample of the workload.  With dump_dir, the outputs
+    of the last timed step are written there (dump_outputs)."""
     from oracle import kbo
     kbo.build()
     sc = build_scenario(workload, sample_envs)
@@ -170,8 +194,10 @@ def time_oracle(workload, sample_envs, steps, warmup, threads):
         ob.step(acts[t])
     t0 = time.perf_counter()
     for t in range(warmup, warmup + steps):
-        ob.step(acts[t])
+        out = ob.step(acts[t])
     dt = time.perf_counter() - t0
+    if dump_dir is not None:
+        dump_outputs(dump_dir, out)
     N = sc.scenes[0].num_kilobots
     return sc.num_envs * steps * N / dt, dt / steps, N
 
@@ -184,7 +210,7 @@ def run_reference(args):
     threads = os.cpu_count() or 1
     E = envs_per_gpu(args.workload, world, args.envs)
     sample = min(E, args.ref_envs)
-    value, sec_per_step, N = time_oracle(args.workload, sample, args.steps, args.warmup, threads)
+    value, sec_per_step, N = time_oracle(args.workload, sample, args.steps, args.warmup, threads, args.dump_outputs)
     out = {
         "impl": "reference", "metric": METRIC, "value": value, "unit": UNIT, "n_gpus": args.gpus,
         "steps": args.steps, "warmup": args.warmup, "ms_per_step": sec_per_step * 1e3, "higher_is_better": True,
@@ -246,10 +272,11 @@ class Rig:
             self.dist.destroy_process_group()
 
 
-def measure(rig, workload, E, steps, warmup, cpu_envs, steady_steps=0, sampler=None):
+def measure(rig, workload, E, steps, warmup, cpu_envs, steady_steps=0, sampler=None, dump_dir=None):
     """One workload on this rank's GPU: device-resident leg (CUDA events per step, L2 flushed between steps), the
     end-to-end leg through KilobotsVecEnv.step with host buffers, optionally a steady-state leg with staggered
-    auto-resets, and (rank 0) the roofline / cpu_baseline objects.  Returns the result dict on rank 0, else None."""
+    auto-resets, and (rank 0) the roofline / cpu_baseline objects.  Returns the result dict on rank 0, else None.
+    With dump_dir, rank 0 writes what the last timed step of the device-resident leg returned (dump_outputs)."""
     torch = rig.torch
     from gym_kilobots_b200.envs import KilobotsVecEnv
     dev, world, rank = rig.dev, rig.world, rig.rank
@@ -272,10 +299,15 @@ def measure(rig, workload, E, steps, warmup, cpu_envs, steady_steps=0, sampler=N
     for i in range(steps):
         rig.flush.zero_()  # L2 flush between timed iterations (not inside the event pair)
         starts[i].record()
-        env.step_device(acts_d[warmup + i])
+        obs, rew, done, info = env.step_device(acts_d[warmup + i])
         ends[i].record()
     rig.barrier()
     wall = time.perf_counter() - wall0
+    if dump_dir is not None and rank == 0:
+        # the step's output tensors are re-used by every later step: copy them out before the next leg
+        dump_outputs(dump_dir, {"kilobots": obs["kilobots"].cpu().numpy(), "objects": obs["objects"].cpu().numpy(),
+                                "light": obs["light"].cpu().numpy(), "reward": rew.cpu().numpy(),
+                                "done": done.cpu().numpy(), "status": info["status"].cpu().numpy()})
     step_ms = np.array([s.elapsed_time(e) for s, e in zip(starts, ends)])
     my_elapsed = float(step_ms.sum()) * 1e-3
     cnt1 = b.counters().astype(np.float64).sum(0)
@@ -418,7 +450,7 @@ def run_ours(args):
     sampler.start()
     E = envs_per_gpu(args.workload, world, args.envs)
     head = measure(rig, args.workload, E, args.steps, args.warmup, args.cpu_envs, steady_steps=args.steady_steps,
-                   sampler=sampler)
+                   sampler=sampler, dump_dir=args.dump_outputs)
     clocks = sampler.stop()
     sweep = []
     if args.sweep:
@@ -455,7 +487,12 @@ def main():
                     help="env-steps of the steady-state leg with staggered auto-resets (0 = skip)")
     ap.add_argument("--sweep", default="c5,c3,c4",
                     help="extra workloads measured after the headline one and reported under 'sweep' ('' = none)")
+    ap.add_argument("--dump-outputs", metavar="DIR",
+                    help="write what the last timed step of the headline workload returned (rank 0's envs) as "
+                         "DIR/<name>.npy; a fixed sample of the envs if that exceeds 64 MB")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
     if args.impl == "reference":
         run_reference(args)
     else:
