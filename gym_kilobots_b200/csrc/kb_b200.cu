@@ -78,14 +78,23 @@ __global__ void __launch_bounds__(KB_BLOCK_OF(LPE), (LPE == 32 ? (512 / KB_BLOCK
   s.initScratch();
   const int A = a.actionMode == KB_ACTION_KILOBOTS ? 2 * a.L.N : a.L.A;
   const double* act = a.action ? a.action + (size_t)envIn * A : nullptr;
-  if (a.actionMode == KB_ACTION_KILOBOTS) s.setKilobotActions(act);
+  // the doubled warp barriers after setKilobotActions and senseControl are redundant but kept: without them the
+  // compiler schedules this kernel differently (measured in SASS)
+  if (a.actionMode == KB_ACTION_KILOBOTS) {
+    setKilobotActions(s, act, s.g.lane, LPE);
+    s.g.usync();
+  }
   s.g.usync();
   if (a.task.mode != KB_TASK_CONST && s.g.lane == 0 && env < a.numEnvs)  // task layer, include/kb_b200.h
-    s.taskBegin(a.task, a.taskState + (size_t)env * KB_TASK_WORDS);
+    taskBegin(s, a.task, a.taskState + (size_t)env * KB_TASK_WORDS);
   for (int step = 0; step < a.L.stepsPerAction; ++step) {
     __syncthreads();  // keeps the warps of a block in the same phase (see KB_T in kb_step.cuh)
-    if (a.actionMode == KB_ACTION_LIGHT && act && a.L.numLights > 0) s.lightStep(act);
-    s.senseControl();
+    if (a.actionMode == KB_ACTION_LIGHT && act && a.L.numLights > 0) {
+      if (s.g.lane == 0) lightStep(s, act);
+      s.g.usync();
+    }
+    senseControl(s, s.g.lane, LPE);
+    s.g.usync();
     s.g.usync();
     s.worldStep();
   }
@@ -134,28 +143,8 @@ __global__ void __launch_bounds__(KB_BLOCK_OF(LPE)) kb_reset_kernel(const __grid
     s.hdr(H_NC) = 0u;
     s.hdr(H_STATUS) = 0u;
     s.hdr(H_SCENE) = (uint32_t)scene;
-    if (a.taskState && env < a.numEnvs) {  // a new episode: return and length restart (task layer)
-      double* ts = a.taskState + (size_t)env * KB_TASK_WORDS;
-      ts[3 + KB_EP_RETURN] = 0.0;
-      ts[3 + KB_EP_LENGTH] = 0.0;
-      ts[3 + KB_EP_SUCCESS] = 0.0;
-    }
   }
-  // light.__init__ / MomentumLight(velocity=...) / GradientLight(angle=...)
-  if (a.lightInit)
-    for (int i = lane; i < L.L; i += LPE) s.lightState()[i] = a.lightInit[(size_t)envIn * L.L + i];
-  // controllers: PhototaxisKilobot.__init__ lib/kilobot.py:307-316 (threshold -inf, turn_left)
-  for (int k = lane; k < L.N; k += LPE) {
-    double* c = s.ctrl(k);
-    const int kind = __ldg(&s.bc[L.M + k].kind);
-    c[0] = c[1] = c[2] = c[3] = 0.0;
-    if (kind == KB_KILOBOT_PHOTOTAXIS) {
-      c[0] = __longlong_as_double(0xFFF0000000000000LL);  // -inf
-    } else if ((kind == KB_KILOBOT_VELOCITY || kind == KB_KILOBOT_ACCELERATION) && a.kbVel) {
-      c[0] = a.kbVel[((size_t)envIn * L.N + k) * 2 + 0];
-      c[1] = a.kbVel[((size_t)envIn * L.N + k) * 2 + 1];
-    }
-  }
+  resetEnvLayer(s, a, env, envIn, lane, LPE);
   // bodies: b2World::CreateBody + CreateFixture (lib/body.py:32-38)
   for (int b = lane; b < L.B; b += LPE) {
     const double* p = a.pose + ((size_t)envIn * L.B + b) * 3;

@@ -120,6 +120,7 @@ struct Swarm {
   // (sin, cos) of the body angle: the q half of the blob's xf4 rows (the static slot B holds (0, 1))
   __device__ __forceinline__ GF2 q2(int b) const { return GF2{reinterpret_cast<float2*>(blob + L.oXf + 4 * b + 2)}; }
   __device__ __forceinline__ float2 massOf(int b) const { return make_float2(__ldg(&bc[b].invMass), __ldg(&bc[b].invI)); }
+  __device__ __forceinline__ int bkind(int b) const { return __ldg(&bc[b].kind); }
   __device__ __forceinline__ SF4 dummy4() const { return SF4{sa + W.zDummy + 16u * (uint32_t)(tid & 31)}; }
   __device__ __forceinline__ SU32 hdr(int i) const { return SU32{sa + W.zHdr + 4u * (uint32_t)i}; }
   __device__ __forceinline__ SU32 moved(int w) const { return SU32{sa + W.zMoved + 4u * (uint32_t)w}; }
@@ -158,6 +159,11 @@ struct Swarm {
     t.q.s = q.x;
     t.q.c = q.y;
     return t;
+  }
+  // the position the task and the observations read: c (== xf.p), from shared memory
+  __device__ __forceinline__ float2 obsPos(int b) const {
+    const float4 p = pos4(b);
+    return make_float2(p.x, p.y);
   }
   __device__ __forceinline__ bool awake(int b) const { return (f2u(vel4(b).get(3)) & BF_AWAKE) != 0u; }
   __device__ __forceinline__ void wake(int b) const {
@@ -248,236 +254,6 @@ struct Swarm {
       c[KB_CNT_PAIR_TESTS] += nTests;
       c[KB_CNT_ISLANDS] += nIsl;
     }
-  }
-
-  // --------------------------------------------------------------------------- lights / controllers
-  // (same arithmetic as Sim::lightStep / lightValueGrad / senseControl in kb_step.cuh; lib/light.py:59-75,176-189,
-  //  237-253,300-316 and lib/kilobot.py:54-55,86-127,188-203,253-258,294-300,318-333)
-  __device__ __forceinline__ static double clipd(double a, double lo, double hi) {
-    double m = a > lo ? a : lo;
-    return m < hi ? m : hi;
-  }
-  __device__ __forceinline__ void lightStep(const double* action) {
-    if (tid == 0) {
-      const SF64Arr ls = lightState();
-      int so = 0, ao = 0;
-      for (int l = 0; l < L.numLights; ++l) {
-        const LCs lc = lightConst(l);
-        const int lt = lc.type();
-        const double dt = 1. / 10;
-        if (lt == KB_LIGHT_CIRCULAR) {
-          double a0 = clipd(action[ao], lc.alo(0), lc.ahi(0));
-          double a1 = clipd(action[ao + 1], lc.alo(1), lc.ahi(1));
-          if (lc.relative()) {
-            ls[so] += a0 * dt;
-            ls[so + 1] += a1 * dt;
-          } else {
-            ls[so] = a0;
-            ls[so + 1] = a1;
-          }
-          ls[so] = clipd(ls[so], lc.blo(0), lc.bhi(0));
-          ls[so + 1] = clipd(ls[so + 1], lc.blo(1), lc.bhi(1));
-          so += 2;
-          ao += 2;
-        } else if (lt == KB_LIGHT_MOMENTUM) {
-          double a0 = clipd(action[ao], lc.alo(0), lc.ahi(0));
-          double a1 = clipd(action[ao + 1], lc.alo(1), lc.ahi(1));
-          ls[so + 2] += a0 * dt;
-          ls[so + 3] += a1 * dt;
-          const double v2 = ls[so + 2], v3 = ls[so + 3];
-          double n = sqrt(v2 * v2 + v3 * v3);
-          const double mv = lc.maxVel();
-          if (n > mv) {
-            double f = mv / n;
-            ls[so + 2] *= f;
-            ls[so + 3] *= f;
-          }
-          ls[so] += (double)ls[so + 2] * dt;
-          ls[so + 1] += (double)ls[so + 3] * dt;
-          ls[so] = clipd(ls[so], lc.blo(0), lc.bhi(0));
-          ls[so + 1] = clipd(ls[so + 1], lc.blo(1), lc.bhi(1));
-          so += 4;
-          ao += 2;
-        } else {
-          double a = clipd(action[ao], lc.alo(0), lc.ahi(0));
-          const double pi = 3.141592653589793;
-          if (a < -pi) a += 2 * pi;
-          if (a > pi) a -= 2 * pi;
-          ls[so] = a;
-          so += 1;
-          ao += 1;
-        }
-      }
-    }
-    __syncthreads();
-  }
-  __device__ __forceinline__ void lightValueGrad(const LCs lc, const SF64Arr ls, double sx, double sy, double* value,
-                                                 double* gx, double* gy) const {
-    if (lc.type() == KB_LIGHT_LINEAR) {
-      const double2 sc = kb_sincosd(ls[0]);
-      const double vx = sc.y, vy = sc.x;
-      *value = vx * sx + vy * sy;
-      *gx = vx;
-      *gy = vy;
-      return;
-    }
-    double g0 = -1 * (sx - (double)ls[0]);
-    double g1 = -1 * (sy - (double)ls[1]);
-    double norm = sqrt(g0 * g0 + g1 * g1);
-    double v = 1.0;
-    const double radius = lc.radius();
-    v -= norm / radius;
-    v = v < 1. ? v : 1.;
-    v = v > .0 ? v : .0;
-    v *= 255;
-    if (norm == 0.0) {
-      g0 = 0.0;
-      g1 = 0.0;
-    } else {
-      g0 /= norm;
-      g1 /= norm;
-    }
-    if (norm > radius) {
-      g0 *= .0;
-      g1 *= .0;
-    }
-    *value = v;
-    *gx = g0;
-    *gy = g1;
-  }
-  __device__ __forceinline__ void setLinearVelocity(int b, V2 v) const {
-    if (dot(v, v) > 0.0f) wake(b);
-    vel4(b).set(0, v.x);
-    vel4(b).set(1, v.y);
-  }
-  __device__ __forceinline__ void setAngularVelocity(int b, float w) const {
-    if (w * w > 0.0f) wake(b);
-    vel4(b).set(2, w);
-  }
-  __device__ __forceinline__ void setKilobotActions(const double* action) {
-    const double hpi = 0.5 * 3.141592653589793;
-    const double pi = 3.141592653589793;
-#pragma unroll 1
-    for (int k = tid; k < L.N; k += NT) {
-      const int kind = __ldg(&bc[k].kind);
-      double* c = ctrl(k);
-      const double* a = action ? action + 2 * k : nullptr;
-      if (kind == KB_KILOBOT_VELOCITY) {
-        c[0] = a ? clipd(a[0], .0, 0.01) : .0;
-        c[1] = a ? clipd(a[1], -hpi, hpi) : .0;
-      } else if (kind == KB_KILOBOT_ACCELERATION) {
-        c[2] = a ? clipd(a[0], -.005, .005) : .0;
-        c[3] = a ? clipd(a[1], -.2 * pi, .2 * pi) : .0;
-      }
-    }
-    __syncthreads();
-  }
-  __device__ __forceinline__ void senseControl() {
-    const SF64Arr ls = lightState();
-#pragma unroll 1
-    for (int k = tid; k < L.N; k += NT) {
-      const int b = k;   // M == 0
-      const int kind = __ldg(&bc[b].kind);
-      const Xf xf = bodyXf(b);
-      double* c = ctrl(k);
-      double value = 0.0, gx = 0.0, gy = 0.0;
-      double c2 = 0.0;
-      if (kind == KB_KILOBOT_PHOTOTAXIS) c2 = c[2];
-      const bool needLight = kind == KB_KILOBOT_SIMPLE_PHOTOTAXIS || (kind == KB_KILOBOT_PHOTOTAXIS && ((int)c2 % 6) == 0);
-      if (L.numLights > 0 && needLight) {
-        double sx, sy;
-        if (kind == KB_KILOBOT_SIMPLE_PHOTOTAXIS) {
-          sx = (double)xf.p.x / 25.0;
-          sy = (double)xf.p.y / 25.0;
-        } else {
-          V2 lp = mk((float)(25.0 * 0.0), (float)(25.0 * -0.0165));
-          V2 wp = xmul(xf, lp);
-          sx = (double)wp.x / 25.0;
-          sy = (double)wp.y / 25.0;
-        }
-        if (L.numLights == 1) {
-          lightValueGrad(lightConst(0), ls, sx, sy, &value, &gx, &gy);
-        } else {
-          double best = 0.0;
-          int so = 0;
-          for (int l = 0; l < L.numLights; ++l) {
-            double v, g0, g1;
-            lightValueGrad(lightConst(l), ls + so, sx, sy, &v, &g0, &g1);
-            value += v;
-            if (l == 0 || v > best) {
-              best = v;
-              gx = g0;
-              gy = g1;
-            }
-            const int lt = lightConst(l).type();
-            so += lt == KB_LIGHT_MOMENTUM ? 4 : (lt == KB_LIGHT_LINEAR ? 1 : 2);
-          }
-        }
-      }
-      switch (kind) {
-        case KB_KILOBOT_PHOTOTAXIS: {
-          int upd = (int)c2;
-          int turnRight = (int)c[1];
-          if (upd % 6) {
-            upd += 1;
-          } else {
-            upd += 1;
-            int noChange = (int)c[3];
-            if (value > c[0] || noChange >= 15) {
-              c[0] = value + .01;
-              turnRight = turnRight ? 0 : 1;
-              noChange = 0;
-            } else {
-              noChange += 1;
-            }
-            c[3] = (double)noChange;
-            c[1] = (double)turnRight;
-          }
-          c[2] = (double)upd;
-          const float tx = turnRight ? L.transRight[0] : L.transLeft[0];
-          const float ty = turnRight ? L.transRight[1] : L.transLeft[1];
-          const float w = turnRight ? L.omegaRight : L.omegaLeft;
-          V2 wv = rmul(xf.q, mk(tx, ty));
-          V2 lv = mk(wv.x / 25.0f, wv.y / 25.0f);
-          lv = mk(lv.x / L.dt, lv.y / L.dt);
-          lv = mk(lv.x * 25.0f, lv.y * 25.0f);
-          setAngularVelocity(b, w);
-          setLinearVelocity(b, lv);
-        } break;
-        case KB_KILOBOT_SIMPLE_PHOTOTAXIS: {
-          double mx = gx, my = gy;
-          double n = sqrt(mx * mx + my * my);
-          if (n > 0.01) {
-            mx = mx / n * 0.01;
-            my = my / n * 0.01;
-          }
-          mx *= 25.0;
-          my *= 25.0;
-          setLinearVelocity(b, mk((float)mx, (float)my));
-        } break;
-        case KB_KILOBOT_ACCELERATION: {
-          const double hpi = 0.5 * 3.141592653589793;
-          const double dt = 1. / 10;
-          c[0] += c[2] * dt;
-          c[1] += c[3] * dt;
-          c[0] = c[0] > .0 ? c[0] : .0;
-          c[1] = c[1] > -hpi ? c[1] : -hpi;
-          c[0] = c[0] < 0.01 ? c[0] : 0.01;
-          c[1] = c[1] < hpi ? c[1] : hpi;
-        }  // fallthrough
-        case KB_KILOBOT_VELOCITY: {
-          double ang = (double)pos4(b).get(2);
-          const double2 sc = kb_sincosd(ang);
-          double lx = sc.y, ly = sc.x;
-          lx *= c[0] * 25.0;
-          ly *= c[0] * 25.0;
-          setLinearVelocity(b, mk((float)lx, (float)ly));
-          setAngularVelocity(b, (float)c[1]);
-        } break;
-        default: break;
-      }
-    }
-    __syncthreads();
   }
 
   // --------------------------------------------------------------------------- collide
@@ -1941,19 +1717,6 @@ struct Swarm {
   }
 
   // ----------------------------------------------------------------------------- outputs
-  __device__ __forceinline__ void taskError(const TaskConst& tk, const double* tgt, double* dist, double* ang) const {
-    // only the swarm task applies (no objects in this tier); sequential float64 sum like the lane-group kernel
-    double sx = 0.0, sy = 0.0;
-    for (int b = 0; b < L.B; ++b) {
-      const float4 x = pos4(b);
-      sx += (double)x.x / 25.0;
-      sy += (double)x.y / 25.0;
-    }
-    const double px_ = sx / (double)L.N, py_ = sy / (double)L.N;
-    const double dx = px_ - tgt[0], dy = py_ - tgt[1];
-    *dist = sqrt(dx * dx + dy * dy);
-    *ang = 0.0;
-  }
   __device__ __forceinline__ void gather(const KernelArgs& a, int env) {
     __syncthreads();
     const int N = L.N;
@@ -1977,42 +1740,9 @@ struct Swarm {
     }
     const bool anyBad = __syncthreads_or(bad) != 0;
     if (anyBad && tid == 0) hdr(H_STATUS) |= KB_STATUS_NONFINITE;
-    if (a.obsLight || flat) {
-      const SF64Arr ls = lightState();
-      for (int i = tid; i < L.L; i += NT) {
-        const double v = ls[i];
-        if (a.obsLight) a.obsLight[(size_t)env * L.L + i] = v;
-        if (flat) flat[2 * N + i] = (float)v;
-      }
-    }
+    observeLights(*this, a, env, flat, tid, NT);
     __syncthreads();
-    if (tid == 0) {
-      float rew = __ldg(&a.scenes[a.envScene ? a.envScene[env] : 0].rewardConst);
-      uint8_t dn = 0;
-      if (a.task.mode != KB_TASK_CONST) {
-        double* ts = a.taskState + (size_t)env * KB_TASK_WORDS;
-        double d1, a1;
-        taskError(a.task, ts, &d1, &a1);
-        const double d0 = ts[3 + KB_EPISODE_STATS], a0 = ts[3 + KB_EPISODE_STATS + 1];
-        const bool success = d1 <= a.task.posTol && a1 <= a.task.angTol;
-        double r = a.task.wPos * (d0 - d1);
-        r = r + a.task.wAng * (a0 - a1);
-        r = r - a.task.stepPenalty;
-        if (success) r = r + a.task.bonus;
-        const double len = ts[3 + KB_EP_LENGTH] + 1.0;
-        dn = (success || (a.task.maxSteps > 0 && len >= (double)a.task.maxSteps)) ? 1 : 0;
-        ts[3 + KB_EP_RETURN] += r;
-        ts[3 + KB_EP_LENGTH] = len;
-        ts[3 + KB_EP_POSITION_ERROR] = d1;
-        ts[3 + KB_EP_ORIENTATION_ERROR] = a1;
-        ts[3 + KB_EP_SUCCESS] = success ? 1.0 : 0.0;
-        if (dn) ts[3 + KB_EP_DONE_COUNT] += 1.0;
-        rew = (float)r;
-      }
-      if (a.reward) a.reward[env] = rew;
-      if (a.done) a.done[env] = dn;
-      if (a.status) a.status[env] = (int32_t)hdr(H_STATUS);
-    }
+    if (tid == 0) taskEnd(*this, a, env);
   }
 };
 
@@ -2036,17 +1766,18 @@ __global__ void __launch_bounds__(NT, NT >= 512 ? 1 : (NT >= 256 ? 2 : 4)) kb_sw
   s.loadConsts(a.lights + (size_t)scene * (a.L.numLights > 0 ? a.L.numLights : 1));
   const int A = a.actionMode == KB_ACTION_KILOBOTS ? 2 * a.L.N : a.L.A;
   const double* act = a.action ? a.action + (size_t)env * A : nullptr;
-  if (a.actionMode == KB_ACTION_KILOBOTS) s.setKilobotActions(act);
-  if (a.task.mode != KB_TASK_CONST && s.tid == 0) {
-    double* ts = a.taskState + (size_t)env * KB_TASK_WORDS;
-    double d0, a0;
-    s.taskError(a.task, ts, &d0, &a0);
-    ts[3 + KB_EPISODE_STATS] = d0;
-    ts[3 + KB_EPISODE_STATS + 1] = a0;
+  if (a.actionMode == KB_ACTION_KILOBOTS) {
+    setKilobotActions(s, act, s.tid, NT);
+    __syncthreads();
   }
+  if (a.task.mode != KB_TASK_CONST && s.tid == 0) taskBegin(s, a.task, a.taskState + (size_t)env * KB_TASK_WORDS);
   for (int step = 0; step < a.L.stepsPerAction; ++step) {
-    if (a.actionMode == KB_ACTION_LIGHT && act && a.L.numLights > 0) s.lightStep(act);
-    s.senseControl();
+    if (a.actionMode == KB_ACTION_LIGHT && act && a.L.numLights > 0) {
+      if (s.tid == 0) lightStep(s, act);
+      __syncthreads();
+    }
+    senseControl(s, s.tid, NT);
+    __syncthreads();
     s.worldStep();
   }
   s.gather(a, env);
@@ -2082,27 +1813,8 @@ __global__ void __launch_bounds__(NT, NT >= 512 ? 1 : (NT >= 256 ? 2 : 4)) kb_sw
   for (int i = tid; i < 2 * KB_NUM_COUNTERS; i += NT) bw[L.oCnt + i] = 0u;
   for (int i = tid; i < H_WORDS; i += NT) s.hdr(i) = 0u;
   __syncthreads();
-  if (tid == 0) {
-    s.hdr(H_SCENE) = (uint32_t)scene;
-    if (a.taskState) {
-      double* ts = a.taskState + (size_t)env * KB_TASK_WORDS;
-      ts[3 + KB_EP_RETURN] = 0.0;
-      ts[3 + KB_EP_LENGTH] = 0.0;
-      ts[3 + KB_EP_SUCCESS] = 0.0;
-    }
-  }
-  for (int i = tid; i < L.L; i += NT) s.lightState()[i] = a.lightInit ? a.lightInit[(size_t)env * L.L + i] : 0.0;
-  for (int k = tid; k < L.N; k += NT) {
-    double* c = s.ctrl(k);
-    const int kind = __ldg(&s.bc[k].kind);
-    c[0] = c[1] = c[2] = c[3] = 0.0;
-    if (kind == KB_KILOBOT_PHOTOTAXIS) {
-      c[0] = __longlong_as_double(0xFFF0000000000000LL);  // -inf
-    } else if ((kind == KB_KILOBOT_VELOCITY || kind == KB_KILOBOT_ACCELERATION) && a.kbVel) {
-      c[0] = a.kbVel[((size_t)env * L.N + k) * 2 + 0];
-      c[1] = a.kbVel[((size_t)env * L.N + k) * 2 + 1];
-    }
-  }
+  if (tid == 0) s.hdr(H_SCENE) = (uint32_t)scene;
+  resetEnvLayer(s, a, env, env, tid, NT);
   for (int b = tid; b <= L.B; b += NT) {
     if (b < L.B) {
       const double* p = a.pose + ((size_t)env * L.B + b) * 3;

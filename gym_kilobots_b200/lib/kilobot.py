@@ -2,7 +2,7 @@
 gym_kilobots/lib/kilobot.py.  The controllers themselves (Kilobot.step :86-127, _loop :318-333,
 SimplePhototaxisKilobot.step :191-203, SimpleVelocityControlKilobot.step :253-258,
 SimpleAccelerationControlKilobot.step :294-300) run inside the CUDA step kernel
-(csrc/kb_step.cuh: senseControl); these classes record which controller a body uses and expose the
+(csrc/kb_env.cuh: senseControl); these classes record which controller a body uses and expose the
 controller state the env mirrors back from the device.
 """
 import numpy as np
