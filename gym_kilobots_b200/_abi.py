@@ -191,6 +191,7 @@ class KbLaunchConfig(C.Structure):
 
 
 PRODUCT_ONLY = {
+    "get_body_counts": (C.c_int, [_VP, _VP, _VP]),
     "get_state": (C.c_int, [_VP, _VP]),
     "set_state": (C.c_int, [_VP, _VP]),
     "get_launch_config": (C.c_int, [_VP, C.POINTER(KbLaunchConfig)]),

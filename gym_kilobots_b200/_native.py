@@ -193,6 +193,15 @@ class NativeBatch:
         _check(_fn["get_status"](self.h, _hptr(out)), "kb_get_status")
         return out
 
+    def body_counts(self):
+        """(objects [E], kilobots [E]) host int32: the counts of the scene each env was last reset with (before its
+        first reset: its scene at creation).  Object j < objects[e] is body j, kilobot k < kilobots[e] is body M + k;
+        the other body indices up to B are absent (include/kb_b200.h kb_create, padded body layout)."""
+        obj = np.zeros(self.E, np.int32)
+        kb = np.zeros(self.E, np.int32)
+        _check(_fn["get_body_counts"](self.h, _hptr(obj), _hptr(kb)), "kb_get_body_counts")
+        return obj, kb
+
     # ---- on-device scene sampling at reset (csrc/kb_sample.cuh)
     def set_sampler(self, spec):
         """spec: sampler.SceneSampler (or anything with to_abi() -> (KbSampleSpec, keep-alive))."""

@@ -65,7 +65,7 @@ __global__ void __launch_bounds__(KB_BLOCK_OF(LPE), (LPE == 32 ? (512 / KB_BLOCK
   s.g.init();
   s.bind(slot);
   s.blob = a.blobs + (size_t)env * a.L.blobWords;
-  const int scene = a.envScene ? a.envScene[envIn] : 0;
+  const int scene = a.envScene ? (int)reinterpret_cast<const uint32_t*>(s.blob)[a.L.oHdr + H_SCENE] : 0;   // (last reset's)
   s.px = a.proxies + (size_t)scene * a.L.Pp;
   s.bc = a.bodies + (size_t)scene * a.L.Bp;
   s.lights = a.lights + (size_t)scene * (a.L.numLights > 0 ? a.L.numLights : 1);
@@ -86,7 +86,7 @@ __global__ void __launch_bounds__(KB_BLOCK_OF(LPE), (LPE == 32 ? (512 / KB_BLOCK
   }
   s.g.usync();
   if (a.task.mode != KB_TASK_CONST && s.g.lane == 0 && env < a.numEnvs)  // task layer, include/kb_b200.h
-    taskBegin(s, a.task, a.taskState + (size_t)env * KB_TASK_WORDS);
+    taskBegin(s, a, env);
   for (int step = 0; step < a.L.stepsPerAction; ++step) {
     __syncthreads();  // keeps the warps of a block in the same phase (see KB_T in kb_step.cuh)
     if (a.actionMode == KB_ACTION_LIGHT && act && a.L.numLights > 0) {
@@ -145,8 +145,15 @@ __global__ void __launch_bounds__(KB_BLOCK_OF(LPE)) kb_reset_kernel(const __grid
     s.hdr(H_SCENE) = (uint32_t)scene;
   }
   resetEnvLayer(s, a, env, envIn, lane, LPE);
-  // bodies: b2World::CreateBody + CreateFixture (lib/body.py:32-38)
+  // bodies: b2World::CreateBody + CreateFixture (lib/body.py:32-38); an absent body (a padded index the scene does not
+  // populate) in the canonical state whatever the pose input holds: zero pose and velocity, asleep, identity transform
   for (int b = lane; b < L.B; b += LPE) {
+    if (__ldg(&s.bc[b].kind) == KB_BODY_ABSENT) {
+      s.pos4(b) = make_float4(0.0f, 0.0f, 0.0f, 0.0f);
+      s.vel4(b) = make_float4(0.0f, 0.0f, 0.0f, 0.0f);
+      s.xf4(b) = make_float4(0.0f, 0.0f, 0.0f, 1.0f);
+      continue;
+    }
     const double* p = a.pose + ((size_t)envIn * L.B + b) * 3;
     const float x = (float)(25.0 * p[0]);
     const float y = (float)(25.0 * p[1]);
@@ -202,7 +209,7 @@ __global__ void __launch_bounds__(KB_BLOCK_OF(LPE)) kb_setpose_kernel(const __gr
   s.g.init();
   s.bind(slot);
   s.blob = a.blobs + (size_t)env * L.blobWords;
-  const int scene = a.envScene ? a.envScene[envIn] : 0;
+  const int scene = a.envScene ? (int)reinterpret_cast<const uint32_t*>(s.blob)[L.oHdr + H_SCENE] : 0;
   s.px = a.proxies + (size_t)scene * L.Pp;
   s.bc = a.bodies + (size_t)scene * L.Bp;
   s.lights = a.lights + (size_t)scene * (a.L.numLights > 0 ? a.L.numLights : 1);
@@ -213,6 +220,7 @@ __global__ void __launch_bounds__(KB_BLOCK_OF(LPE)) kb_setpose_kernel(const __gr
   s.g.sync();
   for (int b = s.g.lane; b < L.B; b += LPE) {
     if (a.mask && !a.mask[(size_t)envIn * L.B + b]) continue;   // Body.set_pose touches this one body only
+    if (s.bkind(b) == KB_BODY_ABSENT) continue;
     const double* p = a.pose + ((size_t)envIn * L.B + b) * 3;
     const float x = (float)(p[0] * 25.0);
     const float y = (float)(p[1] * 25.0);
@@ -274,6 +282,7 @@ struct Handle {
   Layout L;
   std::vector<std::vector<BodyConst>> hostBodies;  // per scene
   std::vector<int> hostNumProxies;                  // per scene
+  std::vector<int> hostNumObjects, hostNumKilobots; // per scene (L.M / L.N are the maxima over the scenes)
   float* dBlobs = nullptr;
   int32_t* dEnvScene = nullptr;
   ProxyConst* dProxies = nullptr;
@@ -314,6 +323,16 @@ struct Handle {
 };
 
 static int launchGrid(const Handle* h) { return (h->numEnvs + h->envsPerBlock - 1) / h->envsPerBlock; }
+
+// The dynamic shared-memory limit is an attribute of the kernel, shared by every handle of the process: only ever raise
+// it, so that a batch created later with a smaller image (same kernel, fewer bodies) does not break an earlier one.
+template <class K>
+static cudaError_t raiseSmemLimit(K* kernel, size_t bytes) {
+  cudaFuncAttributes fa;
+  cudaError_t e = cudaFuncGetAttributes(&fa, kernel);
+  if (e != cudaSuccess || (size_t)fa.maxDynamicSharedSizeBytes >= bytes) return e;
+  return cudaFuncSetAttribute(kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)bytes);
+}
 
 static thread_local std::string g_err;
 static int fail(int code, const std::string& msg) {
@@ -479,9 +498,12 @@ static int lightStateDim(int type) { return type == KB_LIGHT_MOMENTUM ? 4 : (typ
 static int lightActionDim(int type) { return type == KB_LIGHT_LINEAR ? 1 : 2; }
 static int round4(int x) { return (x + 3) & ~3; }
 
-static int buildScene(const KbSceneDesc& sd, int Bp, int Pp, std::vector<ProxyConst>* proxies,
+// The scene's bodies in the batch's padded layout: object j at body index j, kilobot k at Mmax + k; the other indices
+// up to B = Bp - 1 are absent bodies (kind KB_BODY_ABSENT, no proxy, zero mass data).  Proxies are numbered as in a
+// compact world of the scene's own bodies: the table edges, then the fixtures of the present bodies in body order.
+static int buildScene(const KbSceneDesc& sd, int Mmax, int Bp, int Pp, std::vector<ProxyConst>* proxies,
                       std::vector<BodyConst>* bodies, SceneConst* sc) {
-  const int B = sd.num_bodies;
+  const int B = Bp - 1;   // the static table's slot
   proxies->assign(Pp, ProxyConst());
   bodies->assign(Bp, BodyConst());
   std::memset(proxies->data(), 0, sizeof(ProxyConst) * Pp);
@@ -509,8 +531,10 @@ static int buildScene(const KbSceneDesc& sd, int Bp, int Pp, std::vector<ProxyCo
       else if (loop) { pc.vx[3] = vx[1]; pc.vy[3] = vy[1]; pc.has3 = 1; }
     }
   }
-  for (int b = 0; b < B; ++b) {
-    const KbBodyDef& bd = sd.bodies[b];
+  for (int b = 0; b < B; ++b) (*bodies)[b].kind = KB_BODY_ABSENT;
+  for (int be = 0; be < sd.num_bodies; ++be) {
+    const KbBodyDef& bd = sd.bodies[be];
+    const int b = be < sd.num_objects ? be : Mmax + (be - sd.num_objects);
     BodyConst& bcst = (*bodies)[b];
     if (bd.num_fixtures < 1 || bd.num_fixtures > KB_MAX_FIXTURES) return fail(KB_ERR_INVALID, "body needs 1..3 fixtures");
     bcst.kind = bd.kind;
@@ -581,6 +605,8 @@ static int buildScene(const KbSceneDesc& sd, int Bp, int Pp, std::vector<ProxyCo
   }
   sc->wallEdges = sd.wall_edges;
   sc->rewardConst = sd.reward_const;
+  sc->numObjects = (int16_t)sd.num_objects;
+  sc->numKilobots = (int16_t)(sd.num_bodies - sd.num_objects);
   return KB_OK;
 }
 
@@ -624,8 +650,17 @@ int kb_create(const KbSceneDesc* scenes, int32_t num_scenes, const int32_t* env_
   CUDA_TRY(cudaSetDevice(device));
 
   const KbSceneDesc& s0 = scenes[0];
-  const int B = s0.num_bodies, M = s0.num_objects, N = B - M;
-  if (B < 1 || M < 0 || N < 0) return fail(KB_ERR_INVALID, "kb_create: bad body counts");
+  // padded body layout: M / N are the largest object / kilobot counts over the scenes, objects at 0..M-1, kilobots at
+  // M..M+N-1; a scene with fewer leaves absent bodies at the indices it does not populate
+  int M = 0, N = 0;
+  for (int s = 0; s < num_scenes; ++s) {
+    const KbSceneDesc& sd = scenes[s];
+    if (sd.num_bodies < 1 || sd.num_objects < 0 || sd.num_objects > sd.num_bodies || sd.num_bodies > 0xFFFF || !sd.bodies)
+      return fail(KB_ERR_INVALID, "kb_create: bad body counts");
+    M = std::max(M, (int)sd.num_objects);
+    N = std::max(N, (int)(sd.num_bodies - sd.num_objects));
+  }
+  const int B = M + N;
   // tier: the lane-group kernels (kb_step.cuh) hold up to 62 bodies; above that -- or on request (KB_FORCE_SWARM=1, used
   // by the tests to cross-check the two tiers on the same scenes) -- the CTA-per-env swarm tier (kb_swarm.cuh)
   bool swarm = B > KB_MAX_BODIES;
@@ -634,7 +669,7 @@ int kb_create(const KbSceneDesc* scenes, int32_t num_scenes, const int32_t* env_
     if (B > KB_SWARM_MAX_BODIES) return fail(KB_ERR_CAPACITY, "kb_create: more than 2040 bodies per env is not supported");
     if (M != 0) return fail(KB_ERR_CAPACITY, "kb_create: the large-swarm tier (> 62 bodies per env) supports kilobots only (no pushable objects)");
     for (int s = 0; s < num_scenes; ++s)
-      for (int b = 0; b < scenes[s].num_bodies && b < B; ++b) {
+      for (int b = 0; b < scenes[s].num_bodies; ++b) {
         const KbBodyDef& bd = scenes[s].bodies[b];
         if (bd.kind == KB_BODY_OBJECT || bd.num_fixtures != 1 || bd.fixtures[0].shape != KB_SHAPE_CIRCLE ||
             bd.fixtures[0].friction != 0.0f || bd.fixtures[0].restitution != 0.0f || !(bd.fixtures[0].density > 0.0f))
@@ -645,11 +680,11 @@ int kb_create(const KbSceneDesc* scenes, int32_t num_scenes, const int32_t* env_
   int P = 0;
   for (int s = 0; s < num_scenes; ++s) {
     const KbSceneDesc& sd = scenes[s];
-    if (sd.num_bodies != B || sd.num_objects != M || sd.num_lights != s0.num_lights ||
+    if (sd.num_lights != s0.num_lights ||
         sd.steps_per_action != s0.steps_per_action || sd.velocity_iterations != s0.velocity_iterations ||
         sd.position_iterations != s0.position_iterations || sd.dt != s0.dt || sd.damping_mode != s0.damping_mode ||
         sd.enable_toi != s0.enable_toi || sd.enable_sleep != s0.enable_sleep)
-      return fail(KB_ERR_INVALID, "kb_create: scenes must agree in body/light counts and simulation constants");
+      return fail(KB_ERR_INVALID, "kb_create: scenes must agree in light counts and simulation constants");
     {
       // light components may differ between scenes (a shuffled CompositeLight, different radii): the constants are
       // held per scene; the state / action vectors must have the same total length
@@ -661,11 +696,18 @@ int kb_create(const KbSceneDesc* scenes, int32_t num_scenes, const int32_t* env_
       if (sl != sl0 || al != al0) return fail(KB_ERR_INVALID, "kb_create: scenes must agree in light state / action dimensions");
     }
     int p = sd.wall_edges;
-    for (int b = 0; b < B; ++b) {
-      p += sd.bodies[b].num_fixtures;
-      if (sd.bodies[b].kind != s0.bodies[b].kind) return fail(KB_ERR_INVALID, "kb_create: scenes must agree in body kinds");
-    }
+    for (int b = 0; b < sd.num_bodies; ++b) p += sd.bodies[b].num_fixtures;
     P = std::max(P, p);
+    // body kinds agree at every padded index that two scenes both populate
+    for (int t = 0; t < s; ++t) {
+      const KbSceneDesc& st = scenes[t];
+      const int mo = std::min(sd.num_objects, st.num_objects);
+      const int nk = std::min(sd.num_bodies - sd.num_objects, st.num_bodies - st.num_objects);
+      bool same = true;
+      for (int b = 0; b < mo; ++b) same = same && sd.bodies[b].kind == st.bodies[b].kind;
+      for (int k = 0; k < nk; ++k) same = same && sd.bodies[sd.num_objects + k].kind == st.bodies[st.num_objects + k].kind;
+      if (!same) return fail(KB_ERR_INVALID, "kb_create: scenes must agree in body kinds");
+    }
   }
   if (!swarm && P > KB_MAX_PROXIES) return fail(KB_ERR_CAPACITY, "kb_create: more than 64 proxies per env is not supported");
 
@@ -805,13 +847,13 @@ int kb_create(const KbSceneDesc* scenes, int32_t num_scenes, const int32_t* env_
     int maxObjProxies = 0, maxWall = 0;
     for (int s = 0; s < num_scenes; ++s) {
       int op = 0;
-      for (int b = 0; b < M; ++b) op += scenes[s].bodies[b].num_fixtures;
+      for (int b = 0; b < scenes[s].num_objects; ++b) op += scenes[s].bodies[b].num_fixtures;
       maxObjProxies = std::max(maxObjProxies, op);
       maxWall = std::max(maxWall, (int)scenes[s].wall_edges);
     }
     bool allKilobotsFrictionless = true;
     for (int s = 0; s < num_scenes; ++s)
-      for (int b = M; b < B; ++b)
+      for (int b = scenes[s].num_objects; b < scenes[s].num_bodies; ++b)
         for (int f = 0; f < scenes[s].bodies[b].num_fixtures; ++f) {
           const KbFixtureDef& fd = scenes[s].bodies[b].fixtures[f];
           if (fd.friction != 0.0f || fd.restitution != 0.0f || fd.shape != KB_SHAPE_CIRCLE) allKilobotsFrictionless = false;
@@ -924,13 +966,15 @@ int kb_create(const KbSceneDesc* scenes, int32_t num_scenes, const int32_t* env_
   h->hostBodies.resize(num_scenes);
   for (int s = 0; s < num_scenes; ++s) {
     std::vector<ProxyConst> px;
-    int rc = buildScene(scenes[s], L.Bp, L.Pp, &px, &h->hostBodies[s], &allScenes[s]);
+    int rc = buildScene(scenes[s], L.M, L.Bp, L.Pp, &px, &h->hostBodies[s], &allScenes[s]);
     if (rc != KB_OK) {
       delete h;
       return rc;
     }
     allProxies.insert(allProxies.end(), px.begin(), px.end());
     h->hostNumProxies.push_back(allScenes[s].numProxies);
+    h->hostNumObjects.push_back(scenes[s].num_objects);
+    h->hostNumKilobots.push_back(scenes[s].num_bodies - scenes[s].num_objects);
     allBodies.insert(allBodies.end(), h->hostBodies[s].begin(), h->hostBodies[s].end());
   }
   const int NLp = std::max(1, (int)s0.num_lights);
@@ -968,6 +1012,9 @@ int kb_create(const KbSceneDesc* scenes, int32_t num_scenes, const int32_t* env_
   const size_t blobBytes = (size_t)launchGrid(h) * h->envsPerBlock * L.blobWords * 4;  // padded to whole blocks
   CUDA_TRY(cudaMalloc(&h->dBlobs, blobBytes));
   CUDA_TRY(cudaMemset(h->dBlobs, 0, blobBytes));
+  if (env_scene)   // H_SCENE before the first reset: the env's scene, so that kb_get_body_counts is right from the start
+    CUDA_TRY(cudaMemcpy2D(h->dBlobs + L.oHdr + H_SCENE, (size_t)L.blobWords * 4, env_scene, sizeof(int32_t), sizeof(int32_t),
+                          (size_t)num_envs, cudaMemcpyHostToDevice));
   const int Amax = std::max(std::max(L.A, 2 * N), 1);
   CUDA_TRY(cudaMalloc(&h->dAction, sizeof(double) * (size_t)num_envs * Amax));
   {
@@ -996,15 +1043,15 @@ int kb_create(const KbSceneDesc* scenes, int32_t num_scenes, const int32_t* env_
 #endif
 #define KB_SET_SMEM(LPE)                                                                                            \
   case LPE:                                                                                                          \
-    CUDA_TRY(cudaFuncSetAttribute(kb_step_kernel<LPE>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)h->smemBytes));   \
-    CUDA_TRY(cudaFuncSetAttribute(kb_reset_kernel<LPE>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)h->smemBytes));  \
-    CUDA_TRY(cudaFuncSetAttribute(kb_setpose_kernel<LPE>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)h->smemBytes)); \
+    CUDA_TRY(raiseSmemLimit(kb_step_kernel<LPE>, h->smemBytes));                                                     \
+    CUDA_TRY(raiseSmemLimit(kb_reset_kernel<LPE>, h->smemBytes));                                                    \
+    CUDA_TRY(raiseSmemLimit(kb_setpose_kernel<LPE>, h->smemBytes));                                                  \
     break;
   if (swarm) {
 #define KB_SET_SWARM_SMEM(T)                                                                                           \
-    CUDA_TRY(cudaFuncSetAttribute(kb_swarm_step_kernel<T>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)h->smemBytes));  \
-    CUDA_TRY(cudaFuncSetAttribute(kb_swarm_reset_kernel<T>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)h->smemBytes)); \
-    CUDA_TRY(cudaFuncSetAttribute(kb_swarm_setpose_kernel<T>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)h->smemBytes));
+    CUDA_TRY(raiseSmemLimit(kb_swarm_step_kernel<T>, h->smemBytes));                                                 \
+    CUDA_TRY(raiseSmemLimit(kb_swarm_reset_kernel<T>, h->smemBytes));                                                \
+    CUDA_TRY(raiseSmemLimit(kb_swarm_setpose_kernel<T>, h->smemBytes));
     if (L.lanesPerEnv == 128) { KB_SET_SWARM_SMEM(128) } else if (L.lanesPerEnv == 256) { KB_SET_SWARM_SMEM(256) } else { KB_SET_SWARM_SMEM(512) }
 #undef KB_SET_SWARM_SMEM
   } else switch (L.lanesPerEnv) {
@@ -1108,6 +1155,9 @@ int kb_set_sampler(KbHandle* hh, const KbSampleSpec* spec) {
   Handle* h = reinterpret_cast<Handle*>(hh);
   if (!h || !spec) return fail(KB_ERR_INVALID, "kb_set_sampler: null");
   const Layout& L = h->L;
+  for (int s = 0; s < h->numScenes; ++s)
+    if (h->hostNumObjects[s] != L.M || h->hostNumKilobots[s] != L.N)
+      return fail(KB_ERR_UNSUPPORTED, "kb_set_sampler: the scenes differ in their object / kilobot counts (on-device sampling draws one configuration)");
   if (spec->num_objects != L.M || spec->num_objects > KB_SAMPLE_MAX_OBJECTS)
     return fail(KB_ERR_INVALID, "kb_set_sampler: num_objects must equal the batch's (at most 16)");
   if (spec->num_lights != L.numLights) return fail(KB_ERR_INVALID, "kb_set_sampler: num_lights must equal the batch's");
@@ -1396,6 +1446,23 @@ int kb_get_status(KbHandle* hh, int32_t* out) {
   return KB_OK;
 }
 
+int kb_get_body_counts(KbHandle* hh, int32_t* objects, int32_t* kilobots) {
+  Handle* h = reinterpret_cast<Handle*>(hh);
+  if (!h) return fail(KB_ERR_INVALID, "kb_get_body_counts: null");
+  std::vector<int32_t> scene((size_t)h->numEnvs);
+  CUDA_TRY(cudaSetDevice(h->device));
+  CUDA_TRY(cudaDeviceSynchronize());
+  // header word H_SCENE of every blob: the scene each env was last reset with
+  CUDA_TRY(cudaMemcpy2D(scene.data(), sizeof(int32_t), h->dBlobs + h->L.oHdr + H_SCENE, (size_t)h->L.blobWords * 4,
+                        sizeof(int32_t), (size_t)h->numEnvs, cudaMemcpyDeviceToHost));
+  for (int e = 0; e < h->numEnvs; ++e) {
+    const int s = scene[e] >= 0 && scene[e] < h->numScenes ? scene[e] : 0;
+    if (objects) objects[e] = h->hostNumObjects[s];
+    if (kilobots) kilobots[e] = h->hostNumKilobots[s];
+  }
+  return KB_OK;
+}
+
 int kb_get_contacts(KbHandle* hh, int32_t* pairs, int32_t* count) {
   Handle* h = reinterpret_cast<Handle*>(hh);
   std::vector<uint32_t> buf;
@@ -1544,9 +1611,11 @@ int kb_set_task(KbHandle* hh, const KbTaskDef* task, const double* target) {
   if (!h || !task) return fail(KB_ERR_INVALID, "kb_set_task: null");
   if (task->mode != KB_TASK_CONST && task->mode != KB_TASK_OBJECT_TO_TARGET && task->mode != KB_TASK_SWARM_TO_TARGET)
     return fail(KB_ERR_INVALID, "kb_set_task: unknown mode");
-  if (task->mode == KB_TASK_OBJECT_TO_TARGET && (task->object < 0 || task->object >= h->L.M))
-    return fail(KB_ERR_INVALID, "kb_set_task: object index out of range");
-  if (task->mode == KB_TASK_SWARM_TO_TARGET && h->L.N < 1) return fail(KB_ERR_INVALID, "kb_set_task: no kilobots");
+  const int minM = *std::min_element(h->hostNumObjects.begin(), h->hostNumObjects.end());
+  const int minN = *std::min_element(h->hostNumKilobots.begin(), h->hostNumKilobots.end());
+  if (task->mode == KB_TASK_OBJECT_TO_TARGET && (task->object < 0 || task->object >= minM))
+    return fail(KB_ERR_INVALID, "kb_set_task: object index out of range (every scene of the batch must have the object)");
+  if (task->mode == KB_TASK_SWARM_TO_TARGET && minN < 1) return fail(KB_ERR_INVALID, "kb_set_task: a scene without kilobots");
   CUDA_TRY(cudaSetDevice(h->device));
   CUDA_TRY(cudaDeviceSynchronize());
   const size_t E = (size_t)h->numEnvs;

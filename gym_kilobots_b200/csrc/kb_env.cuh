@@ -121,7 +121,8 @@ __device__ __forceinline__ void setAngularVelocity(T& s, int b, float w) {
   s.vel4(b).set(2, w);
 }
 
-// Kilobot.set_action of every velocity / acceleration kilobot (action == null: zero action)
+// Kilobot.set_action of every velocity / acceleration kilobot (action == null: zero action).  An absent kilobot's kind
+// (KB_BODY_ABSENT) takes neither branch: its action row is never read and may hold anything.
 template <class T>
 __device__ __forceinline__ void setKilobotActions(T& s, const double* action, int first, int stride) {
   const double hpi = 0.5 * 3.141592653589793;
@@ -151,7 +152,8 @@ __device__ __forceinline__ void setKilobotActions(T& s, const double* action, in
   }
 }
 
-// every kilobot senses the light and runs its controller, which sets its velocity
+// every kilobot senses the light and runs its controller, which sets its velocity (an absent kilobot neither senses nor
+// runs a controller: KB_BODY_ABSENT needs no light and takes the default case)
 template <class T>
 __device__ __forceinline__ void senseControl(T& s, int first, int stride) {
   const Layout& L = s.L;
@@ -264,10 +266,17 @@ __device__ __forceinline__ void senseControl(T& s, int first, int stride) {
 }
 
 // ------------------------------------------------------------------------------------------------- task layer
-// distance (m) and |angle| (rad) between the task's subject and its target, float64, sequential sums -- the oracle
-// evaluates the same expressions in the same order (oracle/kbo_env.cpp TaskError)
+// The scene the env was last reset with (kb_set_env_scene takes effect at the next reset).
 template <class T>
-__device__ __forceinline__ void taskError(T& s, const TaskConst& tk, const double* tgt, double* dist, double* ang) {
+__device__ __forceinline__ int envSceneOf(T& s, const KernelArgs& a) {
+  return a.envScene ? (int)s.hdr(H_SCENE) : 0;
+}
+
+// distance (m) and |angle| (rad) between the task's subject and its target, float64, sequential sums -- the oracle
+// evaluates the same expressions in the same order (oracle/kbo_env.cpp TaskError).  n: the kilobots of the env's
+// scene (bodies L.M .. L.M + n - 1; in a batch of one size n == L.N).
+template <class T>
+__device__ __forceinline__ void taskError(T& s, const TaskConst& tk, const double* tgt, int n, double* dist, double* ang) {
   const Layout& L = s.L;
   double px, py, th = 0.0;
   if (tk.mode == KB_TASK_OBJECT_TO_TARGET) {
@@ -277,13 +286,13 @@ __device__ __forceinline__ void taskError(T& s, const TaskConst& tk, const doubl
     th = (double)s.pos4(tk.object).get(2);
   } else {
     double sx = 0.0, sy = 0.0;
-    for (int b = L.M; b < L.B; ++b) {
+    for (int b = L.M; b < L.M + n; ++b) {
       const float2 x = s.obsPos(b);
       sx += (double)x.x / 25.0;
       sy += (double)x.y / 25.0;
     }
-    px = sx / (double)L.N;
-    py = sy / (double)L.N;
+    px = sx / (double)n;
+    py = sy / (double)n;
   }
   const double dx = px - tgt[0], dy = py - tgt[1];
   *dist = sqrt(dx * dx + dy * dy);
@@ -292,9 +301,11 @@ __device__ __forceinline__ void taskError(T& s, const TaskConst& tk, const doubl
 
 // task error before the env-step, kept in the env's task words (not in registers) until taskEnd (single thread)
 template <class T>
-__device__ __forceinline__ void taskBegin(T& s, const TaskConst& tk, double* ts) {
+__device__ __forceinline__ void taskBegin(T& s, const KernelArgs& a, int env) {
+  double* ts = a.taskState + (size_t)env * KB_TASK_WORDS;
+  const int n = __ldg(&a.scenes[envSceneOf(s, a)].numKilobots);
   double d0, a0;
-  taskError(s, tk, ts, &d0, &a0);
+  taskError(s, a.task, ts, n, &d0, &a0);
   ts[3 + KB_EPISODE_STATS] = d0;
   ts[3 + KB_EPISODE_STATS + 1] = a0;
 }
@@ -317,12 +328,13 @@ __device__ __forceinline__ void observeLights(T& s, const KernelArgs& a, int env
 // the reward / done / info hooks (kilobots_env.py:123-131): reward, done, episode statistics, status (single thread)
 template <class T>
 __device__ __forceinline__ void taskEnd(T& s, const KernelArgs& a, int env) {
-  float rew = __ldg(&a.scenes[a.envScene ? a.envScene[env] : 0].rewardConst);
+  const SceneConst* sc = a.scenes + envSceneOf(s, a);
+  float rew = __ldg(&sc->rewardConst);
   uint8_t dn = 0;
   if (a.task.mode != KB_TASK_CONST) {
     double* ts = a.taskState + (size_t)env * KB_TASK_WORDS;
     double d1, a1;
-    taskError(s, a.task, ts, &d1, &a1);
+    taskError(s, a.task, ts, __ldg(&sc->numKilobots), &d1, &a1);
     const double d0 = ts[3 + KB_EPISODE_STATS], a0 = ts[3 + KB_EPISODE_STATS + 1];  // stashed by taskBegin
     const bool success = d1 <= a.task.posTol && a1 <= a.task.angTol;
     double r = a.task.wPos * (d0 - d1);

@@ -55,6 +55,7 @@ __device__ __forceinline__ Rgb shadePixel(const RenderArgs& a, const float4* xf,
   }
   // kilobots (:265-266): disc r + .002, grey ring of width .005 drawn inwards, white heading line of width .005
   for (int b = a.L.M; b < a.L.B; ++b) {
+    if (bc[b].kind == KB_BODY_ABSENT) continue;   // a padded index the env's scene does not populate
     const float4 t = xf[b];
     const float dx = x - t.x, dy = y - t.y;
     const float d2 = dx * dx + dy * dy;
@@ -103,7 +104,7 @@ __global__ void __launch_bounds__(256) kb_render_kernel(const RenderArgs a) {
   const float4* xfp = staged ? xf : reinterpret_cast<const float4*>(blob + a.L.oXf);
   const int px_ = blockIdx.x * blockDim.x + threadIdx.x, py = blockIdx.y * blockDim.y + threadIdx.y;
   if (px_ >= a.width || py >= a.height) return;
-  const int scene = a.envScene ? a.envScene[env] : 0;
+  const int scene = a.envScene ? (int)reinterpret_cast<const uint32_t*>(blob)[a.L.oHdr + H_SCENE] : 0;   // (last reset's)
   const float x = a.x0 + ((float)px_ + 0.5f) * ((a.x1 - a.x0) / (float)a.width);
   const float y = a.y1 - ((float)py + 0.5f) * ((a.y1 - a.y0) / (float)a.height);   // image row 0 = top
   const Rgb c = shadePixel(a, xfp, reinterpret_cast<const double*>(blob + a.L.oLight), a.proxies + (size_t)scene * a.L.Pp,

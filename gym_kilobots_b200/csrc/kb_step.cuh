@@ -1790,12 +1790,16 @@ struct Sim {
     float* flat = a.obsFlat ? a.obsFlat + (size_t)env * (2 * N + L.L + 4 * M) : nullptr;
 #pragma unroll 1
     for (int b = g.lane; b < L.B; b += LPE) {
-      const float4 x = xf4(b);
-      const float ang = pos4(b).get(2);
-      bad |= !(isfinite(x.x) && isfinite(x.y) && isfinite(ang));
+      float4 x = xf4(b);
+      float ang = pos4(b).get(2);
+      float ox = (float)((double)x.x / 25.0), oy = (float)((double)x.y / 25.0);
+      if (bkind(b) == KB_BODY_ABSENT) {   // an absent body's rows are quiet NaN: never read as a body at the origin
+        ox = oy = ang = x.z = x.w = __int_as_float(0x7FC00000);
+      } else {
+        bad |= !(isfinite(x.x) && isfinite(x.y) && isfinite(ang));
+      }
       float* o = b < M ? (a.obsObjects ? a.obsObjects + ((size_t)env * M + b) * 3 : nullptr)
                        : (a.obsKilobots ? a.obsKilobots + ((size_t)env * N + (b - M)) * 3 : nullptr);
-      const float ox = (float)((double)x.x / 25.0), oy = (float)((double)x.y / 25.0);
       if (o) {
         o[0] = ox;
         o[1] = oy;

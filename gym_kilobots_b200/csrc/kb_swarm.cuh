@@ -99,6 +99,7 @@ struct Swarm {
   const ProxyConst* px;
   const BodyConst* bc;
   int tid, S, nWall;
+  int nP;               // the scene's proxies: nWall + its kilobots (absent bodies own none); L.P is the batch's maximum
   uint32_t nSub, nCon, nPts, nLvl, nPit, nToi, nTests, nIsl;   // thread 0's copy is flushed
 #ifdef KB_PROFILE
   long long tp[KB_PROF_SLOTS], tlast;
@@ -1188,7 +1189,7 @@ struct Swarm {
 
   // b2BroadPhase::UpdatePairs + b2ContactManager::AddPair.  New pairs are appended in (min proxy, max proxy) order.
   __device__ __forceinline__ void findNewContacts() {
-    const int P = L.P;
+    const int P = nP;   // (the inert slots of a smaller scene are never binned: their centre lands in a real cell)
     bool any = false;
     for (int w = tid; w < W.movedWords; w += NT) any |= (uint32_t)moved(w) != 0u;
     if (__syncthreads_or(any) == 0) return;
@@ -1724,9 +1725,13 @@ struct Swarm {
     float* flat = a.obsFlat ? a.obsFlat + (size_t)env * (2 * N + L.L) : nullptr;
 #pragma unroll 1
     for (int b = tid; b < L.B; b += NT) {
-      const float4 p = pos4(b);
-      bad |= !(isfinite(p.x) && isfinite(p.y) && isfinite(p.z));
-      const float ox = (float)((double)p.x / 25.0), oy = (float)((double)p.y / 25.0);
+      float4 p = pos4(b);
+      float ox = (float)((double)p.x / 25.0), oy = (float)((double)p.y / 25.0);
+      if (b >= nP - nWall) {   // absent kilobot (kilobots only: body b owns proxy nWall + b): quiet NaN rows
+        ox = oy = p.z = __int_as_float(0x7FC00000);
+      } else {
+        bad |= !(isfinite(p.x) && isfinite(p.y) && isfinite(p.z));
+      }
       if (a.obsKilobots) {
         float* o = a.obsKilobots + ((size_t)env * N + b) * 3;
         o[0] = ox;
@@ -1747,21 +1752,26 @@ struct Swarm {
 };
 
 // ----------------------------------------------------------------------------------- kernels
+// the scene an env was last reset with (kb_set_env_scene takes effect at the next reset)
+__device__ __forceinline__ int swarmSceneOf(const KernelArgs& a, int env) {
+  return a.envScene ? (int)reinterpret_cast<const uint32_t*>(a.blobs + (size_t)env * a.L.blobWords)[a.L.oHdr + H_SCENE] : 0;
+}
+
 template <int NT>
-__device__ __forceinline__ void swarmBind(Swarm<NT>& s, const KernelArgs& a, int env, int sceneOverride = -1) {
+__device__ __forceinline__ void swarmBind(Swarm<NT>& s, const KernelArgs& a, int env, int scene) {
   s.blob = a.blobs + (size_t)env * a.L.blobWords;
-  const int scene = sceneOverride >= 0 ? sceneOverride : (a.envScene ? a.envScene[env] : 0);
   s.px = a.proxies + (size_t)scene * a.L.Pp;
   s.bc = a.bodies + (size_t)scene * a.L.Bp;
   s.nWall = __ldg(&a.scenes[scene].wallEdges);
+  s.nP = __ldg(&a.scenes[scene].numProxies);
 }
 
 template <int NT>
 __global__ void __launch_bounds__(NT, NT >= 512 ? 1 : (NT >= 256 ? 2 : 4)) kb_swarm_step_kernel(const __grid_constant__ KernelArgs a) {
   const int env = a.envOffset + blockIdx.x;
   Swarm<NT> s(a.L, a.W);
-  swarmBind(s, a, env);
-  const int scene = a.envScene ? a.envScene[env] : 0;
+  const int scene = swarmSceneOf(a, env);
+  swarmBind(s, a, env, scene);
   s.loadState();
   s.loadConsts(a.lights + (size_t)scene * (a.L.numLights > 0 ? a.L.numLights : 1));
   const int A = a.actionMode == KB_ACTION_KILOBOTS ? 2 * a.L.N : a.L.A;
@@ -1770,7 +1780,7 @@ __global__ void __launch_bounds__(NT, NT >= 512 ? 1 : (NT >= 256 ? 2 : 4)) kb_sw
     setKilobotActions(s, act, s.tid, NT);
     __syncthreads();
   }
-  if (a.task.mode != KB_TASK_CONST && s.tid == 0) taskBegin(s, a.task, a.taskState + (size_t)env * KB_TASK_WORDS);
+  if (a.task.mode != KB_TASK_CONST && s.tid == 0) taskBegin(s, a, env);
   for (int step = 0; step < a.L.stepsPerAction; ++step) {
     if (a.actionMode == KB_ACTION_LIGHT && act && a.L.numLights > 0) {
       if (s.tid == 0) lightStep(s, act);
@@ -1816,7 +1826,7 @@ __global__ void __launch_bounds__(NT, NT >= 512 ? 1 : (NT >= 256 ? 2 : 4)) kb_sw
   if (tid == 0) s.hdr(H_SCENE) = (uint32_t)scene;
   resetEnvLayer(s, a, env, env, tid, NT);
   for (int b = tid; b <= L.B; b += NT) {
-    if (b < L.B) {
+    if (b < s.nP - s.nWall) {
       const double* p = a.pose + ((size_t)env * L.B + b) * 3;
       const float x = (float)(25.0 * p[0]);
       const float y = (float)(25.0 * p[1]);
@@ -1827,9 +1837,12 @@ __global__ void __launch_bounds__(NT, NT >= 512 ? 1 : (NT >= 256 ? 2 : 4)) kb_sw
       s.q2(b) = make_float2(q.s, q.c);
       s.sweepp()[b] = make_float4(x, y, ang, 0.0f);
     } else {
+      // the static slot B, and any absent body (a padded index the scene does not populate) in the canonical state:
+      // zero pose and velocity, asleep, identity transform
       s.pos4(b) = make_float4(0.0f, 0.0f, 0.0f, 0.0f);
-      s.vel4(b) = make_float4(0.0f, 0.0f, 0.0f, u2f(BF_AWAKE));
+      s.vel4(b) = make_float4(0.0f, 0.0f, 0.0f, b == L.B ? u2f(BF_AWAKE) : 0.0f);
       s.q2(b) = make_float2(0.0f, 1.0f);
+      if (b < L.B) s.sweepp()[b] = make_float4(0.0f, 0.0f, 0.0f, 0.0f);
     }
   }
   s.loadConsts(a.lights + (size_t)scene * (L.numLights > 0 ? L.numLights : 1));
@@ -1844,7 +1857,7 @@ __global__ void __launch_bounds__(NT, NT >= 512 ? 1 : (NT >= 256 ? 2 : 4)) kb_sw
       const V2 p1 = xmul(id, v1), p2 = xmul(id, v2);
       f = make_float4(b2min(p1.x, p2.x) - KB_AABB_EXTENSION, b2min(p1.y, p2.y) - KB_AABB_EXTENSION,
                       b2max(p1.x, p2.x) + KB_AABB_EXTENSION, b2max(p1.y, p2.y) + KB_AABB_EXTENSION);
-    } else if (p < s.nWall + L.B) {
+    } else if (p < s.nP) {
       const Xf xf = s.bodyXf(p - s.nWall);
       const float r = __ldg(&s.px[p].radius);
       const V2 cc = xf.p + rmul(xf.q, mk(0.0f, 0.0f));   // b2CircleShape::ComputeAABB
@@ -1854,7 +1867,7 @@ __global__ void __launch_bounds__(NT, NT >= 512 ? 1 : (NT >= 256 ? 2 : 4)) kb_sw
       f = make_float4(3.0e38f, 3.0e38f, -3.0e38f, -3.0e38f);
     }
     s.fatp()[p] = f;
-    if (p < s.nWall + L.B) s.moved(p >> 5).atomOr(1u << (p & 31));
+    if (p < s.nP) s.moved(p >> 5).atomOr(1u << (p & 31));
   }
   __syncthreads();
   s.findNewContacts();   // b2World::Step: m_flags & e_newFixture -> FindNewContacts
@@ -1869,9 +1882,9 @@ __global__ void __launch_bounds__(NT, NT >= 512 ? 1 : (NT >= 256 ? 2 : 4)) kb_sw
   const int env = blockIdx.x;
   const Layout& L = a.L;
   Swarm<NT> s(a.L, a.W);
-  swarmBind(s, a, env);
+  swarmBind(s, a, env, swarmSceneOf(a, env));
   s.loadState();
-  for (int b = s.tid; b < L.B; b += NT) {
+  for (int b = s.tid; b < s.nP - s.nWall; b += NT) {   // (absent bodies are left alone)
     if (a.mask && !a.mask[(size_t)env * L.B + b]) continue;
     const double* p = a.pose + ((size_t)env * L.B + b) * 3;
     const float x = (float)(p[0] * 25.0);

@@ -4,6 +4,8 @@ The reference steps one environment per Python call (gym_kilobots/envs/kilobots_
 this class steps E of them with one kernel launch.  Semantics per environment are exactly those of
 `KilobotsEnv.step` / `reset`; the observation keeps the reference's dict layout
 ({'kilobots': [N,3], 'objects': [M,3], 'light': [L]}, kilobots_env.py:115-118) with a leading env axis.
+The envs of one batch may differ in their numbers of objects and kilobots: N and M are then the largest counts,
+`kilobot_mask` / `object_mask` say which rows an env populates, and the rows it does not are NaN.
 """
 import numpy as np
 
@@ -37,8 +39,51 @@ class KilobotsVecEnv:
         self._host = None
         self._sim_steps = 0
         self.obs_flat = self.batch.bind_flat_observation() if flat_observation else None
+        self._init_masks()
         if task is not None:
             self.set_task(task, targets)
+
+    def _init_masks(self):
+        """kilobot_mask [E,N] / object_mask [E,M]: bool CUDA tensors, True where the env's current scene has that
+        kilobot / object.  They follow every reset on the device: an env's counts change only when a reset rebuilds
+        it after `set_env_scene`."""
+        import torch
+        dev = self.batch.device
+        specs = self.scenario.scenes
+        self._scene_objects = torch.tensor([sp.num_objects for sp in specs], dtype=torch.int64, device=dev)
+        self._scene_kilobots = torch.tensor([sp.num_kilobots for sp in specs], dtype=torch.int64, device=dev)
+        es = self.scenario.env_scene
+        self._env_scene = torch.zeros(self.num_envs, dtype=torch.int64, device=dev) if es is None else \
+            torch.as_tensor(np.asarray(es, np.int64), device=dev)
+        self._scene_now = self._env_scene.clone()   # the scene each env was last reset with
+        self.mixed_counts = len({(sp.num_objects, sp.num_kilobots) for sp in specs}) > 1
+        self._update_masks()
+
+    def _update_masks(self):
+        import torch
+        dev = self.batch.device
+        self.kilobot_mask = torch.arange(self.num_kilobots, device=dev)[None, :] < self._scene_kilobots[self._scene_now][:, None]
+        self.object_mask = torch.arange(self.num_objects, device=dev)[None, :] < self._scene_objects[self._scene_now][:, None]
+
+    def _after_reset(self, mask):
+        if not self.mixed_counts:
+            return
+        import torch
+        if mask is None:
+            self._scene_now = self._env_scene.clone()
+        else:
+            m = torch.as_tensor(mask, device=self.batch.device).reshape(self.num_envs).bool()
+            self._scene_now = torch.where(m, self._env_scene, self._scene_now)
+        self._update_masks()
+
+    def set_env_scene(self, env_scene):
+        """Move envs to other scene templates of the batch (int [E]); an env changes at its next reset, which may change
+        its numbers of objects and kilobots (the masks follow at that reset)."""
+        import torch
+        es = np.asarray(env_scene, np.int32).reshape(self.num_envs)
+        self.batch.set_env_scene(es)
+        self.scenario.env_scene = es
+        self._env_scene = torch.as_tensor(es.astype(np.int64), device=self.batch.device)
 
     @classmethod
     def from_envs(cls, envs, device=0, **kwargs):
@@ -61,12 +106,13 @@ class KilobotsVecEnv:
         if getattr(self, "envs", None) is None:
             raise RuntimeError("resample() needs the source env objects: build the batch with KilobotsVecEnv.from_envs "
                                "(or use on-device sampling: KilobotsVecEnv.from_configuration)")
+        from .. import scenarios
         sc = self.scenario
         for i, env in enumerate(self.envs):
             if mask is not None and not mask[i]:
                 continue
             _, pose, light, _ = env._record_scene()
-            sc.body_pose[i] = pose
+            sc.body_pose[i] = scenarios.stack_poses(sc.scenes, [0 if sc.env_scene is None else sc.env_scene[i]], [pose])[0]
             if light is not None:
                 sc.light_state[i] = light
         return sc.body_pose, sc.light_state
@@ -101,6 +147,9 @@ class KilobotsVecEnv:
         (kb_reset_sampled, one launch, no host round trip).  sampler: a `sampler.SceneSampler`, or a Yaml configuration
         (then the batch's scenes must already be the sampler's: see `from_configuration`)."""
         from ..sampler import SceneSampler
+        if self.mixed_counts:
+            raise ValueError("on-device scene sampling draws one configuration: the batch's scenes differ in their "
+                             "numbers of objects / kilobots")
         if not isinstance(sampler, SceneSampler):
             sampler = SceneSampler(sampler, seed=seed, env_id_base=env_id_base)
         if (sampler.M, sampler.N, sampler.light_state_dim()) != (self.batch.M, self.batch.N, self.batch.L):
@@ -121,6 +170,7 @@ class KilobotsVecEnv:
         pose = self.scenario.body_pose if body_pose is None else body_pose
         light = self.scenario.light_state if light_state is None else light_state
         self.batch.reset(pose, light, None, done)
+        self._after_reset(done)
 
     # -- gym-like surface ---------------------------------------------------------------------
     @property
@@ -144,6 +194,7 @@ class KilobotsVecEnv:
         if kb_velocity is None:
             kb_velocity = getattr(self.scenario, "kb_velocity", None)
         self.batch.reset(pose, light, kb_velocity, mask)
+        self._after_reset(mask)
         self._sim_steps = 0
         return self.get_observation()
 
@@ -251,7 +302,12 @@ class KilobotsVecEnv:
         M = self.num_objects
         pose = np.stack([b[..., 8].astype(np.float64) / 25.0, b[..., 9].astype(np.float64) / 25.0,
                          b[..., 2].astype(np.float64)], axis=-1)
-        return {"kilobots": pose[:, M:], "objects": pose[:, :M], "light": light}
+        kb, obj = pose[:, M:], pose[:, :M]
+        if self.mixed_counts:   # rows of absent bodies are NaN, as in step()
+            n_obj, n_kb = self.batch.body_counts()
+            kb[np.arange(self.num_kilobots)[None, :] >= n_kb[:, None]] = np.nan
+            obj[np.arange(M)[None, :] >= n_obj[:, None]] = np.nan
+        return {"kilobots": kb, "objects": obj, "light": light}
 
     def get_observation(self):
         return self.get_state()

@@ -214,12 +214,31 @@ def swarm_corner(num_envs=8, n=48, seed=0, env_offset=0, kilobot_kind=abi.KB_KIL
     return Scenario("swarm-corner" if corner else "swarm-spread", [sc], None, pose, light, max_contacts=0)
 
 
+def stack_poses(specs, env_scene, poses):
+    """Stack per-env body poses into the padded body layout of a batch over `specs` (include/kb_b200.h kb_create).
+
+    poses[e] is [B_e, 3] for the scene specs[env_scene[e]]: its objects, then its kilobots.  The result is float64
+    [E, Mmax + Nmax, 3], Mmax / Nmax the largest object / kilobot counts of `specs`: object j of env e at row j, kilobot
+    k at row Mmax + k, zeros at the rows the env's scene does not populate (absent bodies).  A batch whose scenes all
+    have the same counts is stacked unchanged."""
+    Mmax = max(sp.num_objects for sp in specs)
+    Nmax = max(sp.num_kilobots for sp in specs)
+    out = np.zeros((len(poses), Mmax + Nmax, 3))
+    for e, (s, p) in enumerate(zip(env_scene, poses)):
+        sp = specs[int(s)]
+        p = np.asarray(p, dtype=np.float64).reshape(sp.num_bodies, 3)
+        out[e, :sp.num_objects] = p[:sp.num_objects]
+        out[e, Mmax:Mmax + sp.num_kilobots] = p[sp.num_objects:]
+    return out
+
+
 def from_envs(envs, name="from_envs"):
     """Vectorise reference-style environments: every element of `envs` is a KilobotsEnv subclass instance
     (YamlKilobotsEnv(configuration=...), QuadAssemblyKilobotsEnv(), a user's own subclass ...).  Each one's
     `_configure_environment` is run once, exactly as `reset()` would (kilobots_env.py:150-156), including its
     random initialisation; the recorded scenes are de-duplicated into templates and the poses stacked.
-    All envs must have the same number of objects / kilobots and the same light layout."""
+    All envs must have the same light layout; their numbers of objects and kilobots may differ (the poses and
+    kb_velocity are stacked in the padded body layout, see `stack_poses`)."""
     from .envs.kilobots_env import KilobotsEnv
     specs, keys, env_scene, poses, lights, vels = [], {}, [], [], [], []
     for env in envs:
@@ -232,13 +251,17 @@ def from_envs(envs, name="from_envs"):
         poses.append(pose)
         lights.append(np.zeros(0) if light is None else np.asarray(light, float))
         vels.append(vel)
-    B, M = specs[0].num_bodies, specs[0].num_objects
     for sp in specs:
-        if sp.num_bodies != B or sp.num_objects != M or sp.light_state_dim != specs[0].light_state_dim:
-            raise ValueError("from_envs: all environments must agree in body counts and light layout")
-    sc = Scenario(name, specs, np.asarray(env_scene, np.int32), np.stack(poses), np.stack(lights))
-    sc.kb_velocity = None if all(v is None for v in vels) else np.stack(
-        [np.zeros((B - M, 2)) if v is None else v for v in vels])
+        if sp.light_state_dim != specs[0].light_state_dim:
+            raise ValueError("from_envs: all environments must agree in their light layout")
+    sc = Scenario(name, specs, np.asarray(env_scene, np.int32), stack_poses(specs, env_scene, poses), np.stack(lights))
+    Nmax = max(sp.num_kilobots for sp in specs)
+    sc.kb_velocity = None
+    if any(v is not None for v in vels):
+        sc.kb_velocity = np.zeros((len(vels), Nmax, 2))
+        for e, v in enumerate(vels):
+            if v is not None:
+                sc.kb_velocity[e, :len(v)] = v
     return sc
 
 

@@ -117,7 +117,8 @@ typedef struct KbSceneDesc {
 
 typedef struct KbHandle KbHandle;
 
-/* derived sizes of a created batch */
+/* derived sizes of a created batch.  num_objects / num_kilobots are the largest counts over the scenes (Mmax, Nmax),
+   num_bodies = Mmax + Nmax: every array shaped by the counts uses these maxima (see kb_create, padded body layout) */
 typedef struct KbDims {
   int32_t num_envs, num_bodies, num_objects, num_kilobots;
   int32_t num_proxies;       /* max over scenes, wall edges included (they come first) */
@@ -150,8 +151,17 @@ typedef struct KbDims {
 
 /*
  * Create a batch of num_envs environments.  scenes[num_scenes] are the distinct scene templates,
- * env_scene[num_envs] (host, may be NULL = all scene 0) picks one per env.  All scenes must agree
- * in num_bodies, num_objects, lights and simulation constants; only fixtures may differ.
+ * env_scene[num_envs] (host, may be NULL = all scene 0) picks one per env.  All scenes must agree in their lights,
+ * light state / action dimensions and simulation constants; fixtures and the numbers of objects and kilobots may differ.
+ * Padded body layout: with Mmax / Nmax the largest object / kilobot counts over the scenes, an env whose scene has M_e
+ * objects and N_e kilobots keeps its objects at body indices 0..M_e-1 and its kilobots at Mmax..Mmax+N_e-1; the other
+ * indices below Bmax = Mmax + Nmax are ABSENT bodies.  Body kinds must agree at every padded index two scenes both
+ * populate.  Proxy ids are those of a compact world of the env's own bodies (table edges, then the fixtures of the
+ * present bodies in body order): an absent body owns no proxy, is never awake and never moves.  Every array shaped by
+ * the counts (poses, kb_velocity, observations, per-kilobot actions, the flat observation) uses the maxima; the pose
+ * and action rows of absent bodies are ignored (they may hold anything, NaN included), their observation rows are quiet
+ * NaN, kb_get_bodies reports them in the canonical state (all zero, xf.q.c = 1) and kb_get_mass_data as zeros.  More
+ * than 62 bodies (Bmax) select the large-swarm tier, whose scenes must all be kilobots only.
  * max_contacts > 0: capacity of the persistent contact list per env; 0: the throughput default (8B + 32 pairs,
  * 3B + 9 touching contacts per solve -- ample for separated swarms; overflow sets KB_STATUS_* bits); < 0: one
  * slot for every proxy pair, so that no pair is ever dropped (the E = 1 drop-in facade: the reference's clipped
@@ -167,7 +177,8 @@ const char* kb_last_error(void);
  * reset (kilobots_env.py:150-159): rebuild every env's bodies at the given poses with zero
  * velocity and fresh controllers, then run ONE world step without controllers (:157, :217-219).
  *   mask        device u8[E] or NULL (= all): which envs to reset
- *   body_pose   device f64[E,B,3]  (x m, y m, theta rad) -- Body.__init__ position/orientation
+ *   body_pose   device f64[E,B,3]  (x m, y m, theta rad) -- Body.__init__ position/orientation (padded layout:
+ *                                  rows of absent bodies are ignored)
  *   light_state device f64[E,L]    light position (+velocity / angle), may be NULL if no light
  *   kb_velocity device f64[E,N,2]  initial (v, omega) of velocity/acceleration-control kilobots
  *                                  (lib/kilobot.py:225-229); NULL = zeros
@@ -215,12 +226,14 @@ typedef struct KbSampleSpec {
   const int32_t* perm_scene;       /* [num_lights!] or NULL */
   double kilobot_mean[2], kilobot_std;
 } KbSampleSpec;
-int kb_set_sampler(KbHandle* h, const KbSampleSpec* spec);          /* also restarts the episode counts */
+/* also restarts the episode counts; KB_ERR_UNSUPPORTED for a batch whose scenes differ in their object / kilobot counts */
+int kb_set_sampler(KbHandle* h, const KbSampleSpec* spec);
 /* like kb_reset, with the poses / light states drawn on the device; mask: device u8[E] or NULL */
 int kb_reset_sampled(KbHandle* h, const uint8_t* mask, void* stream);
 /* what the last sampled resets drew: host f64[E,B,3], f64[E,L], i32[E] scene per env, u32[E] resets so far (any may be NULL) */
 int kb_get_sampled(KbHandle* h, double* body_pose, double* light_state, int32_t* env_scene, uint32_t* episodes);
-/* overwrite the env -> scene map (host i32[E]); takes effect at the env's next reset */
+/* overwrite the env -> scene map (host i32[E]); takes effect at the env's next reset (which may change the env's
+   object / kilobot counts: see kb_get_body_counts) */
 int kb_set_env_scene(KbHandle* h, const int32_t* env_scene);
 
 /*
@@ -228,8 +241,8 @@ int kb_set_env_scene(KbHandle* h, const int32_t* env_scene);
  *   light.step -> sensing -> controllers -> b2World.Step(dt, vel_iters, pos_iters)
  * then gathers the observation (get_state :115-118).  All pointers are device pointers.
  *   action        f64[E,A] (KB_ACTION_LIGHT) / f64[E,N,2] (KB_ACTION_KILOBOTS) / NULL
- *   obs_kilobots  f32[E,N,3]  (x m, y m, theta) = Body.get_pose (lib/body.py:63-65)
- *   obs_objects   f32[E,M,3]
+ *   obs_kilobots  f32[E,N,3]  (x m, y m, theta) = Body.get_pose (lib/body.py:63-65); absent kilobots: quiet NaN rows
+ *   obs_objects   f32[E,M,3]  absent objects: quiet NaN rows
  *   obs_light     f64[E,L]    light.get_state()
  *   reward f32[E], done u8[E], status i32[E]; any output pointer may be NULL.
  */
@@ -257,6 +270,9 @@ int kb_set_poses_masked(KbHandle* h, const double* body_pose, const uint8_t* bod
 /* per-env status word (KB_STATUS_* bits, sticky until the env is reset): host i32[E].  Also set by kb_reset's
    settle step, which kb_step's status output does not cover */
 int kb_get_status(KbHandle* h, int32_t* out);
+/* objects / kilobots of the scene each env was last reset with (before its first reset: its scene at kb_create):
+   host i32[E] each, either may be NULL.  Object j < objects[e] is body j, kilobot k < kilobots[e] is body Mmax + k. */
+int kb_get_body_counts(KbHandle* h, int32_t* objects, int32_t* kilobots);
 /* persistent contact list in Box2D world-list order (newest first):
    pairs i32[E,max_contacts,4] = (proxyA, proxyB, touching, pointCount), count i32[E] */
 int kb_get_contacts(KbHandle* h, int32_t* pairs, int32_t* count);
@@ -294,8 +310,8 @@ int kb_get_mass_data(KbHandle* h, float* out);
  * (yaml_kilobots_env.py:163-178: kilobots (x, y) * N, light state, objects (x, y, sin theta, cos theta) * M),
  * so that a training loop never leaves the device.  All task arithmetic is float64.
  *   error before / after the env-step:  d = |subject - target| (m), a = |wrap(theta - target_theta)| (rad)
- *   subject = pose of object `object` (KB_TASK_OBJECT_TO_TARGET) or the mean kilobot position
- *             (KB_TASK_SWARM_TO_TARGET, a = 0)
+ *   subject = pose of object `object` (KB_TASK_OBJECT_TO_TARGET; every scene must have it) or the mean position of
+ *             the env's own kilobots (KB_TASK_SWARM_TO_TARGET, a = 0)
  *   reward  = w_position * (d0 - d1) + w_orientation * (a0 - a1) - step_penalty + (success ? success_bonus : 0)
  *   success = d1 <= position_tolerance && a1 <= orientation_tolerance
  *   done    = success || (max_episode_steps > 0 && episode length >= max_episode_steps)
