@@ -128,6 +128,7 @@ class KbTaskDef(C.Structure):
 KB_SAMPLE_FIXED, KB_SAMPLE_RANDOM, KB_SAMPLE_AT_OBJECT = 0, 1, 2
 KB_SAMPLE_MEAN_LIGHT, KB_SAMPLE_MEAN_RANDOM = 1, 2
 KB_SAMPLE_MAX_OBJECTS = 16
+KB_SAMPLE_MAX_CONFIGS = 16
 
 
 class KbSampleObject(C.Structure):
@@ -198,6 +199,8 @@ PRODUCT_ONLY = {
     "get_host_layout": (C.c_int, [_VP, C.POINTER(C.c_int64), C.POINTER(C.c_int64)]),
     "reduce_episode_stats": (C.c_int, [_VP, _VP, _VP]),
     "set_sampler": (C.c_int, [_VP, C.POINTER(KbSampleSpec)]),
+    "set_sampler_mix": (C.c_int, [_VP, C.POINTER(KbSampleSpec), C.c_int32, _VP]),
+    "current_scenes": (C.c_int, [_VP, _VP, _VP]),
     "reset_sampled": (C.c_int, [_VP, _VP, _VP]),
     "get_sampled": (C.c_int, [_VP, _VP, _VP, _VP, _VP]),
     "selftest_exact_math": (C.c_int, [C.c_int32, C.c_int32, C.POINTER(C.c_uint64)]),

@@ -209,6 +209,19 @@ class NativeBatch:
         _check(_fn["set_sampler"](self.h, C.byref(s)), "kb_set_sampler")
         self._sampler_keep = keep
 
+    def set_sampler_mix(self, mix):
+        """mix: sampler.SamplerMix (or anything with to_abi() -> (KbSampleSpec[K], K, weights or None, keep-alive))."""
+        specs, k, weights, keep = mix.to_abi()
+        _check(_fn["set_sampler_mix"](self.h, specs, k, weights), "kb_set_sampler_mix")
+        self._sampler_keep = keep
+
+    def current_scenes(self, out=None):
+        """The scene each env was last reset with, as a DEVICE int32 [E] tensor (asynchronous, current stream)."""
+        if out is None:
+            out = self.torch.empty(self.E, dtype=self.torch.int32, device=self.device)
+        _check(_fn["current_scenes"](self.h, C.c_void_p(out.data_ptr()), self._stream()), "kb_current_scenes")
+        return out
+
     def reset_sampled(self, mask=None):
         """kb_reset with poses / light states drawn inside the reset kernel; mask: device or host uint8 [E] or None."""
         m = self._dev(mask, self.torch.uint8, (self.E,))

@@ -123,9 +123,7 @@ __global__ void __launch_bounds__(KB_BLOCK_OF(LPE)) kb_reset_kernel(const __grid
   if (a.sampler && env < a.numEnvs) {
     // a fresh scene for this env, drawn here: counter-based, keyed by (seed, global env id, episode)
     const uint32_t ep = a.episode[env];
-    scene = sampleScene(a.sampler, a.lights, L.numLights > 0 ? L.numLights : 1, L.B, L.M, scene,
-                        a.sampler->envIdBase + env, ep, s.g.lane, LPE, a.samplePose + (size_t)env * L.B * 3,
-                        a.sampleLight + (size_t)env * (L.L > 0 ? L.L : 1), [&]() { s.g.sync(); });
+    scene = sampleScene(a, env, scene, ep, s.g.lane, LPE, [&]() { s.g.sync(); });
     if (s.g.lane == 0) {
       a.episode[env] = ep + 1u;
       if (a.envSceneW) a.envSceneW[env] = scene;
@@ -246,6 +244,13 @@ __global__ void __launch_bounds__(KB_BLOCK_OF(LPE)) kb_setpose_kernel(const __gr
   s.storeState();
 }
 
+// kb_current_scenes: the header word H_SCENE of every env's blob (the scene it was last reset with)
+__global__ void kb_current_scenes_kernel(const float* __restrict__ blobs, int blobWords, int word, int numEnvs,
+                                         int32_t* __restrict__ out) {
+  const int e = blockIdx.x * blockDim.x + threadIdx.x;
+  if (e < numEnvs) out[e] = (int32_t)reinterpret_cast<const uint32_t*>(blobs)[(size_t)e * blobWords + word];
+}
+
 // Episode statistics of a rank, reduced on the device to KB_REDUCED_STATS doubles (the operand of the NCCL
 // all-reduce in KilobotsVecEnv.all_reduce_episode_stats).  One block, fixed summation tree: the result depends
 // on E only, never on scheduling.
@@ -311,9 +316,14 @@ struct Handle {
   // kb_step_host pipeline: chunks of the batch alternate between two side streams, so that the device->host copy of
   // one chunk overlaps the kernel of the next
   // on-device scene sampling at reset (kb_sample.cuh)
-  SamplerConst* dSampler = nullptr;
+  SamplerConst* dSampler = nullptr;             // [KB_SAMPLE_MAX_CONFIGS], numConfigs of them set
   double *dSamplePose = nullptr, *dSampleLight = nullptr;
   uint32_t* dEpisode = nullptr;
+  int numConfigs = 0;
+  std::vector<int> hostSceneConfig;              // configuration of each scene (-1 = none)
+  int32_t* dSceneConfig = nullptr;               // [numScenes]
+  double* dConfigCdf = nullptr;                  // [KB_SAMPLE_MAX_CONFIGS]
+  bool weighted = false;
   cudaStream_t pipe[2] = {nullptr, nullptr};
   cudaEvent_t evFork = nullptr, evJoin[2] = {nullptr, nullptr};
   int hostChunks = 1;
@@ -1089,6 +1099,7 @@ int kb_destroy(KbHandle* hh) {
   cudaFree(h->dBlobs); cudaFree(h->dEnvScene); cudaFree(h->dProxies); cudaFree(h->dBodies);
   cudaFree(h->dScenes); cudaFree(h->dLights); cudaFree(h->dAction); cudaFree(h->dOut); cudaFree(h->dTask); cudaFree(h->dRenderIds);
   cudaFree(h->dSampler); cudaFree(h->dSamplePose); cudaFree(h->dSampleLight); cudaFree(h->dEpisode);
+  cudaFree(h->dSceneConfig); cudaFree(h->dConfigCdf);
   for (int i = 0; i < 2; ++i) {
     if (h->pipe[i]) cudaStreamDestroy(h->pipe[i]);
     if (h->evJoin[i]) cudaEventDestroy(h->evJoin[i]);
@@ -1151,67 +1162,148 @@ int kb_reset(KbHandle* hh, const uint8_t* mask, const double* body_pose, const d
 }
 
 // ---- on-device scene sampling (include/kb_b200.h "Reset with on-device scene sampling") ------------------------
-int kb_set_sampler(KbHandle* hh, const KbSampleSpec* spec) {
-  Handle* h = reinterpret_cast<Handle*>(hh);
-  if (!h || !spec) return fail(KB_ERR_INVALID, "kb_set_sampler: null");
+}  // extern "C"
+
+namespace kb {
+// Validates K sampler specs against the batch and uploads them (kb_set_sampler is the case K = 1): the configurations,
+// the configuration of every scene and the normalised cumulative weights (weights == NULL: the env's scene decides).
+static int setSamplers(Handle* h, const KbSampleSpec* specs, int K, const double* weights, const char* who) {
   const Layout& L = h->L;
-  for (int s = 0; s < h->numScenes; ++s)
-    if (h->hostNumObjects[s] != L.M || h->hostNumKilobots[s] != L.N)
-      return fail(KB_ERR_UNSUPPORTED, "kb_set_sampler: the scenes differ in their object / kilobot counts (on-device sampling draws one configuration)");
-  if (spec->num_objects != L.M || spec->num_objects > KB_SAMPLE_MAX_OBJECTS)
-    return fail(KB_ERR_INVALID, "kb_set_sampler: num_objects must equal the batch's (at most 16)");
-  if (spec->num_lights != L.numLights) return fail(KB_ERR_INVALID, "kb_set_sampler: num_lights must equal the batch's");
-  if ((spec->num_objects > 0 && !spec->objects) || (spec->num_lights > 0 && !spec->lights))
-    return fail(KB_ERR_INVALID, "kb_set_sampler: missing object / light descriptions");
-  SamplerConst sc;
-  std::memset(&sc, 0, sizeof(sc));
-  sc.seedLo = (uint32_t)(spec->seed & 0xFFFFFFFFull);
-  sc.seedHi = (uint32_t)(spec->seed >> 32);
-  sc.envIdBase = spec->env_id_base;
-  sc.sizeX = spec->world_width;
-  sc.sizeY = spec->world_height;
-  sc.numObjects = spec->num_objects;
-  sc.numLights = spec->num_lights;
-  sc.meanMode = spec->kilobot_mean_mode;
-  sc.mean[0] = spec->kilobot_mean[0];
-  sc.mean[1] = spec->kilobot_mean[1];
-  sc.std = spec->kilobot_std;
-  for (int i = 0; i < spec->num_objects; ++i) {
-    sc.objMode[i] = spec->objects[i].mode;
-    for (int k = 0; k < 3; ++k) sc.objPose[i][k] = spec->objects[i].pose[k];
-    sc.objExtent[i] = spec->objects[i].extent;
-  }
-  for (int l = 0; l < spec->num_lights; ++l) {
-    sc.lightMode[l] = spec->lights[l].mode;
-    if (sc.lightMode[l] == KB_SAMPLE_AT_OBJECT && L.M == 0) return fail(KB_ERR_INVALID, "kb_set_sampler: light init 'object' without objects");
-    sc.lightInit[l][0] = spec->lights[l].init[0];
-    sc.lightInit[l][1] = spec->lights[l].init[1];
-  }
-  sc.shuffle = spec->shuffle_lights && spec->num_lights > 1;
-  if (sc.shuffle) {
-    if (!spec->perm_scene) return fail(KB_ERR_INVALID, "kb_set_sampler: shuffle_lights needs perm_scene");
+  auto bad = [&](const char* what) { return fail(KB_ERR_INVALID, std::string(who) + ": " + what); };
+  if (K < 1 || K > KB_SAMPLE_MAX_CONFIGS) return bad("num_specs must be 1..16");
+  std::vector<int> sceneConfig(h->numScenes, -1);
+  std::vector<SamplerConst> scs(K);
+  for (int c = 0; c < K; ++c) {
+    const KbSampleSpec* spec = specs + c;
+    if (spec->seed != specs[0].seed || spec->env_id_base != specs[0].env_id_base)
+      return bad("seed and env_id_base must be equal over the specs");
+    if (spec->num_objects < 0 || spec->num_objects > KB_SAMPLE_MAX_OBJECTS) return bad("num_objects must be at most 16");
+    if (spec->num_lights != L.numLights) return bad("num_lights must equal the batch's");
+    if ((spec->num_objects > 0 && !spec->objects) || (spec->num_lights > 0 && !spec->lights))
+      return bad("missing object / light descriptions");
+    const bool shuffle = spec->shuffle_lights && spec->num_lights > 1;
+    // the scenes of this configuration: one per permutation of a shuffled light, else its one scene; with K = 1 and no
+    // shuffle every scene of the batch (the env keeps its scene)
+    std::vector<int> mine;
     int nperm = 1;
-    for (int q = 2; q <= spec->num_lights; ++q) nperm *= q;
-    for (int r = 0; r < nperm; ++r) {
-      if (spec->perm_scene[r] < 0 || spec->perm_scene[r] >= h->numScenes) return fail(KB_ERR_INVALID, "kb_set_sampler: perm_scene out of range");
-      sc.permScene[r] = spec->perm_scene[r];
+    if (shuffle)
+      for (int q = 2; q <= spec->num_lights; ++q) nperm *= q;
+    if (shuffle || K > 1) {
+      if (!spec->perm_scene) return bad(shuffle ? "shuffle_lights needs perm_scene" : "perm_scene is required with more than one spec");
+      for (int r = 0; r < nperm; ++r) {
+        if (spec->perm_scene[r] < 0 || spec->perm_scene[r] >= h->numScenes) return bad("perm_scene out of range");
+        mine.push_back(spec->perm_scene[r]);
+      }
+    } else {
+      for (int sc = 0; sc < h->numScenes; ++sc) mine.push_back(sc);
+    }
+    for (int s : mine) {
+      if (h->hostNumObjects[s] != spec->num_objects) return bad("num_objects must equal the object count of each of the spec's scenes");
+      if (h->hostNumKilobots[s] != h->hostNumKilobots[mine[0]]) return bad("the scenes of a spec must have one kilobot count");
+      if (sceneConfig[s] >= 0 && sceneConfig[s] != c) return bad("a scene belongs to two specs");
+      sceneConfig[s] = c;
+    }
+    SamplerConst& sc = scs[c];
+    std::memset(&sc, 0, sizeof(sc));
+    sc.seedLo = (uint32_t)(spec->seed & 0xFFFFFFFFull);
+    sc.seedHi = (uint32_t)(spec->seed >> 32);
+    sc.envIdBase = spec->env_id_base;
+    sc.sizeX = spec->world_width;
+    sc.sizeY = spec->world_height;
+    sc.numObjects = spec->num_objects;
+    sc.numLights = spec->num_lights;
+    sc.meanMode = spec->kilobot_mean_mode;
+    sc.mean[0] = spec->kilobot_mean[0];
+    sc.mean[1] = spec->kilobot_mean[1];
+    sc.std = spec->kilobot_std;
+    for (int i = 0; i < spec->num_objects; ++i) {
+      sc.objMode[i] = spec->objects[i].mode;
+      for (int k = 0; k < 3; ++k) sc.objPose[i][k] = spec->objects[i].pose[k];
+      sc.objExtent[i] = spec->objects[i].extent;
+    }
+    for (int l = 0; l < spec->num_lights; ++l) {
+      sc.lightMode[l] = spec->lights[l].mode;
+      if (sc.lightMode[l] == KB_SAMPLE_AT_OBJECT && spec->num_objects == 0) return bad("light init 'object' without objects");
+      sc.lightInit[l][0] = spec->lights[l].init[0];
+      sc.lightInit[l][1] = spec->lights[l].init[1];
+    }
+    sc.shuffle = shuffle;
+    if (shuffle || K > 1)
+      for (int r = 0; r < nperm; ++r) sc.permScene[r] = spec->perm_scene[r];
+    sc.ownScene = !shuffle && K > 1;
+  }
+  std::vector<double> cdf(KB_SAMPLE_MAX_CONFIGS, 1.0);
+  if (weights) {
+    double total = 0.0;
+    for (int c = 0; c < K; ++c) {
+      if (!std::isfinite(weights[c]) || weights[c] < 0.0) return bad("weights must be finite and non-negative");
+      total += weights[c];
+    }
+    if (!(total > 0.0) || !std::isfinite(total)) return bad("weights must have a positive (finite) sum");
+    // from the last configuration of positive weight on, exactly 1.0: u < 1 always finds one, never a zero weight
+    int last = K - 1;
+    while (weights[last] == 0.0) --last;
+    double acc = 0.0;
+    for (int c = 0; c < K; ++c) {
+      acc += weights[c];
+      cdf[c] = c >= last ? 1.0 : acc / total;
     }
   }
   CUDA_TRY(cudaSetDevice(h->device));
   CUDA_TRY(cudaDeviceSynchronize());
   const size_t E = (size_t)h->numEnvs;
+  std::vector<int32_t> envScene(E, 0);
+  if (h->dEnvScene) CUDA_TRY(cudaMemcpy(envScene.data(), h->dEnvScene, sizeof(int32_t) * E, cudaMemcpyDeviceToHost));
+  if (K > 1)
+    for (size_t e = 0; e < E; ++e)
+      if (sceneConfig[envScene[e]] < 0) return bad("an env's scene belongs to no spec");
   if (!h->dSampler) {
-    CUDA_TRY(cudaMalloc(&h->dSampler, sizeof(SamplerConst)));
+    CUDA_TRY(cudaMalloc(&h->dSampler, sizeof(SamplerConst) * KB_SAMPLE_MAX_CONFIGS));
     CUDA_TRY(cudaMalloc(&h->dSamplePose, sizeof(double) * E * L.B * 3));
     CUDA_TRY(cudaMalloc(&h->dSampleLight, sizeof(double) * E * std::max(L.L, 1)));
     CUDA_TRY(cudaMalloc(&h->dEpisode, sizeof(uint32_t) * E));
+    CUDA_TRY(cudaMalloc(&h->dSceneConfig, sizeof(int32_t) * h->numScenes));
+    CUDA_TRY(cudaMalloc(&h->dConfigCdf, sizeof(double) * KB_SAMPLE_MAX_CONFIGS));
   }
   CUDA_TRY(cudaMemset(h->dEpisode, 0, sizeof(uint32_t) * E));
-  CUDA_TRY(cudaMemcpy(h->dSampler, &sc, sizeof(sc), cudaMemcpyHostToDevice));
+  CUDA_TRY(cudaMemcpy(h->dSampler, scs.data(), sizeof(SamplerConst) * K, cudaMemcpyHostToDevice));
+  CUDA_TRY(cudaMemcpy(h->dSceneConfig, sceneConfig.data(), sizeof(int32_t) * h->numScenes, cudaMemcpyHostToDevice));
+  CUDA_TRY(cudaMemcpy(h->dConfigCdf, cdf.data(), sizeof(double) * KB_SAMPLE_MAX_CONFIGS, cudaMemcpyHostToDevice));
   if (!h->dEnvScene) {   // the reset may switch scenes: the per-env scene map becomes device state
     CUDA_TRY(cudaMalloc(&h->dEnvScene, sizeof(int32_t) * E));
     CUDA_TRY(cudaMemset(h->dEnvScene, 0, sizeof(int32_t) * E));
   }
+  h->numConfigs = K;
+  h->weighted = weights != nullptr;
+  h->hostSceneConfig = sceneConfig;
+  return KB_OK;
+}
+}  // namespace kb
+
+extern "C" {
+
+int kb_set_sampler(KbHandle* hh, const KbSampleSpec* spec) {
+  Handle* h = reinterpret_cast<Handle*>(hh);
+  if (!h || !spec) return fail(KB_ERR_INVALID, "kb_set_sampler: null");
+  for (int s = 0; s < h->numScenes; ++s)
+    if (h->hostNumObjects[s] != h->L.M || h->hostNumKilobots[s] != h->L.N)
+      return fail(KB_ERR_UNSUPPORTED, "kb_set_sampler: the scenes differ in their object / kilobot counts (draw them with kb_set_sampler_mix)");
+  return setSamplers(h, spec, 1, nullptr, "kb_set_sampler");
+}
+
+int kb_set_sampler_mix(KbHandle* hh, const KbSampleSpec* specs, int32_t num_specs, const double* weights) {
+  Handle* h = reinterpret_cast<Handle*>(hh);
+  if (!h || !specs) return fail(KB_ERR_INVALID, "kb_set_sampler_mix: null");
+  return setSamplers(h, specs, num_specs, weights, "kb_set_sampler_mix");
+}
+
+int kb_current_scenes(KbHandle* hh, int32_t* out_device, void* stream) {
+  Handle* h = reinterpret_cast<Handle*>(hh);
+  if (!h || !out_device) return fail(KB_ERR_INVALID, "kb_current_scenes: null");
+  CUDA_TRY(cudaSetDevice(h->device));
+  kb_current_scenes_kernel<<<(h->numEnvs + 255) / 256, 256, 0, (cudaStream_t)stream>>>(h->dBlobs, h->L.blobWords,
+                                                                                      h->L.oHdr + H_SCENE, h->numEnvs, out_device);
+  CUDA_TRY(cudaGetLastError());
   return KB_OK;
 }
 
@@ -1232,6 +1324,9 @@ int kb_reset_sampled(KbHandle* hh, const uint8_t* mask, void* stream) {
   a.sampleLight = h->dSampleLight;
   a.envSceneW = h->dEnvScene;
   a.episode = h->dEpisode;
+  a.sceneConfig = h->dSceneConfig;
+  a.configCdf = h->weighted ? h->dConfigCdf : nullptr;
+  a.numConfigs = h->numConfigs;
   KB_LAUNCH(kb_reset_kernel, kb_swarm_reset_kernel, h, (cudaStream_t)stream, a);
   CUDA_TRY(cudaGetLastError());
   return KB_OK;
@@ -1255,6 +1350,8 @@ int kb_set_env_scene(KbHandle* hh, const int32_t* env_scene) {
   if (!h || !env_scene) return fail(KB_ERR_INVALID, "kb_set_env_scene: null");
   for (int i = 0; i < h->numEnvs; ++i)
     if (env_scene[i] < 0 || env_scene[i] >= h->numScenes) return fail(KB_ERR_INVALID, "kb_set_env_scene: scene out of range");
+    else if (h->numConfigs > 1 && h->hostSceneConfig[env_scene[i]] < 0)
+      return fail(KB_ERR_INVALID, "kb_set_env_scene: the scene belongs to no configuration of the sampler");
   CUDA_TRY(cudaSetDevice(h->device));
   CUDA_TRY(cudaDeviceSynchronize());
   if (!h->dEnvScene) CUDA_TRY(cudaMalloc(&h->dEnvScene, sizeof(int32_t) * (size_t)h->numEnvs));

@@ -15,6 +15,11 @@
 //   kilobots  mean = the light (one positional light), a uniformly chosen positional light per kilobot (several),
 //             U^2 * size + lo scaled by 0.9 (RANDOM), or FIXED; position = mean + std * N(0, 1)^2 clipped to the
 //             table -+ 0.02; orientation 0
+//
+// A batch may mix K configurations (kb_set_sampler_mix): one SamplerConst each.  The reset first picks the env's
+// configuration -- drawn from the cumulative weights (stream KS_CONFIG) or looked up from the env's scene -- and then
+// draws that configuration's scene as above, in the batch's padded body layout (objects at 0..M_e-1, kilobots at
+// Mmax + k; the rows of absent bodies are quiet NaN).
 #pragma once
 #include "kb_types.cuh"
 
@@ -27,6 +32,7 @@ namespace kb {
 #define KS_KILOBOT_POS 3
 #define KS_SWARM 5
 #define KS_SHUFFLE 6
+#define KS_CONFIG 8
 
 struct SamplerConst {
   uint32_t seedLo, seedHi;
@@ -40,6 +46,7 @@ struct SamplerConst {
   int32_t lightMode[KB_MAX_LIGHTS];                   // per CANONICAL component: 0 fixed, 1 random, 2 at object
   double lightInit[KB_MAX_LIGHTS][2];
   int32_t permScene[24];                              // scene index of every permutation (lexicographic rank)
+  int32_t ownScene;                                   // 1: the reset moves the env to permScene[0] (no shuffle, K > 1)
 };
 
 struct Philox4 {
@@ -81,18 +88,33 @@ struct EnvRng {
 };
 
 // Draws the scene of one env.  lane / nlanes: the threads that cooperate on this env; sync(): their barrier (global
-// writes of the group are visible to the group after it).  pose [B][3] and light [L] are this env's rows of the
-// handle's sample buffers; lightsAll = light constants of every scene ([scene][NLp]).  Returns the env's scene index.
-template <class SyncFn>
-__device__ __forceinline__ int sampleScene(const SamplerConst* __restrict__ sp, const LightConst* __restrict__ lightsAll,
-                                           int NLp, int B, int M, int sceneIn, long long envGlobal, uint32_t episode, int lane,
-                                           int nlanes, double* pose, double* light, SyncFn sync) {
+// writes of the group are visible to the group after it).  The draws go to the env's rows of the handle's sample
+// buffers (a.samplePose [B][3], a.sampleLight [L]).  KA is KernelArgs (kb_step.cuh): a.sampler[a.numConfigs] are the
+// configurations, a.configCdf their cumulative weights (null: a.sceneConfig[sceneIn] is the env's configuration).
+// Returns the env's scene index.
+template <class KA, class SyncFn>
+__device__ __forceinline__ int sampleScene(const KA& a, int env, int sceneIn, uint32_t episode, int lane, int nlanes,
+                                           SyncFn sync) {
+  const long long envGlobal = a.sampler->envIdBase + env;
+  const int B = a.L.B, Mmax = a.L.M;
+  double* pose = a.samplePose + (size_t)env * B * 3;
+  double* light = a.sampleLight + (size_t)env * (a.L.L > 0 ? a.L.L : 1);
   EnvRng g;
-  g.k0 = sp->seedLo;
-  g.k1 = sp->seedHi;
+  g.k0 = a.sampler->seedLo;   // seed and env id base agree over the configurations
+  g.k1 = a.sampler->seedHi;
   g.e0 = (uint32_t)((unsigned long long)envGlobal & 0xFFFFFFFFull);
   g.e1 = (uint32_t)((unsigned long long)envGlobal >> 32);
   g.ep = episode;
+  // ---- configuration (every lane computes the same one)
+  int cfg = 0;
+  if (a.configCdf) {
+    double u, u1;
+    g.uniform2(KS_CONFIG, 0u, &u, &u1);
+    while (cfg < a.numConfigs - 1 && !(u < a.configCdf[cfg])) ++cfg;
+  } else if (a.numConfigs > 1) {
+    cfg = max(__ldg(&a.sceneConfig[sceneIn]), 0);
+  }
+  const SamplerConst* __restrict__ sp = a.sampler + cfg;
   const double pi = 3.141592653589793;
   const double lox = -sp->sizeX / 2, loy = -sp->sizeY / 2;
   const int NL = sp->numLights;
@@ -137,7 +159,14 @@ __device__ __forceinline__ int sampleScene(const SamplerConst* __restrict__ sp, 
       rank += smaller * f;
     }
     scene = sp->permScene[rank];
+  } else if (sp->ownScene) {
+    scene = sp->permScene[0];
   }
+  // ---- this scene's counts; rows of absent bodies are NaN
+  const int M = __ldg(&a.scenes[scene].numObjects), N = __ldg(&a.scenes[scene].numKilobots);
+  const double qnan = __longlong_as_double(0x7FF8000000000000ll);
+  for (int i = lane; i < B; i += nlanes)
+    if ((i >= M && i < Mmax) || i >= Mmax + N) pose[3 * i] = pose[3 * i + 1] = pose[3 * i + 2] = qnan;
   // ---- objects
   for (int i = lane; i < M; i += nlanes) {
     double* p = pose + 3 * i;
@@ -156,7 +185,7 @@ __device__ __forceinline__ int sampleScene(const SamplerConst* __restrict__ sp, 
   }
   sync();
   // ---- lights (lane 0; positions of the positional lights are kept for the kilobots)
-  const LightConst* lc = lightsAll + (size_t)scene * NLp;
+  const LightConst* lc = a.lights + (size_t)scene * (a.L.numLights > 0 ? a.L.numLights : 1);
   if (lane == 0) {
     int off = 0;
     for (int pos = 0; pos < NL; ++pos) {
@@ -228,7 +257,6 @@ __device__ __forceinline__ int sampleScene(const SamplerConst* __restrict__ sp, 
     rmx = (u0 * sp->sizeX + lox) * 0.9;
     rmy = (u1 * sp->sizeY + loy) * 0.9;
   }
-  const int N = B - M;
   for (int k = lane; k < N; k += nlanes) {
     double mx, my;
     if (meanMode == 1) {
@@ -259,7 +287,7 @@ __device__ __forceinline__ int sampleScene(const SamplerConst* __restrict__ sp, 
     y = fmax(y, loy + 0.02);
     x = fmin(x, -lox - 0.02);
     y = fmin(y, -loy - 0.02);
-    double* p = pose + 3 * (M + k);
+    double* p = pose + 3 * (Mmax + k);
     p[0] = x;
     p[1] = y;
     p[2] = 0.0;

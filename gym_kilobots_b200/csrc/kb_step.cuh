@@ -68,6 +68,12 @@ struct KernelArgs {
   double* sampleLight;
   int32_t* envSceneW;
   uint32_t* episode;
+  // several configurations (kb_set_sampler_mix): sampler[numConfigs]; a sampled reset draws the configuration from
+  // configCdf [numConfigs] (cumulative weights, last entry 1) or, when that is null, takes sceneConfig[env's scene].
+  // Appended so that the offsets of the step kernels' parameters stay where they were.
+  const int32_t* sceneConfig;   // [S], -1 = no configuration
+  const double* configCdf;
+  int32_t numConfigs;
 };
 
 }  // namespace kb

@@ -1808,9 +1808,7 @@ __global__ void __launch_bounds__(NT, NT >= 512 ? 1 : (NT >= 256 ? 2 : 4)) kb_sw
   int scene = a.envScene ? a.envScene[env] : 0;
   if (a.sampler) {   // a fresh scene drawn on the device (kb_sample.cuh)
     const uint32_t ep = a.episode[env];
-    scene = sampleScene(a.sampler, a.lights, L.numLights > 0 ? L.numLights : 1, L.B, L.M, scene, a.sampler->envIdBase + env, ep,
-                        s.tid, NT, a.samplePose + (size_t)env * L.B * 3,
-                        a.sampleLight + (size_t)env * (L.L > 0 ? L.L : 1), []() { __syncthreads(); });
+    scene = sampleScene(a, env, scene, ep, s.tid, NT, []() { __syncthreads(); });
     if (s.tid == 0) {
       a.episode[env] = ep + 1u;
       if (a.envSceneW) a.envSceneW[env] = scene;

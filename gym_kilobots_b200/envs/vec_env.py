@@ -76,6 +76,20 @@ class KilobotsVecEnv:
             self._scene_now = torch.where(m, self._env_scene, self._scene_now)
         self._update_masks()
 
+    def _after_sampled_reset(self, mask):
+        """A sampled reset of a mixed batch may move envs to scenes of other sizes: read the scenes on the device (no
+        synchronisation) and let the masks follow; the reset envs' next scene is the one they were reset with."""
+        if not self.mixed_counts:
+            return
+        import torch
+        self._scene_now = self.batch.current_scenes().long()
+        if mask is None:
+            self._env_scene = self._scene_now.clone()
+        else:
+            m = torch.as_tensor(mask, device=self.batch.device).reshape(self.num_envs).bool()
+            self._env_scene = torch.where(m, self._scene_now, self._env_scene)
+        self._update_masks()
+
     def set_env_scene(self, env_scene):
         """Move envs to other scene templates of the batch (int [E]); an env changes at its next reset, which may change
         its numbers of objects and kilobots (the masks follow at that reset)."""
@@ -142,11 +156,51 @@ class KilobotsVecEnv:
         vec.use_device_sampler(sampler)
         return vec
 
+    @classmethod
+    def from_configurations(cls, configurations, num_envs, weights=None, env_config=None, seed=0, env_id_base=0, device=0,
+                            max_contacts=0, **kwargs):
+        """E envs over several Yaml configurations as ONE batch whose scenes are drawn on the device (`sampler.SamplerMix`):
+        a curriculum or domain randomisation over swarm size and object sets.  The configurations may differ in their
+        numbers of objects and kilobots (`kilobot_mask` / `object_mask` follow every reset on the device).  Give exactly
+        one of
+          weights     [K]: every sampled reset draws the env's configuration with these weights (keyed by seed / global
+                      env id / episode, like every other draw: 1 and 8 GPUs agree);
+          env_config  [E]: the configuration of every env; it keeps it at every reset until `set_env_scene` moves it
+                      (to `sampler.first_scene(c)` of another configuration c).
+        env_id_base: global id of this batch's env 0 (rank * num_envs)."""
+        from .. import scenarios
+        from ..sampler import SamplerMix
+        if (weights is None) == (env_config is None):
+            raise ValueError("give exactly one of weights / env_config")
+        mix = SamplerMix(configurations, weights=weights, seed=seed, env_id_base=env_id_base)
+        env_scene = None
+        if env_config is not None:
+            cfg = np.asarray(env_config, np.int64).reshape(-1)
+            if len(cfg) != num_envs or np.any(cfg < 0) or np.any(cfg >= len(mix.samplers)):
+                raise ValueError("env_config must hold one configuration index per env")
+            env_scene = mix.scene_offset[cfg]
+        # the scenario at creation is the episode-0 draw, so that creation and the first reset() agree
+        pose, light, scene, _ = mix.sample_numpy(np.arange(num_envs), 0, env_scene)
+        sc = scenarios.Scenario("yaml-mix", mix.scene_specs(), scene.astype(np.int32), pose, light,
+                                max_contacts=max_contacts)
+        vec = cls(sc, device=device, **kwargs)
+        vec.use_device_sampler(mix)
+        return vec
+
     def use_device_sampler(self, sampler, seed=0, env_id_base=0):
         """Attach on-device scene sampling: `reset()` and `reset_done()` then draw fresh scenes inside the reset kernel
-        (kb_reset_sampled, one launch, no host round trip).  sampler: a `sampler.SceneSampler`, or a Yaml configuration
-        (then the batch's scenes must already be the sampler's: see `from_configuration`)."""
-        from ..sampler import SceneSampler
+        (kb_reset_sampled, one launch, no host round trip).  sampler: a `sampler.SceneSampler`, a `sampler.SamplerMix`
+        (several configurations: see `from_configurations`), or a Yaml configuration (then the batch's scenes must
+        already be the sampler's: see `from_configuration`)."""
+        from ..sampler import SamplerMix, SceneSampler
+        if isinstance(sampler, SamplerMix):
+            if (sampler.M, sampler.N, sampler.light_state_dim()) != (self.batch.M, self.batch.N, self.batch.L):
+                raise ValueError("the configurations do not match the batch (objects / kilobots / light state)")
+            if len(sampler.scene_config) > len(self.scenario.scenes):
+                raise ValueError("the batch lacks scene templates of the mix (from_configurations)")
+            self.batch.set_sampler_mix(sampler)
+            self.sampler = sampler
+            return sampler
         if self.mixed_counts:
             raise ValueError("on-device scene sampling draws one configuration: the batch's scenes differ in their "
                              "numbers of objects / kilobots")
@@ -166,6 +220,7 @@ class KilobotsVecEnv:
         scenario's initial poses."""
         if body_pose is None and getattr(self, "sampler", None) is not None:
             self.batch.reset_sampled(done)
+            self._after_sampled_reset(done)
             return
         pose = self.scenario.body_pose if body_pose is None else body_pose
         light = self.scenario.light_state if light_state is None else light_state
@@ -187,6 +242,7 @@ class KilobotsVecEnv:
         """KilobotsEnv.reset for every (masked) env: rebuild bodies at the poses, one settle step."""
         if body_pose is None and getattr(self, "sampler", None) is not None:
             self.batch.reset_sampled(mask)    # a fresh scene per env, like every reference reset()
+            self._after_sampled_reset(mask)
             self._sim_steps = 0
             return self.get_observation()
         pose = self.scenario.body_pose if body_pose is None else body_pose

@@ -26,6 +26,7 @@ STREAM_KILOBOT_ANGLE = 4
 STREAM_SWARM = 5
 STREAM_SHUFFLE = 6
 STREAM_ACTION = 7
+STREAM_CONFIG = 8      # the configuration of a reset in a batch that mixes several (sampler.SamplerMix)
 
 
 def philox4x32(c0, c1, c2, c3, k0, k1):

@@ -211,3 +211,117 @@ class SceneSampler:
         xy = np.minimum(np.maximum(xy, lo + 0.02), -lo - 0.02)
         pose[:, M:, :2] = xy
         return pose, light[:, :L], scene
+
+
+class SamplerMix:
+    """Several Yaml configurations over ONE batch (kb_set_sampler_mix): a curriculum or domain randomisation over swarm
+    size and object sets.  Every configuration keeps its own `SceneSampler`; the batch's scene templates are theirs,
+    concatenated (configuration c owns scenes scene_offset[c] ..).  Bodies use the batch's padded layout: with M / N the
+    largest object / kilobot counts, an env's objects are rows 0..M_e-1 and its kilobots rows M + k.
+
+    weights None: a sampled reset draws the configuration of the env's scene (`KilobotsVecEnv.set_env_scene` moves an env
+    to another configuration).  weights [K] (finite, >= 0, positive sum): every sampled reset draws the configuration,
+    c = first k with u < cdf[k], u a uniform of its own stream (philox.STREAM_CONFIG) keyed by (seed, global env id,
+    episode) -- then the scene of c exactly as c's SceneSampler would.  So a size curriculum is a pure device loop whose
+    draws do not depend on the batch size or the number of ranks."""
+
+    def __init__(self, configurations, weights=None, seed=0, env_id_base=0):
+        confs = list(configurations)
+        K = len(confs)
+        if not 1 <= K <= abi.KB_SAMPLE_MAX_CONFIGS:
+            raise ValueError("a mix holds 1 to %d configurations, got %d" % (abi.KB_SAMPLE_MAX_CONFIGS, K))
+        self.seed, self.env_id_base = int(seed), int(env_id_base)
+        self.samplers = [SceneSampler(c, seed=seed, env_id_base=env_id_base) for c in confs]
+        s0 = self.samplers[0]
+        for c, s in enumerate(self.samplers):
+            if s.M > abi.KB_SAMPLE_MAX_OBJECTS:
+                raise ValueError("configuration %d has %d objects: on-device sampling draws at most %d"
+                                 % (c, s.M, abi.KB_SAMPLE_MAX_OBJECTS))
+            if s.light_types != s0.light_types or s.light_state_dim() != s0.light_state_dim():
+                raise ValueError("configuration %d has other light components than configuration 0: the envs of a batch "
+                                 "share their light state and action vectors" % c)
+            if not np.array_equal(s.size, s0.size):
+                raise ValueError("configuration %d has another table size than configuration 0" % c)
+        counts = [len(s.perms) for s in self.samplers]
+        self.scene_offset = np.concatenate([[0], np.cumsum(counts)[:-1]]).astype(np.int64)
+        for s, off in zip(self.samplers, self.scene_offset):
+            s.perm_scene = [int(off) + i for i in range(len(s.perms))]
+        self.scene_config = np.concatenate([np.full(n, c, np.int32) for c, n in enumerate(counts)])
+        self.M = max(s.M for s in self.samplers)
+        self.N = max(s.N for s in self.samplers)
+        self.weights = self.cdf = None
+        if weights is not None:
+            w = np.asarray(weights, dtype=np.float64).reshape(-1)
+            if len(w) != K:
+                raise ValueError("%d weights for %d configurations" % (len(w), K))
+            if not np.all(np.isfinite(w)) or np.any(w < 0):
+                raise ValueError("weights must be finite and non-negative")
+            total = 0.0
+            for x in w:
+                total += float(x)
+            if not (total > 0.0 and math.isfinite(total)):
+                raise ValueError("weights must have a positive sum")
+            # the cumulative weights exactly as kb_set_sampler_mix forms them: 1.0 from the last positive weight on
+            last = int(np.flatnonzero(w > 0)[-1])
+            cdf, acc = [], 0.0
+            for k in range(K):
+                acc += float(w[k])
+                cdf.append(1.0 if k >= last else acc / total)
+            self.weights, self.cdf = w, np.array(cdf)
+
+    def scene_specs(self):
+        """The batch's scene templates: every configuration's (SceneSampler.scene_specs), in configuration order."""
+        return [sp for s in self.samplers for sp in s.scene_specs()]
+
+    def first_scene(self, config):
+        """The scene an env of configuration `config` starts from (set_env_scene moves it there)."""
+        return int(self.scene_offset[config])
+
+    def light_state_dim(self):
+        return self.samplers[0].light_state_dim()
+
+    def to_abi(self):
+        """(KbSampleSpec[K], K, weights f64[K] or None, keep-alive): the arguments of kb_set_sampler_mix."""
+        K = len(self.samplers)
+        specs = (abi.KbSampleSpec * K)()
+        keep = []
+        for c, s in enumerate(self.samplers):
+            specs[c], k = s.to_abi()
+            keep.append(k)
+        w = None if self.weights is None else (C.c_double * K)(*[float(x) for x in self.weights])
+        return specs, K, w, (specs, keep, w)
+
+    def sample_numpy(self, env_ids, episodes=0, env_scene=None):
+        """(body_pose [E, M+N, 3], light_state [E, L], scene [E], config [E]) for the given LOCAL env ids and episode
+        counts, in the padded layout with NaN rows for absent bodies.  env_scene [E]: the envs' scenes, which pick the
+        configuration when the mix has no weights."""
+        env = np.asarray(env_ids, dtype=np.int64).reshape(-1)
+        E = len(env)
+        ep = np.broadcast_to(np.asarray(episodes, dtype=np.int64), (E,))
+        K = len(self.samplers)
+        if self.cdf is not None:
+            u, _ = PX.EnvRng(self.seed, env + self.env_id_base, ep).uniform2(PX.STREAM_CONFIG, 0)
+            config = np.argmax(u[:, None] < self.cdf[None, :], axis=1).astype(np.int32)
+        elif K == 1:
+            config = np.zeros(E, np.int32)
+        elif env_scene is None:
+            raise ValueError("without weights an env's configuration is that of its scene: pass env_scene")
+        else:
+            config = self.scene_config[np.asarray(env_scene, np.int64).reshape(E)]
+            if np.any(config < 0):
+                raise ValueError("env_scene holds a scene of no configuration")
+        pose = np.full((E, self.M + self.N, 3), np.nan)
+        light = np.zeros((E, self.light_state_dim()))
+        scene = np.zeros(E, np.int32)
+        for c, s in enumerate(self.samplers):
+            sel = np.flatnonzero(config == c)
+            if len(sel) == 0:
+                continue
+            p, l, sc = s.sample_numpy(env[sel], ep[sel])
+            pose[sel, :s.M] = p[:, :s.M]
+            pose[sel, self.M:self.M + s.N] = p[:, s.M:]
+            light[sel] = l
+            scene[sel] = sc if s.shuffle else s.perm_scene[0]
+        if K == 1 and not self.samplers[0].shuffle and env_scene is not None:
+            scene = np.asarray(env_scene, np.int32).reshape(E).copy()   # one configuration: the env keeps its scene
+        return pose, light, scene, config

@@ -226,8 +226,29 @@ typedef struct KbSampleSpec {
   const int32_t* perm_scene;       /* [num_lights!] or NULL */
   double kilobot_mean[2], kilobot_std;
 } KbSampleSpec;
-/* also restarts the episode counts; KB_ERR_UNSUPPORTED for a batch whose scenes differ in their object / kilobot counts */
+/* also restarts the episode counts; KB_ERR_UNSUPPORTED for a batch whose scenes differ in their object / kilobot counts
+   (kb_set_sampler_mix draws such a batch).  Without shuffle_lights the env keeps its scene and perm_scene is not read. */
 int kb_set_sampler(KbHandle* h, const KbSampleSpec* spec);
+/*
+ * On-device scene sampling for a batch that mixes K configurations (K = 1 is kb_set_sampler's case, without its refusal
+ * of a mixed batch).  Every configuration c has its own spec; its scenes are specs[c].perm_scene: the scene of every
+ * permutation (num_lights! entries with shuffle_lights, else 1 entry, the configuration's scene).  perm_scene is required
+ * when K > 1; with K = 1 and no shuffle it is not read and the env keeps its scene, as with kb_set_sampler.  Every scene of
+ * the batch belongs to at most one configuration, and every env's current scene to exactly one.  A spec's num_objects
+ * equals the object count of each of its scenes, and its scenes have one kilobot count.
+ *   weights  host f64[K] or NULL.  NULL: a sampled reset draws the configuration of the env's scene (kb_set_env_scene
+ *            moves an env to another one).  Non-NULL (finite, >= 0, positive sum): every sampled reset first draws the
+ *            configuration, c = first k with u < cdf[k] (cdf = the normalised cumulative weights, its last entry 1.0);
+ *            u is a Philox uniform of its own stream keyed by (seed, global env id, episode).
+ * Then the reset draws the scene of c exactly as kb_set_sampler would for a batch of c alone, in the padded body layout:
+ * objects at 0..M_e-1, kilobots at Mmax + k; the rows of absent bodies in kb_get_sampled's body_pose are quiet NaN.
+ * seed and env_id_base come from specs[0] and must agree over the specs.  Restarts the episode counts.  While such a
+ * sampler is attached, kb_set_env_scene refuses a scene that belongs to no configuration.
+ */
+#define KB_SAMPLE_MAX_CONFIGS 16
+int kb_set_sampler_mix(KbHandle* h, const KbSampleSpec* specs, int32_t num_specs, const double* weights);
+/* device i32[E]: the scene each env was last reset with, written on `stream` without synchronising */
+int kb_current_scenes(KbHandle* h, int32_t* out_device, void* stream);
 /* like kb_reset, with the poses / light states drawn on the device; mask: device u8[E] or NULL */
 int kb_reset_sampled(KbHandle* h, const uint8_t* mask, void* stream);
 /* what the last sampled resets drew: host f64[E,B,3], f64[E,L], i32[E] scene per env, u32[E] resets so far (any may be NULL) */
