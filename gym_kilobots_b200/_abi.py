@@ -125,6 +125,14 @@ class KbTaskDef(C.Structure):
     ]
 
 
+# per-kilobot local observations (include/kb_b200.h kb_local_observation)
+KB_LOCAL_NEIGHBOURS, KB_LOCAL_OBJECTS, KB_LOCAL_LIGHT = 1, 2, 4
+
+
+class KbLocalObsDef(C.Structure):
+    _fields_ = [("radius", C.c_float), ("max_neighbours", C.c_int32), ("parts", C.c_int32), ("pad", C.c_int32)]
+
+
 KB_SAMPLE_FIXED, KB_SAMPLE_RANDOM, KB_SAMPLE_AT_OBJECT = 0, 1, 2
 KB_SAMPLE_MEAN_LIGHT, KB_SAMPLE_MEAN_RANDOM = 1, 2
 KB_SAMPLE_MAX_OBJECTS = 16
@@ -204,6 +212,8 @@ PRODUCT_ONLY = {
     "reset_sampled": (C.c_int, [_VP, _VP, _VP]),
     "get_sampled": (C.c_int, [_VP, _VP, _VP, _VP, _VP]),
     "selftest_exact_math": (C.c_int, [C.c_int32, C.c_int32, C.POINTER(C.c_uint64)]),
+    "local_observation_dim": (C.c_int, [_VP, C.POINTER(KbLocalObsDef)]),
+    "local_observation": (C.c_int, [_VP, C.POINTER(KbLocalObsDef), _VP, _VP, _VP]),
 }
 
 

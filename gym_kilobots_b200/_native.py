@@ -304,6 +304,38 @@ class NativeBatch:
         _check(_fn["bind_flat_observation"](self.h, C.c_void_p(self.obs_flat.data_ptr())), "kb_bind_flat_observation")
         return self.obs_flat
 
+    # ---- per-kilobot local observations (csrc/kb_local.cuh)
+    def local_observation_dim(self, spec):
+        """Row width D of scene.LocalObsSpec `spec` on this batch (raises if the batch cannot provide a part)."""
+        d = spec.to_def()
+        D = _fn["local_observation_dim"](self.h, C.byref(d))
+        _check(min(D, 0), "kb_local_observation_dim")
+        return D
+
+    def local_observation(self, spec, mask=None, out=None):
+        """Device float32 [E, Nmax, D]: each kilobot's neighbours, objects and light in its own frame, from the state after
+        the last call on the current stream (asynchronous, no synchronisation).  mask: uint8 / bool [E] (device or
+        host) or None; the rows of unmasked envs are left as they were.  Without `out` the result goes to a buffer
+        kept per spec, so a later call with the same spec overwrites it."""
+        torch = self.torch
+        if out is None:
+            cache = self.__dict__.setdefault("_local_out", {})
+            out = cache.get(spec)
+            if out is None:
+                out = torch.full((self.E, self.N, self.local_observation_dim(spec)), float("nan"), dtype=torch.float32,
+                                 device=self.device)   # (rows a masked call has not written yet)
+                cache[spec] = out
+        elif (out.dtype != torch.float32 or out.device != self.device or not out.is_contiguous()
+              or tuple(out.shape) != (self.E, self.N, self.local_observation_dim(spec))):
+            raise ValueError("out must be a contiguous float32 tensor [E, Nmax, D] on the batch's device")
+        m = self._dev(mask, torch.uint8, (self.E,))
+        d = spec.to_def()
+        _check(_fn["local_observation"](self.h, C.byref(d), None if m is None else C.c_void_p(m.data_ptr()),
+                                        C.c_void_p(out.data_ptr()), self._stream()),
+               "kb_local_observation")
+        self._keep_local = m
+        return out
+
     def render(self, env_ids=(0,), width=1200, height=900):
         """uint8 CUDA tensor [len(env_ids), height, width, 3]: the picture KilobotsEnv.render would draw
         (kilobots_env.py:221-275; default size = screen_size :22), rasterised on the device."""

@@ -20,6 +20,7 @@
 #include "kb_toi.cuh"
 #include "kb_swarm.cuh"
 #include "kb_render.cuh"
+#include "kb_local.cuh"
 
 namespace kb {
 
@@ -1935,6 +1936,91 @@ int kb_render(KbHandle* hh, const int32_t* env_ids, int32_t num_images, int32_t 
   a.out = rgb;
   const dim3 block(16, 16), grid((width + 15) / 16, (height + 15) / 16, num_images);
   kb_render_kernel<<<grid, block, 0, st>>>(a);
+  CUDA_TRY(cudaGetLastError());
+  return KB_OK;
+}
+
+// ---- per-kilobot local observations (kb_local.cuh) -----------------------------------------------------------------
+static int localObsDim(const Handle* h, const KbLocalObsDef* def, const char* who) {
+  if (!h) return fail(KB_ERR_INVALID, std::string(who) + ": null handle");
+  if (!def) return fail(KB_ERR_INVALID, std::string(who) + ": null def");
+  const int all = KB_LOCAL_NEIGHBOURS | KB_LOCAL_OBJECTS | KB_LOCAL_LIGHT;
+  if (def->parts == 0 || (def->parts & ~all) != 0)
+    return fail(KB_ERR_INVALID, std::string(who) + ": parts must be a non-empty set of KB_LOCAL_* bits");
+  if (def->max_neighbours < 1 || def->max_neighbours > 32)
+    return fail(KB_ERR_INVALID, std::string(who) + ": max_neighbours must be in 1..32");
+  if (!std::isfinite(def->radius) || !(def->radius > 0.0f))
+    return fail(KB_ERR_INVALID, std::string(who) + ": radius must be finite and > 0");
+  if ((def->parts & KB_LOCAL_OBJECTS) && h->L.M == 0)
+    return fail(KB_ERR_INVALID, std::string(who) + ": KB_LOCAL_OBJECTS on a batch without objects");
+  if ((def->parts & KB_LOCAL_LIGHT) && h->L.numLights == 0)
+    return fail(KB_ERR_INVALID, std::string(who) + ": KB_LOCAL_LIGHT on a batch without lights");
+  int D = 0;
+  if (def->parts & KB_LOCAL_NEIGHBOURS) D += 1 + 4 * def->max_neighbours;
+  if (def->parts & KB_LOCAL_OBJECTS) D += 5 * h->L.M;
+  if (def->parts & KB_LOCAL_LIGHT) D += 3;
+  return D;
+}
+
+int kb_local_observation_dim(const KbHandle* hh, const KbLocalObsDef* def) {
+  return localObsDim(reinterpret_cast<const Handle*>(hh), def, "kb_local_observation_dim");
+}
+
+int kb_local_observation(KbHandle* hh, const KbLocalObsDef* def, const uint8_t* mask, float* out, void* stream) {
+  Handle* h = reinterpret_cast<Handle*>(hh);
+  const int D = localObsDim(h, def, "kb_local_observation");
+  if (D < 0) return D;
+  if (!out) return fail(KB_ERR_INVALID, "kb_local_observation: null out");
+  if (h->numEnvs == 0 || h->L.N == 0) return KB_OK;
+  CUDA_TRY(cudaSetDevice(h->device));
+  LocalArgs a;
+  a.L = h->L;
+  a.blobs = h->dBlobs;
+  a.envScene = h->dEnvScene;
+  a.bodies = h->dBodies;
+  a.scenes = h->dScenes;
+  a.lights = h->dLights;
+  a.mask = mask;
+  a.out = out;
+  a.numEnvs = h->numEnvs;
+  a.K = def->max_neighbours;
+  a.parts = def->parts;
+  a.D = D;
+  a.r2 = def->radius * def->radius;
+  // grid over the table (metres), cells at least 1.001 radius wide: the slack keeps a pair within the radius in adjacent
+  // cells whatever the rounding of the cell index; a radius wider than the table leaves one cell (brute force)
+  const double x0 = h->wall[0] / 25.0, y0 = h->wall[1] / 25.0;
+  const double w = std::max(h->wall[2] / 25.0 - x0, h->wall[3] / 25.0 - y0);
+  const double cw0 = 1.001 * (double)def->radius;
+  int n = w > 0.0 ? (int)std::min((double)KB_LOCAL_GRID_AXIS, std::floor(w / cw0)) : 1;
+  n = std::max(n, 1);
+  const double cw = w > 0.0 ? w / n : 1.0;
+  a.x0 = (float)x0;
+  a.y0 = (float)y0;
+  a.invCell = (float)(1.0 / cw);
+  a.gx = n;
+  a.gy = n;
+  const bool forceGrid = [] {
+    const char* ev = getenv("KB_LOCAL_FORCE_GRID");
+    return ev && atoi(ev) != 0;
+  }();
+  cudaStream_t st = (cudaStream_t)stream;
+  const bool small = a.K <= 8;
+  if (!forceGrid && h->L.B <= KB_LOCAL_WARP_BODIES) {
+    const int grid = (h->numEnvs + KB_LOCAL_WARPS - 1) / KB_LOCAL_WARPS;
+    if (small)
+      kb_local_warp_kernel<8><<<grid, 32 * KB_LOCAL_WARPS, 0, st>>>(a);
+    else
+      kb_local_warp_kernel<32><<<grid, 32 * KB_LOCAL_WARPS, 0, st>>>(a);
+  } else {
+    const int cells = a.gx * a.gy;
+    const size_t smem = 16 * (size_t)h->L.B + 4 * (size_t)(2 * cells + 1) + 2 * (size_t)h->L.N;
+    if (smem > 48 * 1024) CUDA_TRY(small ? raiseSmemLimit(kb_local_grid_kernel<8>, smem) : raiseSmemLimit(kb_local_grid_kernel<32>, smem));
+    if (small)
+      kb_local_grid_kernel<8><<<h->numEnvs, KB_LOCAL_CTA, smem, st>>>(a);
+    else
+      kb_local_grid_kernel<32><<<h->numEnvs, KB_LOCAL_CTA, smem, st>>>(a);
+  }
   CUDA_TRY(cudaGetLastError());
   return KB_OK;
 }

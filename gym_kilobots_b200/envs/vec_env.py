@@ -6,6 +6,8 @@ this class steps E of them with one kernel launch.  Semantics per environment ar
 ({'kilobots': [N,3], 'objects': [M,3], 'light': [L]}, kilobots_env.py:115-118) with a leading env axis.
 The envs of one batch may differ in their numbers of objects and kilobots: N and M are then the largest counts,
 `kilobot_mask` / `object_mask` say which rows an env populates, and the rows it does not are NaN.
+With `local_observation=scene.LocalObsSpec(...)` the observation also holds obs['local'] [E, N, D]: what each kilobot
+senses in its own frame (neighbours, objects, light), computed on the device after every step and reset.
 """
 import numpy as np
 
@@ -21,10 +23,11 @@ class KilobotsVecEnv:
     """
 
     def __init__(self, scenario, device=0, action_mode=abi.KB_ACTION_LIGHT, task=None, targets=None,
-                 flat_observation=False, allow_status_flags=False):
+                 flat_observation=False, allow_status_flags=False, local_observation=None):
         """task / targets: optional `scene.TaskSpec` and per-env target poses [E,3] -- on-device reward, done and
         episode statistics (an extension: the reference's hooks are abstract and its in-tree envs return constants).
-        flat_observation: also emit obs['flat'], the vector YamlKilobotsEnv.observation_space describes."""
+        flat_observation: also emit obs['flat'], the vector YamlKilobotsEnv.observation_space describes.
+        local_observation: a `scene.LocalObsSpec`; also emit obs['local'], each kilobot's local observation."""
         self.scenario = scenario
         # KB_STATUS_* bits (contact / solver capacity overflow, non-finite pose) raise KbStatusError in step() and
         # check_status() unless explicitly allowed: a dropped pair is silently different physics
@@ -39,6 +42,9 @@ class KilobotsVecEnv:
         self._host = None
         self._sim_steps = 0
         self.obs_flat = self.batch.bind_flat_observation() if flat_observation else None
+        self.local_spec = local_observation
+        if local_observation is not None:
+            self.local_dim = self.batch.local_observation_dim(local_observation)   # refuses a part the batch lacks
         self._init_masks()
         if task is not None:
             self.set_task(task, targets)
@@ -221,11 +227,20 @@ class KilobotsVecEnv:
         if body_pose is None and getattr(self, "sampler", None) is not None:
             self.batch.reset_sampled(done)
             self._after_sampled_reset(done)
-            return
-        pose = self.scenario.body_pose if body_pose is None else body_pose
-        light = self.scenario.light_state if light_state is None else light_state
-        self.batch.reset(pose, light, None, done)
-        self._after_reset(done)
+        else:
+            pose = self.scenario.body_pose if body_pose is None else body_pose
+            light = self.scenario.light_state if light_state is None else light_state
+            self.batch.reset(pose, light, None, done)
+            self._after_reset(done)
+        if self.local_spec is not None:
+            self.batch.local_observation(self.local_spec, mask=done)   # the rebuilt envs' rows of obs['local']
+
+    def local_observation(self, mask=None):
+        """obs['local'] of the current state on demand: device float32 [E, N, D] (the buffer step_device returns);
+        mask [E]: refresh only those envs' rows."""
+        if self.local_spec is None:
+            raise ValueError("the batch was built without local_observation=LocalObsSpec(...)")
+        return self.batch.local_observation(self.local_spec, mask=mask)
 
     # -- gym-like surface ---------------------------------------------------------------------
     @property
@@ -243,16 +258,18 @@ class KilobotsVecEnv:
         if body_pose is None and getattr(self, "sampler", None) is not None:
             self.batch.reset_sampled(mask)    # a fresh scene per env, like every reference reset()
             self._after_sampled_reset(mask)
-            self._sim_steps = 0
-            return self.get_observation()
-        pose = self.scenario.body_pose if body_pose is None else body_pose
-        light = self.scenario.light_state if light_state is None else light_state
-        if kb_velocity is None:
-            kb_velocity = getattr(self.scenario, "kb_velocity", None)
-        self.batch.reset(pose, light, kb_velocity, mask)
-        self._after_reset(mask)
+        else:
+            pose = self.scenario.body_pose if body_pose is None else body_pose
+            light = self.scenario.light_state if light_state is None else light_state
+            if kb_velocity is None:
+                kb_velocity = getattr(self.scenario, "kb_velocity", None)
+            self.batch.reset(pose, light, kb_velocity, mask)
+            self._after_reset(mask)
         self._sim_steps = 0
-        return self.get_observation()
+        obs = self.get_observation()
+        if self.local_spec is not None:
+            obs["local"] = self.batch.local_observation(self.local_spec, mask=mask).cpu().numpy()
+        return obs
 
     def step_device(self, action):
         """Device tensors in, device tensors out, no synchronisation (training-loop path)."""
@@ -261,6 +278,8 @@ class KilobotsVecEnv:
         obs = {"kilobots": k, "objects": o, "light": l}
         if self.obs_flat is not None:
             obs["flat"] = self.obs_flat
+        if self.local_spec is not None:
+            obs["local"] = self.batch.local_observation(self.local_spec)
         return obs, r, d, {"status": s}
 
     def _host_buffers(self):
@@ -309,6 +328,8 @@ class KilobotsVecEnv:
         obs = {"kilobots": hb["kilobots"], "objects": hb["objects"], "light": hb["light"]}
         if self.obs_flat is not None:
             obs["flat"] = self.obs_flat.cpu().numpy()
+        if self.local_spec is not None:
+            obs["local"] = self.batch.local_observation(self.local_spec).cpu().numpy()
         return obs, hb["reward"], hb["done"].astype(bool), {"status": hb["status"]}
 
     def check_status(self):

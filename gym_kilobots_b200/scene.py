@@ -94,6 +94,51 @@ class TaskSpec:
         return t
 
 
+@dataclass(frozen=True)
+class LocalObsSpec:
+    """Per-kilobot local observation (include/kb_b200.h kb_local_observation): each kilobot's neighbours within `radius`
+    metres (their count, then the `max_neighbours` nearest as (x, y, distance, 1) in the kilobot's frame), every object
+    slot as (x, y, cos, sin, 1) in its frame, and the light (value, gradient x, y) at its sensor.  The parts follow each
+    other in that order; `dim(M)` is the row width for a batch with M object slots."""
+    radius: float
+    max_neighbours: int = 8
+    neighbours: bool = True
+    objects: bool = True
+    light: bool = False
+
+    def __post_init__(self):
+        if not (self.neighbours or self.objects or self.light):
+            raise ValueError("LocalObsSpec: select at least one part")
+        if not 1 <= int(self.max_neighbours) <= 32:
+            raise ValueError("LocalObsSpec: max_neighbours must be in 1..32")
+        r = float(self.radius)
+        if not (0.0 < r <= float(np.finfo(np.float32).max) and np.float32(r) > 0.0):   # (NaN fails the comparison)
+            raise ValueError("LocalObsSpec: radius must be finite and > 0 (metres)")
+
+    @property
+    def parts(self):
+        return ((abi.KB_LOCAL_NEIGHBOURS if self.neighbours else 0) | (abi.KB_LOCAL_OBJECTS if self.objects else 0) |
+                (abi.KB_LOCAL_LIGHT if self.light else 0))
+
+    def slices(self, num_objects):
+        """{'neighbours', 'objects', 'light'} -> the column slice of each selected part."""
+        out, c = {}, 0
+        for name, on, width in (("neighbours", self.neighbours, 1 + 4 * int(self.max_neighbours)),
+                                ("objects", self.objects, 5 * int(num_objects)), ("light", self.light, 3)):
+            if on:
+                out[name] = slice(c, c + width)
+                c += width
+        return out
+
+    def dim(self, num_objects):
+        return sum(s.stop - s.start for s in self.slices(num_objects).values())
+
+    def to_def(self):
+        d = abi.KbLocalObsDef()
+        d.radius, d.max_neighbours, d.parts = float(self.radius), int(self.max_neighbours), self.parts
+        return d
+
+
 @dataclass
 class SceneSpec:
     bodies: List[BodySpec] = field(default_factory=list)   # objects first, then kilobots

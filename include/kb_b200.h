@@ -369,6 +369,40 @@ int kb_reduce_episode_stats(KbHandle* h, double* out_device, void* stream);
 int kb_bind_flat_observation(KbHandle* h, float* obs_flat);
 int kb_flat_observation_dim(const KbHandle* h);
 
+/*
+ * Per-kilobot local observations: what each kilobot would sense itself, in its own frame -- the input of a swarm policy
+ * shared across the kilobots.  Computed from the state the handle holds after the last call on `stream` (kb_step*,
+ * kb_reset*, kb_set_poses*, kb_set_state), for the env's present kilobots.  Output: device f32[E, Nmax, D]; row k of env e
+ * belongs to padded kilobot k, the rows of absent kilobots are quiet NaN.  Per body b: p_b = the position kb_step reports
+ * in obs_kilobots / obs_objects, (float)((double)xf.p / 25.0) in metres, and (s_b, c_b) = xf.q.  Float32 arithmetic, every
+ * operation rounded separately.  The parts selected in `parts` follow each other in this order:
+ *   KB_LOCAL_NEIGHBOURS  1 + 4K columns: n_i = the number of other present kilobots j of the env with d2 <= radius^2
+ *                        (dx = p_j.x - p_i.x, dy = p_j.y - p_i.y, d2 = dx*dx + dy*dy; not capped at K), then K slots
+ *                        ascending by (d2, j) of (c_i*dx + s_i*dy, -s_i*dx + c_i*dy, sqrtf(d2), 1); unfilled slots are 0.
+ *   KB_LOCAL_OBJECTS     5 * Mmax columns: per object slot j the env has, its position in the kilobot's frame as above,
+ *                        cos = c_j*c_i + s_j*s_i, sin = s_j*c_i - c_j*s_i, 1; zeros for a slot it does not have.
+ *   KB_LOCAL_LIGHT       3 columns: the light value at the kilobot's light sensor (the point senseControl reads: the body
+ *                        origin of a SimplePhototaxisKilobot, the rear point (0, -r) of the others) and its gradient rotated
+ *                        into the body frame (c*gx + s*gy, -s*gx + c*gy), float64 with (double) of xf.q, then rounded to
+ *                        float32.  Composite light: the sum of the values, the gradient of the brightest child.
+ * max_neighbours (K) must be in 1..32, radius (metres) finite and > 0.  KB_LOCAL_FORCE_GRID=1 in the environment makes
+ * every batch take the uniform-grid kernel of large swarms (same result).
+ */
+#define KB_LOCAL_NEIGHBOURS 1
+#define KB_LOCAL_OBJECTS 2
+#define KB_LOCAL_LIGHT 4
+typedef struct KbLocalObsDef {
+  float radius;
+  int32_t max_neighbours;
+  int32_t parts;   /* KB_LOCAL_* bits */
+  int32_t pad;
+} KbLocalObsDef;
+/* D of the def on this batch, or a negative KbError */
+int kb_local_observation_dim(const KbHandle* h, const KbLocalObsDef* def);
+/* out: device f32[E, Nmax, D]; mask: device u8[E] or NULL = every env (rows of unmasked envs are not written).
+   Asynchronous on `stream`: no allocation, no host synchronisation. */
+int kb_local_observation(KbHandle* h, const KbLocalObsDef* def, const uint8_t* mask, float* out, void* stream);
+
 /* Off-screen rasteriser (SURVEY.md 8(f) n4): the picture KilobotsEnv.render draws through
  * kb_rendering.KilobotsViewer (kilobots_env.py:221-275) -- table, objects, kilobots, light -- for num_images
  * environments, straight from the device state.  env_ids: host i32[num_images]; rgb: DEVICE u8[num_images,
