@@ -196,7 +196,8 @@ PROTOTYPES = {
 class KbLaunchConfig(C.Structure):
     _fields_ = [("lanes_per_env", C.c_int32), ("block_threads", C.c_int32), ("grid_blocks", C.c_int32),
                 ("smem_bytes_per_block", C.c_int32), ("state_words_per_env", C.c_int32),
-                ("smem_words_per_env", C.c_int32)]
+                ("smem_words_per_env", C.c_int32), ("specialised", C.c_int32), ("jit_ms", C.c_float),
+                ("jit_reason", C.c_char * 256)]
 
 
 PRODUCT_ONLY = {
@@ -204,6 +205,8 @@ PRODUCT_ONLY = {
     "get_state": (C.c_int, [_VP, _VP]),
     "set_state": (C.c_int, [_VP, _VP]),
     "get_launch_config": (C.c_int, [_VP, C.POINTER(KbLaunchConfig)]),
+    "jit_step_source": (C.c_int, [C.POINTER(KbSceneDesc), C.c_int32, C.c_int32, C.c_int32, C.c_char_p, C.c_int64,
+                                  C.c_char_p, C.c_int64, C.POINTER(C.c_double)]),
     "get_host_layout": (C.c_int, [_VP, C.POINTER(C.c_int64), C.POINTER(C.c_int64)]),
     "reduce_episode_stats": (C.c_int, [_VP, _VP, _VP]),
     "set_sampler": (C.c_int, [_VP, C.POINTER(KbSampleSpec)]),

@@ -62,6 +62,24 @@ def exported_symbols():
     return ["kb_" + n for n in list(abi.PROTOTYPES) + list(abi.PRODUCT_ONLY)]
 
 
+def jit_step_source(scenes, max_contacts=0, compile=False):
+    """(source, log, compile_ms) of the specialised step kernel kb_create would build for a lane-group batch of
+    `scenes`; with compile=True it is also compiled with NVRTC, and log holds ptxas's resource report.  No GPU needed."""
+    load()
+    scenes = list(scenes) if isinstance(scenes, (list, tuple)) else [scenes]
+    descs = (abi.KbSceneDesc * len(scenes))()
+    keep = []
+    for i, s in enumerate(scenes):
+        descs[i], k = s.to_desc()
+        keep.append(k)
+    src = C.create_string_buffer(1 << 16)
+    log = C.create_string_buffer(1 << 20)
+    ms = C.c_double(0.0)
+    _check(_fn["jit_step_source"](descs, len(scenes), max_contacts, int(compile), src, len(src), log, len(log),
+                                  C.byref(ms)), "kb_jit_step_source")
+    return src.value.decode(), log.value.decode(), ms.value
+
+
 def _check(rc, what):
     if rc != 0:
         raise RuntimeError("%s failed (%d): %s" % (what, rc, _fn["last_error"]().decode()))
@@ -355,7 +373,10 @@ class NativeBatch:
     def launch_config(self):
         cfg = abi.KbLaunchConfig()
         _check(_fn["get_launch_config"](self.h, C.byref(cfg)), "kb_get_launch_config")
-        out = {k: int(getattr(cfg, k)) for k, _ in cfg._fields_}
+        out = {k: int(getattr(cfg, k)) for k, _ in cfg._fields_ if k not in ("specialised", "jit_ms", "jit_reason")}
+        out["specialised"] = bool(cfg.specialised)
+        out["jit_ms"] = round(float(cfg.jit_ms), 1)
+        out["jit_reason"] = cfg.jit_reason.decode()
         out["kernel"] = ("kb_swarm_step_kernel (one CTA per env)" if out["lanes_per_env"] > 32
                          else "kb_step_kernel<%d>" % out["lanes_per_env"])
         return out

@@ -17,95 +17,19 @@
 #include <string>
 #include <vector>
 
-#include "kb_toi.cuh"
+#include "kb_step_kernel.cuh"
 #include "kb_swarm.cuh"
 #include "kb_render.cuh"
 #include "kb_local.cuh"
+#include "kb_jit.h"
 
 namespace kb {
 
 // ----------------------------------------------------------------------------------- kernels
-// threads per block.  The warps of a block rendezvous at the phase boundaries (KB_T in kb_step.cuh) and so share
-// instruction-cache lines: with one warp per block the 4-lane kernel spent 10 of 17 cycles per issue waiting for
-// instructions (profiles/ncu_step_kernel_r01_c5_block32_before.txt).  Measured on C5 (2^18 envs, kilobot-steps/s):
-// 32 threads 70 M, 64 threads 114 M, 96 threads 132 M, 128 threads 139 M, 192 threads 132 M; the wider kernels are best
-// at two warps (C2: 64 threads 1.215 ms, 128 threads 1.239 ms; C3: 5.39 vs 5.55 ms).
-#ifndef KB_BLOCK4
-#define KB_BLOCK4 128
-#endif
-#ifndef KB_BLOCK8
-#define KB_BLOCK8 64
-#endif
-#ifndef KB_BLOCK16
-#define KB_BLOCK16 64
-#endif
-#ifndef KB_MINBLOCKS16
-#define KB_MINBLOCKS16 6
-#endif
-#ifndef KB_MINBLOCKS8
-#define KB_MINBLOCKS8 3
-#endif
-#ifndef KB_MINBLOCKS4
-#define KB_MINBLOCKS4 6   /* 6 blocks of 64 threads per SM: <= 168 registers (C5: 96 resident envs per SM) */
-#endif
-#ifndef KB_BLOCK32
-#define KB_BLOCK32 64
-#endif
-#define KB_BLOCK_OF(LPE) ((LPE) == 4 ? KB_BLOCK4 : ((LPE) == 8 ? KB_BLOCK8 : ((LPE) == 16 ? KB_BLOCK16 : KB_BLOCK32)))
-
-// The batch is padded to a whole number of blocks (numEnvs <= grid * EPB): every lane of the step kernel owns
-// a real environment, so the groups of a warp can run in lock step.  Padding envs replicate the inputs of the
-// last real env and never write outputs.
+// the generic step kernel: offsets, counts and constants come from the Layout in the kernel parameters
 template <int LPE>
-__global__ void __launch_bounds__(KB_BLOCK_OF(LPE), (LPE == 32 ? (512 / KB_BLOCK32) : (KB_BLOCK_OF(LPE) > 64 ? (384 / KB_BLOCK_OF(LPE)) : (LPE == 16 ? KB_MINBLOCKS16 : (LPE == 4 ? KB_MINBLOCKS4 : KB_MINBLOCKS8))))) kb_step_kernel(const __grid_constant__ KernelArgs a) {
-  constexpr int EPB = KB_BLOCK_OF(LPE) / LPE;
-  const int slot = threadIdx.x / LPE;
-  const int env = a.envOffset + blockIdx.x * EPB + slot;
-  const int envIn = min(env, a.numEnvs - 1);
-  Sim<LPE, true> s(a.L);
-  s.g.init();
-  s.bind(slot);
-  s.blob = a.blobs + (size_t)env * a.L.blobWords;
-  const int scene = a.envScene ? (int)reinterpret_cast<const uint32_t*>(s.blob)[a.L.oHdr + H_SCENE] : 0;   // (last reset's)
-  s.px = a.proxies + (size_t)scene * a.L.Pp;
-  s.bc = a.bodies + (size_t)scene * a.L.Bp;
-  s.lights = a.lights + (size_t)scene * (a.L.numLights > 0 ? a.L.numLights : 1);
-  s.S = a.L.B;
-#ifdef KB_PROFILE
-  s.profOut = a.prof ? a.prof + (size_t)envIn * KB_PROF_SLOTS : nullptr;
-  if (s.profOut && s.g.lane == 0) s.profOut[13] = s.profOut[14] = s.profOut[15] = 0ull;
-#endif
-  s.loadState();
-  s.initScratch();
-  const int A = a.actionMode == KB_ACTION_KILOBOTS ? 2 * a.L.N : a.L.A;
-  const double* act = a.action ? a.action + (size_t)envIn * A : nullptr;
-  // the doubled warp barriers after setKilobotActions and senseControl are redundant but kept: without them the
-  // compiler schedules this kernel differently (measured in SASS)
-  if (a.actionMode == KB_ACTION_KILOBOTS) {
-    setKilobotActions(s, act, s.g.lane, LPE);
-    s.g.usync();
-  }
-  s.g.usync();
-  if (a.task.mode != KB_TASK_CONST && s.g.lane == 0 && env < a.numEnvs)  // task layer, include/kb_b200.h
-    taskBegin(s, a, env);
-  for (int step = 0; step < a.L.stepsPerAction; ++step) {
-    __syncthreads();  // keeps the warps of a block in the same phase (see KB_T in kb_step.cuh)
-    if (a.actionMode == KB_ACTION_LIGHT && act && a.L.numLights > 0) {
-      if (s.g.lane == 0) lightStep(s, act);
-      s.g.usync();
-    }
-    senseControl(s, s.g.lane, LPE);
-    s.g.usync();
-    s.g.usync();
-    s.worldStep();
-  }
-  if (env < a.numEnvs) s.gather(a, env);
-  s.storeState();
-#ifdef KB_PROFILE
-  s.tp[12] += clock64() - s.tlast;
-  if (a.prof && s.g.lane == 0 && env < a.numEnvs)
-    for (int i = 0; i < 13; ++i) a.prof[(size_t)env * KB_PROF_SLOTS + i] = (unsigned long long)s.tp[i];
-#endif
+__global__ void __launch_bounds__(KB_STEP_BOUNDS(LPE)) kb_step_kernel(const __grid_constant__ KernelArgs a) {
+  stepKernelBody<LPE>(a, a.L);
 }
 
 template <int LPE>
@@ -328,6 +252,10 @@ struct Handle {
   cudaStream_t pipe[2] = {nullptr, nullptr};
   cudaEvent_t evFork = nullptr, evJoin[2] = {nullptr, nullptr};
   int hostChunks = 1;
+  // the step kernel compiled for this batch's layout (kb_jit.h); null: the generic kb_step_kernel<LPE> runs
+  cudaKernel_t stepJit = nullptr;
+  float jitMs = 0.0f;          // its compile time in kb_create (0: from a cache)
+  std::string jitReason;       // why the generic kernel runs instead
 #ifdef KB_PROFILE
   unsigned long long* dProf = nullptr;
 #endif
@@ -639,27 +567,10 @@ static void fillArgs(const Handle* h, KernelArgs* a) {
 #endif
 }
 
-}  // namespace kb
-
-using namespace kb;
-
-extern "C" {
-
-const char* kb_last_error(void) { return g_err.c_str(); }
-
-int kb_create(const KbSceneDesc* scenes, int32_t num_scenes, const int32_t* env_scene, int32_t num_envs,
-              int32_t max_contacts, int32_t device, KbHandle** out) {
-  if (!scenes || num_scenes < 1 || num_envs < 1 || !out) return fail(KB_ERR_INVALID, "kb_create: invalid arguments");
-  int ndev = 0;
-  if (cudaGetDeviceCount(&ndev) != cudaSuccess || ndev <= 0 || device < 0 || device >= ndev) {
-    cudaGetLastError();
-    return fail(KB_ERR_NO_DEVICE, "kb_create: no CUDA device (this library has no CPU fallback)");
-  }
-  cudaDeviceProp prop;
-  CUDA_TRY(cudaGetDeviceProperties(&prop, device));
-  if (prop.major != 10) return fail(KB_ERR_NO_DEVICE, "kb_create: device is not sm_100 (B200); no fallback path exists");
-  CUDA_TRY(cudaSetDevice(device));
-
+// The batch's layout (h->L, h->W), tier, lane width and shared-memory size from its scenes.  Needs no device: `prop`
+// only sizes the large-swarm tier's image.
+static int planBatch(const KbSceneDesc* scenes, int32_t num_scenes, int32_t max_contacts, const cudaDeviceProp& prop,
+                     Handle* h) {
   const KbSceneDesc& s0 = scenes[0];
   // padded body layout: M / N are the largest object / kilobot counts over the scenes, objects at 0..M-1, kilobots at
   // M..M+N-1; a scene with fewer leaves absent bodies at the indices it does not populate
@@ -722,10 +633,6 @@ int kb_create(const KbSceneDesc* scenes, int32_t num_scenes, const int32_t* env_
   }
   if (!swarm && P > KB_MAX_PROXIES) return fail(KB_ERR_CAPACITY, "kb_create: more than 64 proxies per env is not supported");
 
-  Handle* h = new Handle();
-  h->device = device;
-  h->numEnvs = num_envs;
-  h->numScenes = num_scenes;
   Layout& L = h->L;
   std::memset(&L, 0, sizeof(L));
   L.B = B; L.M = M; L.N = N; L.P = P;
@@ -965,6 +872,45 @@ int kb_create(const KbSceneDesc* scenes, int32_t num_scenes, const int32_t* env_
     h->envsPerBlock = KB_BLOCK_OF(L.lanesPerEnv) / L.lanesPerEnv;
     h->smemBytes = (size_t)h->envsPerBlock * L.smemWords * 4;
   }
+  return KB_OK;
+}
+
+}  // namespace kb
+
+using namespace kb;
+
+extern "C" {
+
+const char* kb_last_error(void) { return g_err.c_str(); }
+
+int kb_create(const KbSceneDesc* scenes, int32_t num_scenes, const int32_t* env_scene, int32_t num_envs,
+              int32_t max_contacts, int32_t device, KbHandle** out) {
+  if (!scenes || num_scenes < 1 || num_envs < 1 || !out) return fail(KB_ERR_INVALID, "kb_create: invalid arguments");
+  int ndev = 0;
+  if (cudaGetDeviceCount(&ndev) != cudaSuccess || ndev <= 0 || device < 0 || device >= ndev) {
+    cudaGetLastError();
+    return fail(KB_ERR_NO_DEVICE, "kb_create: no CUDA device (this library has no CPU fallback)");
+  }
+  cudaDeviceProp prop;
+  CUDA_TRY(cudaGetDeviceProperties(&prop, device));
+  if (prop.major != 10) return fail(KB_ERR_NO_DEVICE, "kb_create: device is not sm_100 (B200); no fallback path exists");
+  CUDA_TRY(cudaSetDevice(device));
+
+  Handle* h = new Handle();
+  h->device = device;
+  h->numEnvs = num_envs;
+  h->numScenes = num_scenes;
+  {
+    const int rc = planBatch(scenes, num_scenes, max_contacts, prop, h);
+    if (rc != KB_OK) {
+      delete h;
+      return rc;
+    }
+  }
+  const KbSceneDesc& s0 = scenes[0];
+  const Layout& L = h->L;
+  const bool swarm = h->W.enabled != 0;
+  const int M = L.M, N = L.N;
   if (h->smemBytes > (size_t)prop.sharedMemPerBlockOptin) {
     delete h;
     return fail(KB_ERR_CAPACITY, swarm ? "kb_create: this swarm does not fit one SM's shared memory (about 1700 kilobots per env at the minimal capacities)"
@@ -1072,6 +1018,34 @@ int kb_create(const KbSceneDesc* scenes, int32_t num_scenes, const int32_t* env_
     KB_SET_SMEM(32)
   }
 #undef KB_SET_SMEM
+  if (!swarm) {
+    // KB_JIT=0: the generic kernel; KB_JIT=1: the specialised kernel or an error; unset: the specialised kernel when
+    // it can be had
+    const char* ev = getenv("KB_JIT");
+    const int mode = ev && *ev ? atoi(ev) : -1;
+    if (mode == 0) {
+      h->jitReason = "KB_JIT=0";
+    } else {
+      double ms = 0.0;
+      h->stepJit = jitStepKernel(L, &ms, &h->jitReason);
+      h->jitMs = (float)ms;
+      if (h->stepJit) {
+        const cudaError_t e = raiseSmemLimit((const void*)h->stepJit, h->smemBytes);
+        if (e != cudaSuccess) {
+          cudaGetLastError();
+          h->stepJit = nullptr;
+          h->jitReason = std::string("load error: ") + cudaGetErrorString(e);
+        }
+      }
+      if (!h->stepJit && mode == 1) {
+        const std::string why = h->jitReason;
+        kb_destroy(reinterpret_cast<KbHandle*>(h));
+        return fail(KB_ERR_CUDA, "kb_create: KB_JIT=1 but the specialised step kernel is not available: " + why);
+      }
+    }
+  } else {
+    h->jitReason = "large-swarm tier";
+  }
   {
     // end-to-end pipeline depth: one chunk per ~2 MB of outputs, at most 8, each a whole number of blocks and at
     // least a few waves long (small batches -- C2's 4096 envs are ONE wave -- stay a single launch)
@@ -1375,6 +1349,13 @@ static int stepRange(Handle* h, const double* action, int32_t action_mode, float
   a.status = status;
   a.obsFlat = h->obsFlat;
   a.envOffset = envBegin;
+  if (h->stepJit) {
+    void* args[] = {&a};
+    const int grid = (envCount + h->envsPerBlock - 1) / h->envsPerBlock;
+    CUDA_TRY(cudaLaunchKernel((const void*)h->stepJit, dim3(grid), dim3(KB_BLOCK_OF(h->L.lanesPerEnv)), args,
+                              h->smemBytes, stream));
+    return KB_OK;
+  }
   KB_LAUNCH_RANGE(kb_step_kernel, kb_swarm_step_kernel, h, stream, a, envCount);
   CUDA_TRY(cudaGetLastError());
   return KB_OK;
@@ -1691,6 +1672,27 @@ int kb_get_host_layout(const KbHandle* hh, int64_t* offsets, int64_t* total) {
   return KB_OK;
 }
 
+int kb_jit_step_source(const KbSceneDesc* scenes, int32_t num_scenes, int32_t max_contacts, int32_t compile,
+                       char* source, int64_t source_cap, char* log, int64_t log_cap, double* compile_ms) {
+  if (!scenes || num_scenes < 1 || !source || source_cap < 1) return fail(KB_ERR_INVALID, "kb_jit_step_source: invalid arguments");
+  cudaDeviceProp prop;
+  std::memset(&prop, 0, sizeof(prop));   // sizes only the large-swarm tier's image, which has no specialised kernel
+  Handle h;
+  const int rc = planBatch(scenes, num_scenes, max_contacts, prop, &h);
+  if (rc != KB_OK) return rc;
+  if (h.W.enabled) return fail(KB_ERR_INVALID, "kb_jit_step_source: the large-swarm tier has no specialised step kernel");
+  const std::string prelude = jitPrelude(h.L);
+  std::snprintf(source, (size_t)source_cap, "%s", prelude.c_str());
+  if (!compile) return KB_OK;
+  std::vector<char> cubin;
+  std::string text, err;
+  const auto t0 = std::chrono::steady_clock::now();
+  const bool ok = jitCompile(prelude, &cubin, &text, &err);
+  if (compile_ms) *compile_ms = std::chrono::duration<double, std::milli>(std::chrono::steady_clock::now() - t0).count();
+  if (log && log_cap > 0) std::snprintf(log, (size_t)log_cap, "%s", text.c_str());
+  return ok ? KB_OK : fail(KB_ERR_CUDA, "kb_jit_step_source: " + err);
+}
+
 int kb_get_launch_config(const KbHandle* hh, KbLaunchConfig* cfg) {
   const Handle* h = reinterpret_cast<const Handle*>(hh);
   if (!h || !cfg) return fail(KB_ERR_INVALID, "kb_get_launch_config: null");
@@ -1700,6 +1702,9 @@ int kb_get_launch_config(const KbHandle* hh, KbLaunchConfig* cfg) {
   cfg->smem_bytes_per_block = (int32_t)h->smemBytes;
   cfg->state_words_per_env = h->L.stateWords;
   cfg->smem_words_per_env = h->L.smemWords;
+  cfg->specialised = h->stepJit != nullptr;
+  cfg->jit_ms = h->jitMs;
+  std::snprintf(cfg->jit_reason, sizeof(cfg->jit_reason), "%s", h->jitReason.c_str());
   return KB_OK;
 }
 

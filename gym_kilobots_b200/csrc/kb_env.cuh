@@ -2,7 +2,7 @@
 // (lib/light.py:59-75,176-189,237-253,300-316), kilobot controllers (lib/kilobot.py:54-55,86-127,188-203,253-258,
 // 294-300,307-316,318-333) and the task layer (include/kb_b200.h "Task layer").
 //
-// Every function is a template over the tier's simulation struct T -- Sim<LPE, UNI> (kb_step.cuh, a lane group per
+// Every function is a template over the tier's simulation struct T -- Sim<LPE, UNI, LT> (kb_step.cuh, a lane group per
 // env) or Swarm<NT> (kb_swarm.cuh, a CTA per env) -- and reaches it through the members both define: L, bc,
 // lightState(), lightConst(l), ctrl(k), bodyXf(b), pos4(b), vel4(b), wake(b), bkind(b), hdr(i) and obsPos(b), the
 // position the task and the observations read.  Kilobot k is body L.M + k.  The caller picks the thread (single-thread
@@ -156,7 +156,7 @@ __device__ __forceinline__ void setKilobotActions(T& s, const double* action, in
 // runs a controller: KB_BODY_ABSENT needs no light and takes the default case)
 template <class T>
 __device__ __forceinline__ void senseControl(T& s, int first, int stride) {
-  const Layout& L = s.L;
+  const auto& L = s.L;
   const SF64Arr ls = s.lightState();
 #pragma unroll 1
   for (int k = first; k < L.N; k += stride) {
@@ -277,7 +277,7 @@ __device__ __forceinline__ int envSceneOf(T& s, const KernelArgs& a) {
 // scene (bodies L.M .. L.M + n - 1; in a batch of one size n == L.N).
 template <class T>
 __device__ __forceinline__ void taskError(T& s, const TaskConst& tk, const double* tgt, int n, double* dist, double* ang) {
-  const Layout& L = s.L;
+  const auto& L = s.L;
   double px, py, th = 0.0;
   if (tk.mode == KB_TASK_OBJECT_TO_TARGET) {
     const float2 x = s.obsPos(tk.object);
@@ -313,7 +313,7 @@ __device__ __forceinline__ void taskBegin(T& s, const KernelArgs& a, int env) {
 // get_state's light part (kilobots_env.py:115-118): the light state into the light and the flat observation
 template <class T>
 __device__ __forceinline__ void observeLights(T& s, const KernelArgs& a, int env, float* flat, int first, int stride) {
-  const Layout& L = s.L;
+  const auto& L = s.L;
   if (a.obsLight || flat) {
     const SF64Arr ls = s.lightState();
 #pragma unroll 1
@@ -362,7 +362,7 @@ __device__ __forceinline__ void taskEnd(T& s, const KernelArgs& a, int env) {
 // The kinds are read from the scene's body constants: a tier's own copy of them may not be written yet.
 template <class T>
 __device__ __forceinline__ void resetEnvLayer(T& s, const KernelArgs& a, int env, int envIn, int first, int stride) {
-  const Layout& L = s.L;
+  const auto& L = s.L;
   if (first == 0 && a.taskState && env < a.numEnvs) {
     double* ts = a.taskState + (size_t)env * KB_TASK_WORDS;
     ts[3 + KB_EP_RETURN] = 0.0;

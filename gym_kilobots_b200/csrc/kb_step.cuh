@@ -128,20 +128,32 @@ extern __shared__ __align__(16) uint32_t kb_smem[];
 #define KB_T(i) do { if (UNI && ((KB_SYNC_PHASES >> (i)) & 1u)) __syncthreads(); } while (0)
 #endif
 
-template <int LPE, bool UNI>
+// The layout a Sim reads its offsets, counts and constants from: the runtime Layout in the kernel parameters (held by
+// reference), or a compile-time layout -- an empty struct whose members are static constexpr copies of one batch's
+// Layout, generated by kb_create for the step kernel it compiles at run time (kb_jit.h).  Code reads s.L.x either way.
+template <class LT>
+struct LayoutHold {
+  typedef LT type;
+};
+template <>
+struct LayoutHold<Layout> {
+  typedef const Layout& type;
+};
+
+template <int LPE, bool UNI, class LT = Layout>
 struct Sim;
 // out-of-line (cold) paths: the Sim travels BY VALUE so that the caller's copy stays in registers
-template <int LPE, bool UNI> __device__ __noinline__ void warmStartGeneralNI(Sim<LPE, UNI> s, int q);
-template <int LPE, bool UNI> __device__ __noinline__ void solveVelocityGeneralNI(Sim<LPE, UNI> s, int q);
-template <int LPE, bool UNI> __device__ __noinline__ bool solvePositionGeneralNI(Sim<LPE, UNI> s, int q);
-template <int LPE, bool UNI> __device__ __noinline__ void initGeneralNI(Sim<LPE, UNI> s, int q, int ci, uint32_t item);
-template <int LPE, bool UNI> __device__ __noinline__ void storeGeneralNI(Sim<LPE, UNI> s, int q);
-template <int LPE, bool UNI> __device__ __noinline__ uint32_t solveTOINI(Sim<LPE, UNI> s);
+template <int LPE, bool UNI, class LT> __device__ __noinline__ void warmStartGeneralNI(Sim<LPE, UNI, LT> s, int q);
+template <int LPE, bool UNI, class LT> __device__ __noinline__ void solveVelocityGeneralNI(Sim<LPE, UNI, LT> s, int q);
+template <int LPE, bool UNI, class LT> __device__ __noinline__ bool solvePositionGeneralNI(Sim<LPE, UNI, LT> s, int q);
+template <int LPE, bool UNI, class LT> __device__ __noinline__ void initGeneralNI(Sim<LPE, UNI, LT> s, int q, int ci, uint32_t item);
+template <int LPE, bool UNI, class LT> __device__ __noinline__ void storeGeneralNI(Sim<LPE, UNI, LT> s, int q);
+template <int LPE, bool UNI, class LT> __device__ __noinline__ uint32_t solveTOINI(Sim<LPE, UNI, LT> s);
 
-template <int LPE, bool UNI>
+template <int LPE, bool UNI, class LT>
 struct Sim {
   Group<LPE, UNI> g;
-  const Layout& L;
+  typename LayoutHold<LT>::type L;
   uint32_t sa;                  // shared-window byte address of this env's shared-memory region
   float* blob;                  // this env's state blob in HBM
   const ProxyConst* px;         // scene proxies
@@ -156,7 +168,7 @@ struct Sim {
   unsigned long long* profOut;   // this env's row of the profile buffer (TOI internals add to slots 13..15 directly)
 #endif
 
-  __device__ __forceinline__ Sim(const Layout& l) : L(l) {
+  __device__ __forceinline__ Sim(const LT& l) : L(l) {
     nSub = nCon = nPts = nLvl = nPit = nToi = nTests = nIsl = 0u;
     genBase = nullptr;
 #ifdef KB_PROFILE
@@ -1829,19 +1841,19 @@ struct Sim {
   }
 };
 
-template <int LPE, bool UNI>
-__device__ __noinline__ void warmStartGeneralNI(Sim<LPE, UNI> s, int q) { s.warmStartGeneral(q); }
-template <int LPE, bool UNI>
-__device__ __noinline__ void solveVelocityGeneralNI(Sim<LPE, UNI> s, int q) { s.solveVelocityGeneral(q); }
-template <int LPE, bool UNI>
-__device__ __noinline__ bool solvePositionGeneralNI(Sim<LPE, UNI> s, int q) {
+template <int LPE, bool UNI, class LT>
+__device__ __noinline__ void warmStartGeneralNI(Sim<LPE, UNI, LT> s, int q) { s.warmStartGeneral(q); }
+template <int LPE, bool UNI, class LT>
+__device__ __noinline__ void solveVelocityGeneralNI(Sim<LPE, UNI, LT> s, int q) { s.solveVelocityGeneral(q); }
+template <int LPE, bool UNI, class LT>
+__device__ __noinline__ bool solvePositionGeneralNI(Sim<LPE, UNI, LT> s, int q) {
   return s.solvePositionGeneral(q, KB_BAUMGARTE, -3.0f * KB_LINEAR_SLOP, -1, -1);
 }
-template <int LPE, bool UNI>
-__device__ __noinline__ void initGeneralNI(Sim<LPE, UNI> s, int q, int ci, uint32_t item) {
+template <int LPE, bool UNI, class LT>
+__device__ __noinline__ void initGeneralNI(Sim<LPE, UNI, LT> s, int q, int ci, uint32_t item) {
   s.initGeneral(q, ci, IT_BA(item), IT_BB(item), (uint32_t)ci | ((uint32_t)IT_ISL(item) << 16), false);
 }
-template <int LPE, bool UNI>
-__device__ __noinline__ void storeGeneralNI(Sim<LPE, UNI> s, int q) { s.storeGeneral(q); }
+template <int LPE, bool UNI, class LT>
+__device__ __noinline__ void storeGeneralNI(Sim<LPE, UNI, LT> s, int q) { s.storeGeneral(q); }
 
 }  // namespace kb

@@ -471,16 +471,16 @@ __device__ __noinline__ float time_of_impact_edge_circle(const ProxyConst* shape
 }
 
 // ------------------------------------------------------------------------ b2World::SolveTOI
-template <int LPE, bool UNI>
-__device__ __noinline__ uint32_t solveTOINI(Sim<LPE, UNI> s) {
+template <int LPE, bool UNI, class LT>
+__device__ __noinline__ uint32_t solveTOINI(Sim<LPE, UNI, LT> s) {
   const uint32_t before = s.nToi;
   s.solveTOI();
   return s.nToi - before;
 }
 
 // (the caller has already established that at least one contact with the table exists)
-template <int LPE, bool UNI>
-__device__ __forceinline__ void Sim<LPE, UNI>::solveTOI() {
+template <int LPE, bool UNI, class LT>
+__device__ __forceinline__ void Sim<LPE, UNI, LT>::solveTOI() {
   const int B = L.B;
   int nC = (int)hdr(H_NC);
 

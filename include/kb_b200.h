@@ -24,7 +24,9 @@
 #ifndef KB_B200_H
 #define KB_B200_H
 
+#ifndef __CUDACC_RTC__   /* the library's run-time compiled step kernel includes this header too */
 #include <stdint.h>
+#endif
 
 #ifdef __cplusplus
 extern "C" {
@@ -317,8 +319,21 @@ typedef struct KbLaunchConfig {
   int32_t lanes_per_env, block_threads, grid_blocks, smem_bytes_per_block;
   int32_t state_words_per_env;   /* 32-bit words of per-env state resident in shared memory during a launch */
   int32_t smem_words_per_env;    /* state + solver scratch */
+  /* the lane-group step kernel compiled at kb_create for this batch's layout (offsets, counts and solver constants as
+   * immediates; same results as the generic kernel): 1 when it runs, 0 when the generic kb_step_kernel<LPE> runs.
+   * KB_JIT=0 asks for the generic kernel, KB_JIT=1 makes kb_create fail when the specialised one cannot be had;
+   * compiled kernels are cached under $KB_JIT_CACHE (default ~/.cache/gym_kilobots_b200). */
+  int32_t specialised;
+  float jit_ms;                  /* its compile time in kb_create, ms (0: taken from a cache) */
+  char jit_reason[256];          /* why the generic kernel runs ("" when specialised) */
 } KbLaunchConfig;
 int kb_get_launch_config(const KbHandle* h, KbLaunchConfig* cfg);
+/* Needs no GPU: the source kb_create generates for the specialised step kernel of a lane-group batch of `scenes`
+ * (the batch's layout as constants; the kernel's headers are embedded in the library) into source[source_cap].  With
+ * compile != 0 it also compiles it with NVRTC (no cache, nothing loaded) and writes NVRTC's log, ptxas's resource
+ * report included, into log[log_cap] and the compile time into *compile_ms.  KB_ERR_INVALID for a large-swarm batch. */
+int kb_jit_step_source(const KbSceneDesc* scenes, int32_t num_scenes, int32_t max_contacts, int32_t compile,
+                       char* source, int64_t source_cap, char* log, int64_t log_cap, double* compile_ms);
 /* derived mass data per scene: f32[num_scenes,B,4] = invMass invI localCenter.x localCenter.y */
 int kb_get_mass_data(KbHandle* h, float* out);
 
