@@ -165,6 +165,22 @@ class KbSampleSpec(C.Structure):
     ]
 
 
+# test-only geometry probe (include/kb_b200.h kb_probe_geometry)
+KB_PROBE_SHAPE, KB_PROBE_COLLIDE, KB_PROBE_DISTANCE, KB_PROBE_TOI = 0, 1, 2, 3
+KB_PROBE_OUT_WORDS = 40
+KB_PROBE_FIXTURE, KB_PROBE_EDGE = 0, 1
+
+
+class KbProbeShape(C.Structure):
+    _fields_ = [("kind", C.c_int32), ("edge", C.c_int32), ("wall_edges", C.c_int32), ("wall_x0", C.c_float),
+                ("wall_y0", C.c_float), ("wall_x1", C.c_float), ("wall_y1", C.c_float), ("fixture", KbFixtureDef)]
+
+
+class KbProbeCase(C.Structure):
+    _fields_ = [("a", C.c_int32), ("b", C.c_int32), ("fixed_rot_a", C.c_int32), ("fixed_rot_b", C.c_int32),
+                ("xf_a", C.c_float * 4), ("xf_b", C.c_float * 4), ("sweep_a", C.c_float * 8), ("sweep_b", C.c_float * 8)]
+
+
 # name -> (restype, argtypes); the exported symbol is prefix + name
 _VP = C.c_void_p
 PROTOTYPES = {
@@ -191,6 +207,7 @@ PROTOTYPES = {
     "bind_flat_observation": (C.c_int, [_VP, _VP]),
     "flat_observation_dim": (C.c_int, [_VP]),
     "render": (C.c_int, [_VP, _VP, C.c_int32, C.c_int32, C.c_int32, _VP, _VP]),
+    "probe_geometry": (C.c_int, [C.c_int32, C.c_int32, C.c_int32, _VP, C.c_int32, _VP, _VP]),
 }
 # exported by the product library only (the oracle has no state blob)
 class KbLaunchConfig(C.Structure):

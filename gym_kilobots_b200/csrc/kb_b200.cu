@@ -437,6 +437,45 @@ static int lightStateDim(int type) { return type == KB_LIGHT_MOMENTUM ? 4 : (typ
 static int lightActionDim(int type) { return type == KB_LIGHT_LINEAR ? 1 : 2; }
 static int round4(int x) { return (x + 3) & ~3; }
 
+// type, radius and geometry of a fixture's proxy
+static int buildFixtureShape(const KbFixtureDef& fd, ProxyConst* out) {
+  ProxyConst& pc = *out;
+  if (fd.shape == KB_SHAPE_CIRCLE) {
+    pc.type = SHAPE_CIRCLE;
+    pc.radius = fd.radius;
+  } else if (fd.shape == KB_SHAPE_BOX) {
+    pc.type = SHAPE_POLYGON;
+    pc.radius = 2.0f * 0.005f;
+    buildBox(fd.hx, fd.hy, &pc);
+  } else if (fd.shape == KB_SHAPE_POLYGON) {
+    pc.type = SHAPE_POLYGON;
+    pc.radius = 2.0f * 0.005f;
+    if (!buildPolygon(fd, &pc)) return fail(KB_ERR_INVALID, "degenerate polygon fixture");
+  } else {
+    return fail(KB_ERR_INVALID, "unknown fixture shape");
+  }
+  return KB_OK;
+}
+
+// child i of the table chain, kilobots_env.py:46-51: (x0,y1) -> (x0,y0) -> (x1,y0) -> (x1,y1) [-> (x0,y1)], with the ghost
+// vertices of b2ChainShape::GetChildEdge.  pc is zeroed; body and friction are the caller's.
+static void buildChainEdge(const KbSceneDesc& sd, int i, ProxyConst* out) {
+  const float vx[5] = {sd.wall_x0, sd.wall_x0, sd.wall_x1, sd.wall_x1, sd.wall_x0};
+  const float vy[5] = {sd.wall_y1, sd.wall_y0, sd.wall_y0, sd.wall_y1, sd.wall_y1};
+  const bool loop = sd.wall_edges == 4;
+  const int count = loop ? 5 : 4;
+  ProxyConst& pc = *out;
+  pc.type = SHAPE_EDGE;
+  pc.radius = 2.0f * 0.005f;
+  pc.restitution = 0.0f;
+  pc.vx[1] = vx[i]; pc.vy[1] = vy[i];
+  pc.vx[2] = vx[i + 1]; pc.vy[2] = vy[i + 1];
+  if (i > 0) { pc.vx[0] = vx[i - 1]; pc.vy[0] = vy[i - 1]; pc.has0 = 1; }
+  else if (loop) { pc.vx[0] = vx[count - 2]; pc.vy[0] = vy[count - 2]; pc.has0 = 1; }
+  if (i < count - 2) { pc.vx[3] = vx[i + 2]; pc.vy[3] = vy[i + 2]; pc.has3 = 1; }
+  else if (loop) { pc.vx[3] = vx[1]; pc.vy[3] = vy[1]; pc.has3 = 1; }
+}
+
 // The scene's bodies in the batch's padded layout: object j at body index j, kilobot k at Mmax + k; the other indices
 // up to B = Bp - 1 are absent bodies (kind KB_BODY_ABSENT, no proxy, zero mass data).  Proxies are numbered as in a
 // compact world of the scene's own bodies: the table edges, then the fixtures of the present bodies in body order.
@@ -448,27 +487,12 @@ static int buildScene(const KbSceneDesc& sd, int Mmax, int Bp, int Pp, std::vect
   std::memset(proxies->data(), 0, sizeof(ProxyConst) * Pp);
   std::memset(bodies->data(), 0, sizeof(BodyConst) * Bp);
   int p = 0;
-  // table chain, kilobots_env.py:46-51: (x0,y1) -> (x0,y0) -> (x1,y0) -> (x1,y1) [-> (x0,y1)]
   if (sd.wall_edges != 0 && sd.wall_edges != 3 && sd.wall_edges != 4) return fail(KB_ERR_INVALID, "wall_edges must be 0, 3 or 4");
-  {
-    const float vx[5] = {sd.wall_x0, sd.wall_x0, sd.wall_x1, sd.wall_x1, sd.wall_x0};
-    const float vy[5] = {sd.wall_y1, sd.wall_y0, sd.wall_y0, sd.wall_y1, sd.wall_y1};
-    const bool loop = sd.wall_edges == 4;
-    const int count = loop ? 5 : 4;
-    for (int i = 0; i < sd.wall_edges; ++i) {
-      ProxyConst& pc = (*proxies)[p++];
-      pc.body = B;  // static slot
-      pc.type = SHAPE_EDGE;
-      pc.radius = 2.0f * 0.005f;
-      pc.friction = sd.wall_friction;
-      pc.restitution = 0.0f;
-      pc.vx[1] = vx[i]; pc.vy[1] = vy[i];
-      pc.vx[2] = vx[i + 1]; pc.vy[2] = vy[i + 1];
-      if (i > 0) { pc.vx[0] = vx[i - 1]; pc.vy[0] = vy[i - 1]; pc.has0 = 1; }
-      else if (loop) { pc.vx[0] = vx[count - 2]; pc.vy[0] = vy[count - 2]; pc.has0 = 1; }
-      if (i < count - 2) { pc.vx[3] = vx[i + 2]; pc.vy[3] = vy[i + 2]; pc.has3 = 1; }
-      else if (loop) { pc.vx[3] = vx[1]; pc.vy[3] = vy[1]; pc.has3 = 1; }
-    }
+  for (int i = 0; i < sd.wall_edges; ++i) {
+    ProxyConst& pc = (*proxies)[p++];
+    pc.body = B;  // static slot
+    pc.friction = sd.wall_friction;
+    buildChainEdge(sd, i, &pc);
   }
   for (int b = 0; b < B; ++b) (*bodies)[b].kind = KB_BODY_ABSENT;
   for (int be = 0; be < sd.num_bodies; ++be) {
@@ -490,20 +514,8 @@ static int buildScene(const KbSceneDesc& sd, int Mmax, int Bp, int Pp, std::vect
       pc.body = b;
       pc.friction = fd.friction;
       pc.restitution = fd.restitution;
-      if (fd.shape == KB_SHAPE_CIRCLE) {
-        pc.type = SHAPE_CIRCLE;
-        pc.radius = fd.radius;
-      } else if (fd.shape == KB_SHAPE_BOX) {
-        pc.type = SHAPE_POLYGON;
-        pc.radius = 2.0f * 0.005f;
-        buildBox(fd.hx, fd.hy, &pc);
-      } else if (fd.shape == KB_SHAPE_POLYGON) {
-        pc.type = SHAPE_POLYGON;
-        pc.radius = 2.0f * 0.005f;
-        if (!buildPolygon(fd, &pc)) return fail(KB_ERR_INVALID, "degenerate polygon fixture");
-      } else {
-        return fail(KB_ERR_INVALID, "unknown fixture shape");
-      }
+      const int rc = buildFixtureShape(fd, &pc);
+      if (rc != KB_OK) return rc;
     }
     // b2Body::ResetMassData: fixtures are visited newest first (m_fixtureList is LIFO)
     float mass = 0.0f, I = 0.0f;
@@ -1903,6 +1915,86 @@ int kb_selftest_exact_math(int32_t device, int32_t div_rounds_log2, uint64_t* mi
   CUDA_TRY(cudaDeviceSynchronize());
   CUDA_TRY(cudaMemcpy(mismatches, d, 6 * sizeof(unsigned long long), cudaMemcpyDeviceToHost));
   CUDA_TRY(cudaFree(d));
+  return KB_OK;
+}
+
+// ---- geometry probe (kb_narrow.cuh, kb_toi.cuh one case at a time; the kernel is in kb_probe.cu) -------------------
+}  // extern "C"
+cudaError_t kbLaunchProbeGeometry(int op, int n, const void* px, const KbProbeCase* cases, uint32_t* out);
+extern "C" {
+int kb_probe_geometry(int32_t device, int32_t op, int32_t n, const KbProbeShape* shapes, int32_t num_shapes,
+                      const KbProbeCase* cases, uint32_t* out) {
+  using namespace kb;
+  if (!shapes || num_shapes < 1 || !out || op < KB_PROBE_SHAPE || op > KB_PROBE_TOI || (op != KB_PROBE_SHAPE && (!cases || n < 0)))
+    return fail(KB_ERR_INVALID, "kb_probe_geometry: invalid arguments");
+  std::vector<ProxyConst> px((size_t)num_shapes);
+  std::memset(px.data(), 0, sizeof(ProxyConst) * px.size());
+  for (int s = 0; s < num_shapes; ++s) {
+    const KbProbeShape& ps = shapes[s];
+    if (ps.kind == KB_PROBE_EDGE) {
+      if ((ps.wall_edges != 3 && ps.wall_edges != 4) || ps.edge < 0 || ps.edge >= ps.wall_edges)
+        return fail(KB_ERR_INVALID, "kb_probe_geometry: bad chain edge");
+      KbSceneDesc sd;
+      std::memset(&sd, 0, sizeof(sd));
+      sd.wall_x0 = ps.wall_x0; sd.wall_y0 = ps.wall_y0; sd.wall_x1 = ps.wall_x1; sd.wall_y1 = ps.wall_y1;
+      sd.wall_edges = ps.wall_edges;
+      buildChainEdge(sd, ps.edge, &px[s]);
+    } else {
+      const int rc = buildFixtureShape(ps.fixture, &px[s]);
+      if (rc != KB_OK) return rc;
+    }
+  }
+  if (op == KB_PROBE_SHAPE) {
+    for (int s = 0; s < num_shapes; ++s) {
+      const ProxyConst& pc = px[s];
+      uint32_t* o = out + (size_t)s * KB_PROBE_OUT_WORDS;
+      std::memset(o, 0, KB_PROBE_OUT_WORDS * 4);
+      const float head[6] = {0.0f, pc.radius, 0.0f, 0.0f, pc.cx, pc.cy};
+      std::memcpy(o, head, sizeof(head));
+      o[0] = (uint32_t)(pc.type == SHAPE_EDGE ? 2 : (pc.type == SHAPE_CIRCLE ? 1 : pc.count));
+      o[2] = (uint32_t)pc.has0;
+      o[3] = (uint32_t)pc.has3;
+      std::memcpy(o + 6, pc.vx, 4 * KB_MAX_POLY_VERTS);
+      std::memcpy(o + 14, pc.vy, 4 * KB_MAX_POLY_VERTS);
+      std::memcpy(o + 22, pc.nx, 4 * KB_MAX_POLY_VERTS);
+      std::memcpy(o + 30, pc.ny, 4 * KB_MAX_POLY_VERTS);
+    }
+    return KB_OK;
+  }
+  for (int i = 0; i < n; ++i) {
+    if (cases[i].a < 0 || cases[i].a >= num_shapes || cases[i].b < 0 || cases[i].b >= num_shapes)
+      return fail(KB_ERR_INVALID, "kb_probe_geometry: shape index out of range");
+    // the pairs the contact register forms (Sim::evaluate): A a circle only against a circle, B never an edge
+    const int tA = px[cases[i].a].type, tB = px[cases[i].b].type;
+    if (op == KB_PROBE_COLLIDE && (tB == SHAPE_EDGE || (tA == SHAPE_CIRCLE && tB != SHAPE_CIRCLE)))
+      return fail(KB_ERR_INVALID, "kb_probe_geometry: no narrowphase routine for this pair of shapes");
+  }
+  if (n == 0) return KB_OK;
+  int count = 0;
+  if (cudaGetDeviceCount(&count) != cudaSuccess || count < 1) {
+    cudaGetLastError();
+    return fail(KB_ERR_NO_DEVICE, "kb_probe_geometry: no CUDA device");
+  }
+  if (device >= 0) CUDA_TRY(cudaSetDevice(device));
+  ProxyConst* dPx = nullptr;
+  KbProbeCase* dCases = nullptr;
+  uint32_t* dOut = nullptr;
+  const size_t outBytes = (size_t)n * KB_PROBE_OUT_WORDS * 4;
+  cudaError_t e = cudaMalloc(&dPx, sizeof(ProxyConst) * px.size());
+  if (e == cudaSuccess) e = cudaMalloc(&dCases, sizeof(KbProbeCase) * (size_t)n);
+  if (e == cudaSuccess) e = cudaMalloc(&dOut, outBytes);
+  if (e == cudaSuccess) e = cudaMemcpy(dPx, px.data(), sizeof(ProxyConst) * px.size(), cudaMemcpyHostToDevice);
+  if (e == cudaSuccess) e = cudaMemcpy(dCases, cases, sizeof(KbProbeCase) * (size_t)n, cudaMemcpyHostToDevice);
+  if (e == cudaSuccess) e = cudaMemset(dOut, 0, outBytes);
+  if (e == cudaSuccess) {
+    e = kbLaunchProbeGeometry(op, n, dPx, dCases, dOut);
+  }
+  if (e == cudaSuccess) e = cudaDeviceSynchronize();
+  if (e == cudaSuccess) e = cudaMemcpy(out, dOut, outBytes, cudaMemcpyDeviceToHost);
+  cudaFree(dPx);
+  cudaFree(dCases);
+  cudaFree(dOut);
+  if (e != cudaSuccess) return fail(KB_ERR_CUDA, std::string("kb_probe_geometry: ") + cudaGetErrorString(e));
   return KB_OK;
 }
 

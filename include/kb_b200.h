@@ -436,6 +436,44 @@ int kb_render(KbHandle* h, const int32_t* env_ids, int32_t num_images, int32_t w
  * needs entries 0, 1, 2 and 4 to be 0.  device < 0: the current device. */
 int kb_selftest_exact_math(int32_t device, int32_t div_rounds_log2, uint64_t* mismatches);
 
+/* Test-only probe of the narrowphase, distance and time-of-impact routines, one case per thread (no reference
+ * counterpart; kbo_probe_geometry runs the oracle's routines on the same layout).  A shape is a fixture built the way
+ * kb_create builds it, or child `edge` of the table chain of a scene with the given wall fields.  Every output row has
+ * KB_PROBE_OUT_WORDS 32-bit words (floats as their bit patterns):
+ *   KB_PROBE_SHAPE    (host only, needs no GPU; one row per shape, `cases` unused) count, radius, has0, has3, cx, cy,
+ *                     vx[8], vy[8], nx[8], ny[8] (an edge: count 2 and v0..v3 in vx/vy[0..3])
+ *   KB_PROBE_COLLIDE  the manifold of the pair (a, b) at xf_a / xf_b, dispatched as the step kernels do:
+ *                     type, pointCount, localNormal.xy, localPoint.xy, then per point x, y, id
+ *   KB_PROBE_DISTANCE b2Distance of the core shapes (fresh simplex cache) at xf_a / xf_b: distance, simplex count
+ *   KB_PROBE_TOI      b2TimeOfImpact (tMax = 1) over sweep_a / sweep_b with the flags fixed_rot_*: t if touching, else a
+ *                     negative value; then, for an edge against a circle, the edge-circle specialisation's result (else
+ *                     0); then the generic result with both fixed_rot flags cleared.  The oracle has no fixed_rot
+ *                     shortcut: it always rotates, and writes its TOIOutput state into word 3.
+ * xf = p.x p.y q.s q.c; sweep = localCenter.xy c0.xy c.xy a0 a.  shapes / cases / out are host arrays; device < 0: the
+ * current device. */
+#define KB_PROBE_SHAPE 0
+#define KB_PROBE_COLLIDE 1
+#define KB_PROBE_DISTANCE 2
+#define KB_PROBE_TOI 3
+#define KB_PROBE_OUT_WORDS 40
+#define KB_PROBE_FIXTURE 0
+#define KB_PROBE_EDGE 1
+typedef struct KbProbeShape {
+  int32_t kind;        /* KB_PROBE_FIXTURE | KB_PROBE_EDGE */
+  int32_t edge;        /* KB_PROBE_EDGE: child index of the chain */
+  int32_t wall_edges;  /* KB_PROBE_EDGE: 3 (open chain) or 4 (closed loop), as KbSceneDesc */
+  float wall_x0, wall_y0, wall_x1, wall_y1;
+  KbFixtureDef fixture;  /* KB_PROBE_FIXTURE */
+} KbProbeShape;
+typedef struct KbProbeCase {
+  int32_t a, b;        /* indices into shapes */
+  int32_t fixed_rot_a, fixed_rot_b;
+  float xf_a[4], xf_b[4];
+  float sweep_a[8], sweep_b[8];
+} KbProbeCase;
+int kb_probe_geometry(int32_t device, int32_t op, int32_t n, const KbProbeShape* shapes, int32_t num_shapes,
+                      const KbProbeCase* cases, uint32_t* out);
+
 #ifdef __cplusplus
 }
 #endif

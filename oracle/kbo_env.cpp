@@ -1027,4 +1027,135 @@ void kbo_sensor_pos(double x, double y, double angle, double* out) {
   out[1] = (double)wp.y / 25.0;
 }
 
+// Test-only probe of the narrowphase, distance and TOI routines (include/kb_b200.h kb_probe_geometry): the same layout,
+// with the oracle's own shape code and the dispatch of Contact::Evaluate.
+int kbo_probe_geometry(int32_t device, int32_t op, int32_t n, const KbProbeShape* shapes, int32_t num_shapes,
+                       const KbProbeCase* cases, uint32_t* out) {
+  (void)device;
+  if (!shapes || num_shapes < 1 || !out || op < KB_PROBE_SHAPE || op > KB_PROBE_TOI || (op != KB_PROBE_SHAPE && (!cases || n < 0))) {
+    g_err = "kbo_probe_geometry: invalid arguments";
+    return KB_ERR_INVALID;
+  }
+  std::vector<Shape> sh((size_t)num_shapes);
+  for (int s = 0; s < num_shapes; ++s) {
+    const KbProbeShape& ps = shapes[s];
+    if (ps.kind == KB_PROBE_EDGE) {
+      if ((ps.wall_edges != 3 && ps.wall_edges != 4) || ps.edge < 0 || ps.edge >= ps.wall_edges) {
+        g_err = "kbo_probe_geometry: bad chain edge";
+        return KB_ERR_INVALID;
+      }
+      sh[s] = MakeChainEdge(ps.wall_x0, ps.wall_y0, ps.wall_x1, ps.wall_y1, ps.wall_edges, ps.edge);
+    } else {
+      sh[s] = MakeShape(ps.fixture);
+    }
+  }
+  auto f2u = [](float f) {
+    uint32_t u;
+    std::memcpy(&u, &f, 4);
+    return u;
+  };
+  if (op == KB_PROBE_SHAPE) {
+    for (int s = 0; s < num_shapes; ++s) {
+      const Shape& x = sh[s];
+      uint32_t* o = out + (size_t)s * KB_PROBE_OUT_WORDS;
+      std::memset(o, 0, KB_PROBE_OUT_WORDS * 4);
+      o[0] = (uint32_t)(x.type == kEdge ? 2 : (x.type == kCircle ? 1 : x.count));
+      o[1] = f2u(x.radius);
+      o[2] = x.type == kEdge ? (uint32_t)x.hasVertex0 : 0u;
+      o[3] = x.type == kEdge ? (uint32_t)x.hasVertex3 : 0u;
+      if (x.type == kPolygon) {
+        o[4] = f2u(x.centroid.x);
+        o[5] = f2u(x.centroid.y);
+        for (int i = 0; i < x.count; ++i) {
+          o[6 + i] = f2u(x.vertices[i].x);
+          o[14 + i] = f2u(x.vertices[i].y);
+          o[22 + i] = f2u(x.normals[i].x);
+          o[30 + i] = f2u(x.normals[i].y);
+        }
+      } else if (x.type == kEdge) {
+        const Vec2 v[4] = {x.v0, x.v1, x.v2, x.v3};
+        for (int i = 0; i < 4; ++i) {
+          o[6 + i] = f2u(v[i].x);
+          o[14 + i] = f2u(v[i].y);
+        }
+      }
+    }
+    return KB_OK;
+  }
+  for (int i = 0; i < n; ++i) {
+    const KbProbeCase& c = cases[i];
+    if (c.a < 0 || c.a >= num_shapes || c.b < 0 || c.b >= num_shapes) {
+      g_err = "kbo_probe_geometry: shape index out of range";
+      return KB_ERR_INVALID;
+    }
+    // the pairs the contact register forms (Contact::Evaluate): A a circle only against a circle, B never an edge
+    const int tA = sh[c.a].type, tB = sh[c.b].type;
+    if (op == KB_PROBE_COLLIDE && (tB == kEdge || (tA == kCircle && tB != kCircle))) {
+      g_err = "kbo_probe_geometry: no narrowphase routine for this pair of shapes";
+      return KB_ERR_INVALID;
+    }
+  }
+  for (int i = 0; i < n; ++i) {
+    const KbProbeCase& c = cases[i];
+    const Shape* sA = &sh[c.a];
+    const Shape* sB = &sh[c.b];
+    uint32_t* o = out + (size_t)i * KB_PROBE_OUT_WORDS;
+    std::memset(o, 0, KB_PROBE_OUT_WORDS * 4);
+    Xf xfA, xfB;
+    xfA.p.Set(c.xf_a[0], c.xf_a[1]);
+    xfA.q.s = c.xf_a[2];
+    xfA.q.c = c.xf_a[3];
+    xfB.p.Set(c.xf_b[0], c.xf_b[1]);
+    xfB.q.s = c.xf_b[2];
+    xfB.q.c = c.xf_b[3];
+    if (op == KB_PROBE_COLLIDE) {
+      Manifold m;
+      if (sA->type == kCircle && sB->type == kCircle) CollideCircles(&m, sA, xfA, sB, xfB);
+      else if (sA->type == kPolygon && sB->type == kCircle) CollidePolygonAndCircle(&m, sA, xfA, sB, xfB);
+      else if (sA->type == kPolygon && sB->type == kPolygon) CollidePolygons(&m, sA, xfA, sB, xfB);
+      else if (sA->type == kEdge && sB->type == kCircle) CollideEdgeAndCircle(&m, sA, xfA, sB, xfB);
+      else if (sA->type == kEdge && sB->type == kPolygon) CollideEdgeAndPolygon(&m, sA, xfA, sB, xfB);
+      else m.pointCount = 0;
+      o[0] = (uint32_t)m.type;
+      o[1] = (uint32_t)m.pointCount;
+      o[2] = f2u(m.localNormal.x);
+      o[3] = f2u(m.localNormal.y);
+      o[4] = f2u(m.localPoint.x);
+      o[5] = f2u(m.localPoint.y);
+      for (int k = 0; k < 2; ++k) {
+        o[6 + 3 * k] = f2u(m.points[k].localPoint.x);
+        o[7 + 3 * k] = f2u(m.points[k].localPoint.y);
+        o[8 + 3 * k] = m.points[k].id.key;
+      }
+    } else if (op == KB_PROBE_DISTANCE) {
+      int count = 0;
+      o[0] = f2u(DistanceCore(sA, xfA, sB, xfB, &count));
+      o[1] = (uint32_t)count;
+    } else {
+      TOIInput in;
+      in.shapeA = sA;
+      in.shapeB = sB;
+      const float* w[2] = {c.sweep_a, c.sweep_b};
+      Sweep* sw[2] = {&in.sweepA, &in.sweepB};
+      for (int k = 0; k < 2; ++k) {
+        sw[k]->localCenter.Set(w[k][0], w[k][1]);
+        sw[k]->c0.Set(w[k][2], w[k][3]);
+        sw[k]->c.Set(w[k][4], w[k][5]);
+        sw[k]->a0 = w[k][6];
+        sw[k]->a = w[k][7];
+        sw[k]->alpha0 = 0.0f;
+      }
+      in.tMax = 1.0f;
+      TOIOutput res;
+      TimeOfImpact(&res, &in);
+      const float t = res.state == TOIOutput::kTouching ? res.t : -1.0f;
+      o[0] = f2u(t);
+      o[1] = (sA->type == kEdge && sB->type == kCircle) ? f2u(t) : 0u;
+      o[2] = f2u(t);
+      o[3] = (uint32_t)res.state;
+    }
+  }
+  return KB_OK;
+}
+
 }  // extern "C"

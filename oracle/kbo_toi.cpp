@@ -427,6 +427,18 @@ struct SeparationFunction {
 
 }  // namespace
 
+float DistanceCore(const Shape* shapeA, const Xf& xfA, const Shape* shapeB, const Xf& xfB, int* simplexCount) {
+  DistanceProxy proxyA, proxyB;
+  proxyA.Set(shapeA);
+  proxyB.Set(shapeB);
+  SimplexCache cache;
+  cache.metric = 0.0f;
+  cache.count = 0;
+  const float d = Distance(&cache, &proxyA, xfA, &proxyB, xfB);
+  *simplexCount = cache.count;
+  return d;
+}
+
 void TimeOfImpact(TOIOutput* output, const TOIInput* input) {
   output->state = TOIOutput::kUnknown;
   output->t = input->tMax;

@@ -150,9 +150,35 @@ World::~World() {
   delete table;
 }
 
-// Static table + chain shape, kilobots_env.py:46-51.  One proxy per chain child, created first so
-// the table's proxy ids are the lowest.  edges == 3: open chain (b2ChainShape::CreateChain, no
-// ghost vertices at the ends); edges == 4: closed loop (CreateLoop).
+// Child i of the table's chain shape, kilobots_env.py:46-51 (b2ChainShape::GetChildEdge).  edges == 3: open chain
+// (b2ChainShape::CreateChain, no ghost vertices at the ends); edges == 4: closed loop (CreateLoop).
+Shape MakeChainEdge(float x0, float y0, float x1, float y1, int edges, int i) {
+  Vec2 v[5] = {Vec2(x0, y1), Vec2(x0, y0), Vec2(x1, y0), Vec2(x1, y1), Vec2(x0, y1)};
+  const int count = edges == 4 ? 5 : 4;  // b2ChainShape::m_count
+  const bool loop = edges == 4;
+  Shape s;
+  s.type = kEdge;
+  s.radius = kPolygonRadius;
+  s.v1 = v[i];
+  s.v2 = v[i + 1];
+  if (i > 0) {
+    s.v0 = v[i - 1];
+    s.hasVertex0 = true;
+  } else {
+    s.v0 = loop ? v[count - 2] : Vec2(0.0f, 0.0f);
+    s.hasVertex0 = loop;
+  }
+  if (i < count - 2) {
+    s.v3 = v[i + 2];
+    s.hasVertex3 = true;
+  } else {
+    s.v3 = loop ? v[1] : Vec2(0.0f, 0.0f);
+    s.hasVertex3 = loop;
+  }
+  return s;
+}
+
+// Static table + chain shape.  One proxy per chain child, created first so the table's proxy ids are the lowest.
 void World::CreateTable(float x0, float y0, float x1, float y1, int edges, float friction) {
   table = new Body();
   table->isStatic = true;
@@ -160,29 +186,8 @@ void World::CreateTable(float x0, float y0, float x1, float y1, int edges, float
   table->xf.q.Set(0.0f);
   table->index = -1;
   if (edges <= 0) return;
-  Vec2 v[5] = {Vec2(x0, y1), Vec2(x0, y0), Vec2(x1, y0), Vec2(x1, y1), Vec2(x0, y1)};
-  const int count = edges == 4 ? 5 : 4;  // b2ChainShape::m_count
-  const bool loop = edges == 4;
-  for (int i = 0; i < count - 1; ++i) {
-    Shape s;
-    s.type = kEdge;
-    s.radius = kPolygonRadius;
-    s.v1 = v[i];
-    s.v2 = v[i + 1];
-    if (i > 0) {
-      s.v0 = v[i - 1];
-      s.hasVertex0 = true;
-    } else {
-      s.v0 = loop ? v[count - 2] : Vec2(0.0f, 0.0f);
-      s.hasVertex0 = loop;
-    }
-    if (i < count - 2) {
-      s.v3 = v[i + 2];
-      s.hasVertex3 = true;
-    } else {
-      s.v3 = loop ? v[1] : Vec2(0.0f, 0.0f);
-      s.hasVertex3 = loop;
-    }
+  for (int i = 0; i < edges; ++i) {
+    Shape s = MakeChainEdge(x0, y0, x1, y1, edges, i);
     Fixture* f = new Fixture();
     f->shape = s;
     f->body = table;

@@ -196,6 +196,11 @@ struct TOIOutput {
   float t;
 };
 void TimeOfImpact(TOIOutput* out, const TOIInput* in);
+// b2Distance (useRadii = false) of the core shapes with a fresh simplex cache; *simplexCount = the cache's count
+float DistanceCore(const Shape* shapeA, const Xf& xfA, const Shape* shapeB, const Xf& xfB, int* simplexCount);
+
+// child i of the table chain (kbo_world.cpp)
+Shape MakeChainEdge(float x0, float y0, float x1, float y1, int edges, int i);
 
 // contact solver over an island (kbo_solver.cpp)
 struct Position { Vec2 c; float a; };
