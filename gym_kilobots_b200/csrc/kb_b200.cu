@@ -14,7 +14,9 @@
 #include <cstdlib>
 #include <cstring>
 #include <limits>
+#include <memory>
 #include <string>
+#include <type_traits>
 #include <vector>
 
 #include "kb_step_kernel.cuh"
@@ -206,6 +208,40 @@ __global__ void __launch_bounds__(1024) kb_reduce_stats_kernel(const double* tas
 }
 
 // ------------------------------------------------------------------------------- host state
+// Owners of device allocations, streams and events.  An empty owner releases nothing, so a Handle that owns nothing
+// (kb_jit_step_source's) is destroyed without a call into the CUDA runtime.
+struct CudaRelease {
+  void operator()(void* p) const { cudaFree(p); }
+  void operator()(cudaStream_t s) const { cudaStreamDestroy(s); }
+  void operator()(cudaEvent_t e) const { cudaEventDestroy(e); }
+};
+template <class T>
+using DevBuf = std::unique_ptr<T, CudaRelease>;
+using Stream = std::unique_ptr<std::remove_pointer_t<cudaStream_t>, CudaRelease>;
+using Event = std::unique_ptr<std::remove_pointer_t<cudaEvent_t>, CudaRelease>;
+
+// frees what `p` holds, then allocates `count` elements into it
+template <class T>
+static cudaError_t devAlloc(DevBuf<T>& p, size_t count) {
+  p.reset();
+  T* q = nullptr;
+  const cudaError_t e = cudaMalloc(&q, sizeof(T) * count);
+  if (e == cudaSuccess) p.reset(q);
+  return e;
+}
+static cudaError_t create(Stream& s) {
+  cudaStream_t q = nullptr;
+  const cudaError_t e = cudaStreamCreateWithFlags(&q, cudaStreamNonBlocking);
+  if (e == cudaSuccess) s.reset(q);
+  return e;
+}
+static cudaError_t create(Event& ev) {
+  cudaEvent_t q = nullptr;
+  const cudaError_t e = cudaEventCreateWithFlags(&q, cudaEventDisableTiming);
+  if (e == cudaSuccess) ev.reset(q);
+  return e;
+}
+
 struct Handle {
   int device = 0;
   int numEnvs = 0, numScenes = 0;
@@ -213,55 +249,95 @@ struct Handle {
   std::vector<std::vector<BodyConst>> hostBodies;  // per scene
   std::vector<int> hostNumProxies;                  // per scene
   std::vector<int> hostNumObjects, hostNumKilobots; // per scene (L.M / L.N are the maxima over the scenes)
-  float* dBlobs = nullptr;
-  int32_t* dEnvScene = nullptr;
-  ProxyConst* dProxies = nullptr;
-  BodyConst* dBodies = nullptr;
-  SceneConst* dScenes = nullptr;
-  LightConst* dLights = nullptr;
+  DevBuf<float> dBlobs;
+  DevBuf<int32_t> dEnvScene;
+  DevBuf<ProxyConst> dProxies;
+  DevBuf<BodyConst> dBodies;
+  DevBuf<SceneConst> dScenes;
+  DevBuf<LightConst> dLights;
   // staging for kb_step_host
-  double* dAction = nullptr;
+  DevBuf<double> dAction;
   // kb_step_host staging: ONE device allocation, sections at hostOff[] (see kb_get_host_layout)
-  uint8_t* dOut = nullptr;
+  DevBuf<uint8_t> dOut;
   int64_t hostOff[6] = {0, 0, 0, 0, 0, 0}, hostTotal = 0;
   float *dObsK = nullptr, *dObsO = nullptr, *dReward = nullptr;
   double* dObsL = nullptr;
   uint8_t* dDone = nullptr;
   int32_t* dStatus = nullptr;
   float wall[4] = {0.0f, 0.0f, 0.0f, 0.0f};   // table rectangle x0 y0 x1 y1, b2 units (render window)
-  int32_t* dRenderIds = nullptr;
+  DevBuf<int32_t> dRenderIds;
   int renderIdsCap = 0;
   // task layer (extension)
   TaskConst task = {};
-  double* dTask = nullptr;   // [E][KB_TASK_WORDS]
+  DevBuf<double> dTask;      // [E][KB_TASK_WORDS]
   float* obsFlat = nullptr;  // caller-owned device buffer bound by kb_bind_flat_observation
   int envsPerBlock = 4;
   size_t smemBytes = 0;
   SwarmLayout W = {};          // W.enabled: the large-swarm tier (kb_swarm.cuh) runs this batch
-  // kb_step_host pipeline: chunks of the batch alternate between two side streams, so that the device->host copy of
-  // one chunk overlaps the kernel of the next
   // on-device scene sampling at reset (kb_sample.cuh)
-  SamplerConst* dSampler = nullptr;             // [KB_SAMPLE_MAX_CONFIGS], numConfigs of them set
-  double *dSamplePose = nullptr, *dSampleLight = nullptr;
-  uint32_t* dEpisode = nullptr;
+  DevBuf<SamplerConst> dSampler;                 // [KB_SAMPLE_MAX_CONFIGS], numConfigs of them set
+  DevBuf<double> dSamplePose, dSampleLight;
+  DevBuf<uint32_t> dEpisode;
   int numConfigs = 0;
   std::vector<int> hostSceneConfig;              // configuration of each scene (-1 = none)
-  int32_t* dSceneConfig = nullptr;               // [numScenes]
-  double* dConfigCdf = nullptr;                  // [KB_SAMPLE_MAX_CONFIGS]
+  DevBuf<int32_t> dSceneConfig;                  // [numScenes]
+  DevBuf<double> dConfigCdf;                     // [KB_SAMPLE_MAX_CONFIGS]
   bool weighted = false;
-  cudaStream_t pipe[2] = {nullptr, nullptr};
-  cudaEvent_t evFork = nullptr, evJoin[2] = {nullptr, nullptr};
+  // kb_step_host pipeline: chunks of the batch alternate between two side streams, so that the device->host copy of
+  // one chunk overlaps the kernel of the next
+  Stream pipe[2];
+  Event evFork, evJoin[2];
   int hostChunks = 1;
   // the step kernel compiled for this batch's layout (kb_jit.h); null: the generic kb_step_kernel<LPE> runs
   cudaKernel_t stepJit = nullptr;
   float jitMs = 0.0f;          // its compile time in kb_create (0: from a cache)
   std::string jitReason;       // why the generic kernel runs instead
 #ifdef KB_PROFILE
-  unsigned long long* dProf = nullptr;
+  DevBuf<unsigned long long> dProf;
 #endif
 };
 
 static int launchGrid(const Handle* h) { return (h->numEnvs + h->envsPerBlock - 1) / h->envsPerBlock; }
+static int blockThreads(const Handle* h) { return h->W.enabled ? h->L.lanesPerEnv : KB_BLOCK_OF(h->L.lanesPerEnv); }
+
+// The kernel widths the library is built with: lanes per env of the lane-group tier, threads per CTA of the
+// large-swarm tier.  Each width is one instance of every kernel of its tier.
+template <bool Swarm, int... Width>
+struct Tier {
+  static bool has(int w) { return ((w == Width) || ...); }
+};
+using LaneGroupTier = Tier<false, 4, 8, 16, 32>;
+using SwarmTier = Tier<true, 128, 256, 512>;
+
+template <class F, bool Swarm, int... Width>
+static void dispatchWidth(Tier<Swarm, Width...>, int w, F& f) {
+  (void)((w == Width && (f(std::bool_constant<Swarm>(), std::integral_constant<int, Width>()), true)) || ...);
+}
+
+// Calls f(swarm, width) with the batch's tier and kernel width as compile-time constants.
+template <class F>
+static void withTierWidth(const Handle* h, F&& f) {
+  if (h->W.enabled)
+    dispatchWidth(SwarmTier(), h->L.lanesPerEnv, f);
+  else
+    dispatchWidth(LaneGroupTier(), h->L.lanesPerEnv, f);
+}
+
+// the generic step, reset and set-pose kernels of the batch's tier and width
+struct TierKernels {
+  const void *step = nullptr, *reset = nullptr, *setpose = nullptr;
+};
+static TierKernels tierKernels(const Handle* h) {
+  TierKernels k;
+  withTierWidth(h, [&](auto swarm, auto width) {
+    constexpr int W = decltype(width)::value;
+    if constexpr (decltype(swarm)::value)
+      k = {(const void*)kb_swarm_step_kernel<W>, (const void*)kb_swarm_reset_kernel<W>, (const void*)kb_swarm_setpose_kernel<W>};
+    else
+      k = {(const void*)kb_step_kernel<W>, (const void*)kb_reset_kernel<W>, (const void*)kb_setpose_kernel<W>};
+  });
+  return k;
+}
 
 // The dynamic shared-memory limit is an attribute of the kernel, shared by every handle of the process: only ever raise
 // it, so that a batch created later with a smaller image (same kernel, fewer bodies) does not break an earlier one.
@@ -283,6 +359,38 @@ static int fail(int code, const std::string& msg) {
     cudaError_t e_ = (expr);                                                                       \
     if (e_ != cudaSuccess) return fail(KB_ERR_CUDA, std::string(#expr) + ": " + cudaGetErrorString(e_)); \
   } while (0)
+
+// The preamble of an entry point that works on the device: the handle exists, its device is made current and, with
+// `sync`, its earlier work has finished.
+static int enter(const Handle* h, const char* who, bool sync) {
+  if (!h) return fail(KB_ERR_INVALID, std::string(who) + ": null handle");
+  CUDA_TRY(cudaSetDevice(h->device));
+  if (sync) CUDA_TRY(cudaDeviceSynchronize());
+  return KB_OK;
+}
+
+// launches `kernel` (a TierKernels member or the specialised step kernel) over the envs [a.envOffset, a.envOffset + count)
+static int launch(const Handle* h, const void* kernel, KernelArgs& a, int count, cudaStream_t stream) {
+  void* args[] = {&a};
+  CUDA_TRY(cudaLaunchKernel(kernel, dim3((count + h->envsPerBlock - 1) / h->envsPerBlock), dim3(blockThreads(h)), args,
+                            h->smemBytes, stream));
+  return KB_OK;
+}
+
+// copies the state blobs to the host and calls perEnv(e, words of env e's blob) for every env
+template <class F>
+static int fetchBlobs(const Handle* h, const char* who, F&& perEnv) {
+  if (const int rc = enter(h, who, true)) return rc;
+  std::vector<uint32_t> buf((size_t)h->numEnvs * h->L.blobWords);
+  CUDA_TRY(cudaMemcpy(buf.data(), h->dBlobs.get(), buf.size() * 4, cudaMemcpyDeviceToHost));
+  for (int e = 0; e < h->numEnvs; ++e) perEnv(e, buf.data() + (size_t)e * h->L.blobWords);
+  return KB_OK;
+}
+static inline float asf(uint32_t u) {
+  float f;
+  std::memcpy(&f, &u, 4);
+  return f;
+}
 
 // --- Box2D fixture preprocessing (float32, same operation order as Box2D) ---------------------
 struct HV2 {
@@ -565,17 +673,17 @@ static void fillArgs(const Handle* h, KernelArgs* a) {
   std::memset(a, 0, sizeof(*a));
   a->L = h->L;
   a->W = h->W;
-  a->blobs = h->dBlobs;
-  a->envScene = h->dEnvScene;
-  a->proxies = h->dProxies;
-  a->bodies = h->dBodies;
-  a->scenes = h->dScenes;
-  a->lights = h->dLights;
+  a->blobs = h->dBlobs.get();
+  a->envScene = h->dEnvScene.get();
+  a->proxies = h->dProxies.get();
+  a->bodies = h->dBodies.get();
+  a->scenes = h->dScenes.get();
+  a->lights = h->dLights.get();
   a->numEnvs = h->numEnvs;
   a->task = h->task;
-  a->taskState = h->dTask;
+  a->taskState = h->dTask.get();
 #ifdef KB_PROFILE
-  a->prof = h->dProf;
+  a->prof = h->dProf.get();
 #endif
 }
 
@@ -757,7 +865,7 @@ static int planBatch(const KbSceneDesc* scenes, int32_t num_scenes, int32_t max_
       L.lanesPerEnv = perSm >= 4 ? 128 : (perSm >= 2 ? 256 : 512);
       if (const char* ev = getenv("KB_SWARM_THREADS")) {
         const int v = atoi(ev);
-        if (v == 128 || v == 256 || v == 512) L.lanesPerEnv = v;
+        if (SwarmTier::has(v)) L.lanesPerEnv = v;
       }
     }
     L.smemWords = W.smemBytes / 4;
@@ -871,7 +979,7 @@ static int planBatch(const KbSceneDesc* scenes, int32_t num_scenes, int32_t max_
     int lpe = B <= 6 ? 4 : (B <= 24 ? 8 : (B <= 40 ? 16 : 32));
     if (const char* ev = getenv("KB_LANES_PER_ENV")) {
       const int v = atoi(ev);
-      if (v == 4 || v == 8 || v == 16 || v == 32) lpe = v;
+      if (LaneGroupTier::has(v)) lpe = v;
     }
     L.lanesPerEnv = lpe;
 #ifndef KB_NO_BANK_STAGGER
@@ -898,6 +1006,9 @@ const char* kb_last_error(void) { return g_err.c_str(); }
 int kb_create(const KbSceneDesc* scenes, int32_t num_scenes, const int32_t* env_scene, int32_t num_envs,
               int32_t max_contacts, int32_t device, KbHandle** out) {
   if (!scenes || num_scenes < 1 || num_envs < 1 || !out) return fail(KB_ERR_INVALID, "kb_create: invalid arguments");
+  if (env_scene)
+    for (int i = 0; i < num_envs; ++i)
+      if (env_scene[i] < 0 || env_scene[i] >= num_scenes) return fail(KB_ERR_INVALID, "kb_create: env_scene out of range");
   int ndev = 0;
   if (cudaGetDeviceCount(&ndev) != cudaSuccess || ndev <= 0 || device < 0 || device >= ndev) {
     cudaGetLastError();
@@ -908,26 +1019,23 @@ int kb_create(const KbSceneDesc* scenes, int32_t num_scenes, const int32_t* env_
   if (prop.major != 10) return fail(KB_ERR_NO_DEVICE, "kb_create: device is not sm_100 (B200); no fallback path exists");
   CUDA_TRY(cudaSetDevice(device));
 
-  Handle* h = new Handle();
+  // owned here until the batch is complete: every early return frees what was allocated
+  std::unique_ptr<Handle> hp(new Handle());
+  Handle* h = hp.get();
   h->device = device;
   h->numEnvs = num_envs;
   h->numScenes = num_scenes;
   {
     const int rc = planBatch(scenes, num_scenes, max_contacts, prop, h);
-    if (rc != KB_OK) {
-      delete h;
-      return rc;
-    }
+    if (rc != KB_OK) return rc;
   }
   const KbSceneDesc& s0 = scenes[0];
   const Layout& L = h->L;
   const bool swarm = h->W.enabled != 0;
   const int M = L.M, N = L.N;
-  if (h->smemBytes > (size_t)prop.sharedMemPerBlockOptin) {
-    delete h;
+  if (h->smemBytes > (size_t)prop.sharedMemPerBlockOptin)
     return fail(KB_ERR_CAPACITY, swarm ? "kb_create: this swarm does not fit one SM's shared memory (about 1700 kilobots per env at the minimal capacities)"
                                        : "kb_create: per-env shared-memory image too large; lower max_contacts");
-  }
 
   std::vector<ProxyConst> allProxies;
   std::vector<BodyConst> allBodies;
@@ -936,10 +1044,7 @@ int kb_create(const KbSceneDesc* scenes, int32_t num_scenes, const int32_t* env_
   for (int s = 0; s < num_scenes; ++s) {
     std::vector<ProxyConst> px;
     int rc = buildScene(scenes[s], L.M, L.Bp, L.Pp, &px, &h->hostBodies[s], &allScenes[s]);
-    if (rc != KB_OK) {
-      delete h;
-      return rc;
-    }
+    if (rc != KB_OK) return rc;
     allProxies.insert(allProxies.end(), px.begin(), px.end());
     h->hostNumProxies.push_back(allScenes[s].numProxies);
     h->hostNumObjects.push_back(scenes[s].num_objects);
@@ -965,27 +1070,25 @@ int kb_create(const KbSceneDesc* scenes, int32_t num_scenes, const int32_t* env_
       lc.maxVel = ld.max_velocity;
     }
 #define ALLOC_COPY(dst, vec)                                                                   \
-  CUDA_TRY(cudaMalloc(&(dst), sizeof((vec)[0]) * (vec).size()));                               \
-  CUDA_TRY(cudaMemcpy((dst), (vec).data(), sizeof((vec)[0]) * (vec).size(), cudaMemcpyHostToDevice));
+  CUDA_TRY(devAlloc((dst), (vec).size()));                                                     \
+  CUDA_TRY(cudaMemcpy((dst).get(), (vec).data(), sizeof((vec)[0]) * (vec).size(), cudaMemcpyHostToDevice));
   ALLOC_COPY(h->dProxies, allProxies);
   ALLOC_COPY(h->dBodies, allBodies);
   ALLOC_COPY(h->dScenes, allScenes);
   ALLOC_COPY(h->dLights, lights);
 #undef ALLOC_COPY
   if (env_scene) {
-    for (int i = 0; i < num_envs; ++i)
-      if (env_scene[i] < 0 || env_scene[i] >= num_scenes) return fail(KB_ERR_INVALID, "kb_create: env_scene out of range");
-    CUDA_TRY(cudaMalloc(&h->dEnvScene, sizeof(int32_t) * num_envs));
-    CUDA_TRY(cudaMemcpy(h->dEnvScene, env_scene, sizeof(int32_t) * num_envs, cudaMemcpyHostToDevice));
+    CUDA_TRY(devAlloc(h->dEnvScene, num_envs));
+    CUDA_TRY(cudaMemcpy(h->dEnvScene.get(), env_scene, sizeof(int32_t) * num_envs, cudaMemcpyHostToDevice));
   }
   const size_t blobBytes = (size_t)launchGrid(h) * h->envsPerBlock * L.blobWords * 4;  // padded to whole blocks
-  CUDA_TRY(cudaMalloc(&h->dBlobs, blobBytes));
-  CUDA_TRY(cudaMemset(h->dBlobs, 0, blobBytes));
+  CUDA_TRY(devAlloc(h->dBlobs, blobBytes / 4));
+  CUDA_TRY(cudaMemset(h->dBlobs.get(), 0, blobBytes));
   if (env_scene)   // H_SCENE before the first reset: the env's scene, so that kb_get_body_counts is right from the start
-    CUDA_TRY(cudaMemcpy2D(h->dBlobs + L.oHdr + H_SCENE, (size_t)L.blobWords * 4, env_scene, sizeof(int32_t), sizeof(int32_t),
-                          (size_t)num_envs, cudaMemcpyHostToDevice));
+    CUDA_TRY(cudaMemcpy2D(h->dBlobs.get() + L.oHdr + H_SCENE, (size_t)L.blobWords * 4, env_scene, sizeof(int32_t),
+                          sizeof(int32_t), (size_t)num_envs, cudaMemcpyHostToDevice));
   const int Amax = std::max(std::max(L.A, 2 * N), 1);
-  CUDA_TRY(cudaMalloc(&h->dAction, sizeof(double) * (size_t)num_envs * Amax));
+  CUDA_TRY(devAlloc(h->dAction, (size_t)num_envs * Amax));
   {
     const int64_t sizes[6] = {(int64_t)sizeof(float) * num_envs * N * 3, (int64_t)sizeof(float) * num_envs * M * 3,
                               (int64_t)sizeof(double) * num_envs * L.L, (int64_t)sizeof(float) * num_envs,
@@ -996,40 +1099,25 @@ int kb_create(const KbSceneDesc* scenes, int32_t num_scenes, const int32_t* env_
       off += (sizes[i] + 255) & ~(int64_t)255;
     }
     h->hostTotal = off;
-    CUDA_TRY(cudaMalloc(&h->dOut, (size_t)off + 256));
-    h->dObsK = reinterpret_cast<float*>(h->dOut + h->hostOff[0]);
-    h->dObsO = reinterpret_cast<float*>(h->dOut + h->hostOff[1]);
-    h->dObsL = reinterpret_cast<double*>(h->dOut + h->hostOff[2]);
-    h->dReward = reinterpret_cast<float*>(h->dOut + h->hostOff[3]);
-    h->dStatus = reinterpret_cast<int32_t*>(h->dOut + h->hostOff[4]);
-    h->dDone = h->dOut + h->hostOff[5];
+    CUDA_TRY(devAlloc(h->dOut, (size_t)off + 256));
+    uint8_t* base = h->dOut.get();
+    h->dObsK = reinterpret_cast<float*>(base + h->hostOff[0]);
+    h->dObsO = reinterpret_cast<float*>(base + h->hostOff[1]);
+    h->dObsL = reinterpret_cast<double*>(base + h->hostOff[2]);
+    h->dReward = reinterpret_cast<float*>(base + h->hostOff[3]);
+    h->dStatus = reinterpret_cast<int32_t*>(base + h->hostOff[4]);
+    h->dDone = base + h->hostOff[5];
   }
   h->wall[0] = s0.wall_x0; h->wall[1] = s0.wall_y0; h->wall[2] = s0.wall_x1; h->wall[3] = s0.wall_y1;
-  CUDA_TRY(cudaMalloc(&h->dTask, sizeof(double) * KB_TASK_WORDS * (size_t)num_envs));
-  CUDA_TRY(cudaMemset(h->dTask, 0, sizeof(double) * KB_TASK_WORDS * (size_t)num_envs));
+  CUDA_TRY(devAlloc(h->dTask, KB_TASK_WORDS * (size_t)num_envs));
+  CUDA_TRY(cudaMemset(h->dTask.get(), 0, sizeof(double) * KB_TASK_WORDS * (size_t)num_envs));
 #ifdef KB_PROFILE
-  CUDA_TRY(cudaMalloc(&h->dProf, sizeof(unsigned long long) * KB_PROF_SLOTS * (size_t)num_envs));
+  CUDA_TRY(devAlloc(h->dProf, KB_PROF_SLOTS * (size_t)num_envs));
 #endif
-#define KB_SET_SMEM(LPE)                                                                                            \
-  case LPE:                                                                                                          \
-    CUDA_TRY(raiseSmemLimit(kb_step_kernel<LPE>, h->smemBytes));                                                     \
-    CUDA_TRY(raiseSmemLimit(kb_reset_kernel<LPE>, h->smemBytes));                                                    \
-    CUDA_TRY(raiseSmemLimit(kb_setpose_kernel<LPE>, h->smemBytes));                                                  \
-    break;
-  if (swarm) {
-#define KB_SET_SWARM_SMEM(T)                                                                                           \
-    CUDA_TRY(raiseSmemLimit(kb_swarm_step_kernel<T>, h->smemBytes));                                                 \
-    CUDA_TRY(raiseSmemLimit(kb_swarm_reset_kernel<T>, h->smemBytes));                                                \
-    CUDA_TRY(raiseSmemLimit(kb_swarm_setpose_kernel<T>, h->smemBytes));
-    if (L.lanesPerEnv == 128) { KB_SET_SWARM_SMEM(128) } else if (L.lanesPerEnv == 256) { KB_SET_SWARM_SMEM(256) } else { KB_SET_SWARM_SMEM(512) }
-#undef KB_SET_SWARM_SMEM
-  } else switch (L.lanesPerEnv) {
-    KB_SET_SMEM(4)
-    KB_SET_SMEM(8)
-    KB_SET_SMEM(16)
-    KB_SET_SMEM(32)
+  {
+    const TierKernels k = tierKernels(h);
+    for (const void* kernel : {k.step, k.reset, k.setpose}) CUDA_TRY(raiseSmemLimit(kernel, h->smemBytes));
   }
-#undef KB_SET_SMEM
   if (!swarm) {
     // KB_JIT=0: the generic kernel; KB_JIT=1: the specialised kernel or an error; unset: the specialised kernel when
     // it can be had
@@ -1049,11 +1137,8 @@ int kb_create(const KbSceneDesc* scenes, int32_t num_scenes, const int32_t* env_
           h->jitReason = std::string("load error: ") + cudaGetErrorString(e);
         }
       }
-      if (!h->stepJit && mode == 1) {
-        const std::string why = h->jitReason;
-        kb_destroy(reinterpret_cast<KbHandle*>(h));
-        return fail(KB_ERR_CUDA, "kb_create: KB_JIT=1 but the specialised step kernel is not available: " + why);
-      }
+      if (!h->stepJit && mode == 1)
+        return fail(KB_ERR_CUDA, "kb_create: KB_JIT=1 but the specialised step kernel is not available: " + h->jitReason);
     }
   } else {
     h->jitReason = "large-swarm tier";
@@ -1069,13 +1154,13 @@ int kb_create(const KbSceneDesc* scenes, int32_t num_scenes, const int32_t* env_
     h->hostChunks = nc;
     if (nc > 1) {
       for (int i = 0; i < 2; ++i) {
-        CUDA_TRY(cudaStreamCreateWithFlags(&h->pipe[i], cudaStreamNonBlocking));
-        CUDA_TRY(cudaEventCreateWithFlags(&h->evJoin[i], cudaEventDisableTiming));
+        CUDA_TRY(create(h->pipe[i]));
+        CUDA_TRY(create(h->evJoin[i]));
       }
-      CUDA_TRY(cudaEventCreateWithFlags(&h->evFork, cudaEventDisableTiming));
+      CUDA_TRY(create(h->evFork));
     }
   }
-  *out = reinterpret_cast<KbHandle*>(h);
+  *out = reinterpret_cast<KbHandle*>(hp.release());
   return KB_OK;
 }
 
@@ -1083,15 +1168,6 @@ int kb_destroy(KbHandle* hh) {
   Handle* h = reinterpret_cast<Handle*>(hh);
   if (!h) return KB_OK;
   cudaSetDevice(h->device);
-  cudaFree(h->dBlobs); cudaFree(h->dEnvScene); cudaFree(h->dProxies); cudaFree(h->dBodies);
-  cudaFree(h->dScenes); cudaFree(h->dLights); cudaFree(h->dAction); cudaFree(h->dOut); cudaFree(h->dTask); cudaFree(h->dRenderIds);
-  cudaFree(h->dSampler); cudaFree(h->dSamplePose); cudaFree(h->dSampleLight); cudaFree(h->dEpisode);
-  cudaFree(h->dSceneConfig); cudaFree(h->dConfigCdf);
-  for (int i = 0; i < 2; ++i) {
-    if (h->pipe[i]) cudaStreamDestroy(h->pipe[i]);
-    if (h->evJoin[i]) cudaEventDestroy(h->evJoin[i]);
-  }
-  if (h->evFork) cudaEventDestroy(h->evFork);
   delete h;
   return KB_OK;
 }
@@ -1111,31 +1187,12 @@ int kb_get_dims(const KbHandle* hh, KbDims* d) {
   return KB_OK;
 }
 
-// launches `kernel` over the envs [a.envOffset, a.envOffset + count)
-#define KB_LAUNCH_RANGE(kernel, swarmKernel, h, st, a, count)                                     \
-  if ((h)->W.enabled) {                                                                           \
-    switch ((h)->L.lanesPerEnv) {                                                                 \
-      case 128: swarmKernel<128><<<(count), 128, (h)->smemBytes, (st)>>>(a); break;                     \
-      case 256: swarmKernel<256><<<(count), 256, (h)->smemBytes, (st)>>>(a); break;                     \
-      default: swarmKernel<512><<<(count), 512, (h)->smemBytes, (st)>>>(a); break;                      \
-    }                                                                                             \
-  } else {                                                                                        \
-    const int grid_ = ((count) + (h)->envsPerBlock - 1) / (h)->envsPerBlock;                      \
-    switch ((h)->L.lanesPerEnv) {                                                                 \
-      case 4: kernel<4><<<grid_, KB_BLOCK_OF(4), (h)->smemBytes, (st)>>>(a); break;                     \
-      case 8: kernel<8><<<grid_, KB_BLOCK_OF(8), (h)->smemBytes, (st)>>>(a); break;                     \
-      case 16: kernel<16><<<grid_, KB_BLOCK_OF(16), (h)->smemBytes, (st)>>>(a); break;                   \
-      default: kernel<32><<<grid_, KB_BLOCK_OF(32), (h)->smemBytes, (st)>>>(a); break;                   \
-    }                                                                                             \
-  }
-#define KB_LAUNCH(kernel, swarmKernel, h, st, a) KB_LAUNCH_RANGE(kernel, swarmKernel, h, st, a, (h)->numEnvs)
-
 int kb_reset(KbHandle* hh, const uint8_t* mask, const double* body_pose, const double* light_state,
              const double* kb_velocity, void* stream) {
   Handle* h = reinterpret_cast<Handle*>(hh);
-  if (!h || !body_pose) return fail(KB_ERR_INVALID, "kb_reset: null handle or poses");
+  if (const int rc = enter(h, "kb_reset", false)) return rc;
+  if (!body_pose) return fail(KB_ERR_INVALID, "kb_reset: null poses");
   if (h->L.L > 0 && !light_state) return fail(KB_ERR_INVALID, "kb_reset: light_state required");
-  CUDA_TRY(cudaSetDevice(h->device));
   KernelArgs a;
   fillArgs(h, &a);
   a.mask = mask;
@@ -1143,9 +1200,7 @@ int kb_reset(KbHandle* hh, const uint8_t* mask, const double* body_pose, const d
   a.lightInit = light_state;
   a.kbVel = kb_velocity;
   a.status = h->dStatus;
-  KB_LAUNCH(kb_reset_kernel, kb_swarm_reset_kernel, h, (cudaStream_t)stream, a);
-  CUDA_TRY(cudaGetLastError());
-  return KB_OK;
+  return launch(h, tierKernels(h).reset, a, h->numEnvs, (cudaStream_t)stream);
 }
 
 // ---- on-device scene sampling (include/kb_b200.h "Reset with on-device scene sampling") ------------------------
@@ -1236,29 +1291,38 @@ static int setSamplers(Handle* h, const KbSampleSpec* specs, int K, const double
       cdf[c] = c >= last ? 1.0 : acc / total;
     }
   }
-  CUDA_TRY(cudaSetDevice(h->device));
-  CUDA_TRY(cudaDeviceSynchronize());
+  if (const int rc = enter(h, who, true)) return rc;
   const size_t E = (size_t)h->numEnvs;
   std::vector<int32_t> envScene(E, 0);
-  if (h->dEnvScene) CUDA_TRY(cudaMemcpy(envScene.data(), h->dEnvScene, sizeof(int32_t) * E, cudaMemcpyDeviceToHost));
+  if (h->dEnvScene) CUDA_TRY(cudaMemcpy(envScene.data(), h->dEnvScene.get(), sizeof(int32_t) * E, cudaMemcpyDeviceToHost));
   if (K > 1)
     for (size_t e = 0; e < E; ++e)
       if (sceneConfig[envScene[e]] < 0) return bad("an env's scene belongs to no spec");
-  if (!h->dSampler) {
-    CUDA_TRY(cudaMalloc(&h->dSampler, sizeof(SamplerConst) * KB_SAMPLE_MAX_CONFIGS));
-    CUDA_TRY(cudaMalloc(&h->dSamplePose, sizeof(double) * E * L.B * 3));
-    CUDA_TRY(cudaMalloc(&h->dSampleLight, sizeof(double) * E * std::max(L.L, 1)));
-    CUDA_TRY(cudaMalloc(&h->dEpisode, sizeof(uint32_t) * E));
-    CUDA_TRY(cudaMalloc(&h->dSceneConfig, sizeof(int32_t) * h->numScenes));
-    CUDA_TRY(cudaMalloc(&h->dConfigCdf, sizeof(double) * KB_SAMPLE_MAX_CONFIGS));
+  if (!h->dSampler) {   // the handle takes the six buffers only when all of them exist
+    DevBuf<SamplerConst> sampler;
+    DevBuf<double> pose, light, configCdf;
+    DevBuf<uint32_t> episode;
+    DevBuf<int32_t> sceneCfg;
+    CUDA_TRY(devAlloc(sampler, KB_SAMPLE_MAX_CONFIGS));
+    CUDA_TRY(devAlloc(pose, E * L.B * 3));
+    CUDA_TRY(devAlloc(light, E * std::max(L.L, 1)));
+    CUDA_TRY(devAlloc(episode, E));
+    CUDA_TRY(devAlloc(sceneCfg, h->numScenes));
+    CUDA_TRY(devAlloc(configCdf, KB_SAMPLE_MAX_CONFIGS));
+    h->dSampler = std::move(sampler);
+    h->dSamplePose = std::move(pose);
+    h->dSampleLight = std::move(light);
+    h->dEpisode = std::move(episode);
+    h->dSceneConfig = std::move(sceneCfg);
+    h->dConfigCdf = std::move(configCdf);
   }
-  CUDA_TRY(cudaMemset(h->dEpisode, 0, sizeof(uint32_t) * E));
-  CUDA_TRY(cudaMemcpy(h->dSampler, scs.data(), sizeof(SamplerConst) * K, cudaMemcpyHostToDevice));
-  CUDA_TRY(cudaMemcpy(h->dSceneConfig, sceneConfig.data(), sizeof(int32_t) * h->numScenes, cudaMemcpyHostToDevice));
-  CUDA_TRY(cudaMemcpy(h->dConfigCdf, cdf.data(), sizeof(double) * KB_SAMPLE_MAX_CONFIGS, cudaMemcpyHostToDevice));
+  CUDA_TRY(cudaMemset(h->dEpisode.get(), 0, sizeof(uint32_t) * E));
+  CUDA_TRY(cudaMemcpy(h->dSampler.get(), scs.data(), sizeof(SamplerConst) * K, cudaMemcpyHostToDevice));
+  CUDA_TRY(cudaMemcpy(h->dSceneConfig.get(), sceneConfig.data(), sizeof(int32_t) * h->numScenes, cudaMemcpyHostToDevice));
+  CUDA_TRY(cudaMemcpy(h->dConfigCdf.get(), cdf.data(), sizeof(double) * KB_SAMPLE_MAX_CONFIGS, cudaMemcpyHostToDevice));
   if (!h->dEnvScene) {   // the reset may switch scenes: the per-env scene map becomes device state
-    CUDA_TRY(cudaMalloc(&h->dEnvScene, sizeof(int32_t) * E));
-    CUDA_TRY(cudaMemset(h->dEnvScene, 0, sizeof(int32_t) * E));
+    CUDA_TRY(devAlloc(h->dEnvScene, E));
+    CUDA_TRY(cudaMemset(h->dEnvScene.get(), 0, sizeof(int32_t) * E));
   }
   h->numConfigs = K;
   h->weighted = weights != nullptr;
@@ -1286,49 +1350,46 @@ int kb_set_sampler_mix(KbHandle* hh, const KbSampleSpec* specs, int32_t num_spec
 
 int kb_current_scenes(KbHandle* hh, int32_t* out_device, void* stream) {
   Handle* h = reinterpret_cast<Handle*>(hh);
-  if (!h || !out_device) return fail(KB_ERR_INVALID, "kb_current_scenes: null");
-  CUDA_TRY(cudaSetDevice(h->device));
-  kb_current_scenes_kernel<<<(h->numEnvs + 255) / 256, 256, 0, (cudaStream_t)stream>>>(h->dBlobs, h->L.blobWords,
-                                                                                      h->L.oHdr + H_SCENE, h->numEnvs, out_device);
+  if (const int rc = enter(h, "kb_current_scenes", false)) return rc;
+  if (!out_device) return fail(KB_ERR_INVALID, "kb_current_scenes: null");
+  kb_current_scenes_kernel<<<(h->numEnvs + 255) / 256, 256, 0, (cudaStream_t)stream>>>(
+      h->dBlobs.get(), h->L.blobWords, h->L.oHdr + H_SCENE, h->numEnvs, out_device);
   CUDA_TRY(cudaGetLastError());
   return KB_OK;
 }
 
 int kb_reset_sampled(KbHandle* hh, const uint8_t* mask, void* stream) {
   Handle* h = reinterpret_cast<Handle*>(hh);
-  if (!h) return fail(KB_ERR_INVALID, "kb_reset_sampled: null handle");
+  if (const int rc = enter(h, "kb_reset_sampled", false)) return rc;
   if (!h->dSampler) return fail(KB_ERR_INVALID, "kb_reset_sampled: no sampler (kb_set_sampler)");
-  CUDA_TRY(cudaSetDevice(h->device));
   KernelArgs a;
   fillArgs(h, &a);
   a.mask = mask;
-  a.pose = h->dSamplePose;
-  a.lightInit = h->dSampleLight;
+  a.pose = h->dSamplePose.get();
+  a.lightInit = h->dSampleLight.get();
   a.kbVel = nullptr;
   a.status = h->dStatus;
-  a.sampler = h->dSampler;
-  a.samplePose = h->dSamplePose;
-  a.sampleLight = h->dSampleLight;
-  a.envSceneW = h->dEnvScene;
-  a.episode = h->dEpisode;
-  a.sceneConfig = h->dSceneConfig;
-  a.configCdf = h->weighted ? h->dConfigCdf : nullptr;
+  a.sampler = h->dSampler.get();
+  a.samplePose = h->dSamplePose.get();
+  a.sampleLight = h->dSampleLight.get();
+  a.envSceneW = h->dEnvScene.get();
+  a.episode = h->dEpisode.get();
+  a.sceneConfig = h->dSceneConfig.get();
+  a.configCdf = h->weighted ? h->dConfigCdf.get() : nullptr;
   a.numConfigs = h->numConfigs;
-  KB_LAUNCH(kb_reset_kernel, kb_swarm_reset_kernel, h, (cudaStream_t)stream, a);
-  CUDA_TRY(cudaGetLastError());
-  return KB_OK;
+  return launch(h, tierKernels(h).reset, a, h->numEnvs, (cudaStream_t)stream);
 }
 
 int kb_get_sampled(KbHandle* hh, double* body_pose, double* light_state, int32_t* env_scene, uint32_t* episodes) {
   Handle* h = reinterpret_cast<Handle*>(hh);
-  if (!h || !h->dSampler) return fail(KB_ERR_INVALID, "kb_get_sampled: no sampler");
-  CUDA_TRY(cudaSetDevice(h->device));
-  CUDA_TRY(cudaDeviceSynchronize());
+  if (const int rc = enter(h, "kb_get_sampled", true)) return rc;
+  if (!h->dSampler) return fail(KB_ERR_INVALID, "kb_get_sampled: no sampler");
   const size_t E = (size_t)h->numEnvs;
-  if (body_pose) CUDA_TRY(cudaMemcpy(body_pose, h->dSamplePose, sizeof(double) * E * h->L.B * 3, cudaMemcpyDeviceToHost));
-  if (light_state && h->L.L > 0) CUDA_TRY(cudaMemcpy(light_state, h->dSampleLight, sizeof(double) * E * h->L.L, cudaMemcpyDeviceToHost));
-  if (env_scene) CUDA_TRY(cudaMemcpy(env_scene, h->dEnvScene, sizeof(int32_t) * E, cudaMemcpyDeviceToHost));
-  if (episodes) CUDA_TRY(cudaMemcpy(episodes, h->dEpisode, sizeof(uint32_t) * E, cudaMemcpyDeviceToHost));
+  if (body_pose) CUDA_TRY(cudaMemcpy(body_pose, h->dSamplePose.get(), sizeof(double) * E * h->L.B * 3, cudaMemcpyDeviceToHost));
+  if (light_state && h->L.L > 0)
+    CUDA_TRY(cudaMemcpy(light_state, h->dSampleLight.get(), sizeof(double) * E * h->L.L, cudaMemcpyDeviceToHost));
+  if (env_scene) CUDA_TRY(cudaMemcpy(env_scene, h->dEnvScene.get(), sizeof(int32_t) * E, cudaMemcpyDeviceToHost));
+  if (episodes) CUDA_TRY(cudaMemcpy(episodes, h->dEpisode.get(), sizeof(uint32_t) * E, cudaMemcpyDeviceToHost));
   return KB_OK;
 }
 
@@ -1339,10 +1400,9 @@ int kb_set_env_scene(KbHandle* hh, const int32_t* env_scene) {
     if (env_scene[i] < 0 || env_scene[i] >= h->numScenes) return fail(KB_ERR_INVALID, "kb_set_env_scene: scene out of range");
     else if (h->numConfigs > 1 && h->hostSceneConfig[env_scene[i]] < 0)
       return fail(KB_ERR_INVALID, "kb_set_env_scene: the scene belongs to no configuration of the sampler");
-  CUDA_TRY(cudaSetDevice(h->device));
-  CUDA_TRY(cudaDeviceSynchronize());
-  if (!h->dEnvScene) CUDA_TRY(cudaMalloc(&h->dEnvScene, sizeof(int32_t) * (size_t)h->numEnvs));
-  CUDA_TRY(cudaMemcpy(h->dEnvScene, env_scene, sizeof(int32_t) * (size_t)h->numEnvs, cudaMemcpyHostToDevice));
+  if (const int rc = enter(h, "kb_set_env_scene", true)) return rc;
+  if (!h->dEnvScene) CUDA_TRY(devAlloc(h->dEnvScene, h->numEnvs));
+  CUDA_TRY(cudaMemcpy(h->dEnvScene.get(), env_scene, sizeof(int32_t) * (size_t)h->numEnvs, cudaMemcpyHostToDevice));
   return KB_OK;
 }
 
@@ -1361,25 +1421,18 @@ static int stepRange(Handle* h, const double* action, int32_t action_mode, float
   a.status = status;
   a.obsFlat = h->obsFlat;
   a.envOffset = envBegin;
-  if (h->stepJit) {
-    void* args[] = {&a};
-    const int grid = (envCount + h->envsPerBlock - 1) / h->envsPerBlock;
-    CUDA_TRY(cudaLaunchKernel((const void*)h->stepJit, dim3(grid), dim3(KB_BLOCK_OF(h->L.lanesPerEnv)), args,
-                              h->smemBytes, stream));
-    return KB_OK;
-  }
-  KB_LAUNCH_RANGE(kb_step_kernel, kb_swarm_step_kernel, h, stream, a, envCount);
-  CUDA_TRY(cudaGetLastError());
-  return KB_OK;
+  return launch(h, h->stepJit ? (const void*)h->stepJit : tierKernels(h).step, a, envCount, stream);
+}
+
+static bool badActionMode(int32_t mode) {
+  return mode != KB_ACTION_NONE && mode != KB_ACTION_LIGHT && mode != KB_ACTION_KILOBOTS;
 }
 
 int kb_step(KbHandle* hh, const double* action, int32_t action_mode, float* obs_kilobots, float* obs_objects,
             double* obs_light, float* reward, uint8_t* done, int32_t* status, void* stream) {
   Handle* h = reinterpret_cast<Handle*>(hh);
-  if (!h) return fail(KB_ERR_INVALID, "kb_step: null handle");
-  if (action_mode != KB_ACTION_NONE && action_mode != KB_ACTION_LIGHT && action_mode != KB_ACTION_KILOBOTS)
-    return fail(KB_ERR_INVALID, "kb_step: bad action_mode");
-  CUDA_TRY(cudaSetDevice(h->device));
+  if (const int rc = enter(h, "kb_step", false)) return rc;
+  if (badActionMode(action_mode)) return fail(KB_ERR_INVALID, "kb_step: bad action_mode");
   return stepRange(h, action, action_mode, obs_kilobots, obs_objects, obs_light, reward, done, status, 0, h->numEnvs,
                    (cudaStream_t)stream);
 }
@@ -1387,103 +1440,70 @@ int kb_step(KbHandle* hh, const double* action, int32_t action_mode, float* obs_
 int kb_step_host(KbHandle* hh, const double* action, int32_t action_mode, float* obs_kilobots, float* obs_objects,
                  double* obs_light, float* reward, uint8_t* done, int32_t* status, void* stream) {
   Handle* h = reinterpret_cast<Handle*>(hh);
-  if (!h) return fail(KB_ERR_INVALID, "kb_step_host: null handle");
-  CUDA_TRY(cudaSetDevice(h->device));
+  if (const int rc = enter(h, "kb_step_host", false)) return rc;
+  if (badActionMode(action_mode)) return fail(KB_ERR_INVALID, "kb_step_host: bad action_mode");
   cudaStream_t st = (cudaStream_t)stream;
   const Layout& L = h->L;
-  const size_t E = (size_t)h->numEnvs;
-  if (action_mode != KB_ACTION_NONE && action_mode != KB_ACTION_LIGHT && action_mode != KB_ACTION_KILOBOTS)
-    return fail(KB_ERR_INVALID, "kb_step_host: bad action_mode");
-  if (h->hostChunks > 1) {
-    // pipelined: chunk c = H2D of its actions, kernel over its envs, D2H of its outputs, on side stream c % 2; the
-    // copies of one chunk overlap the kernel of the next.  Chunks are whole blocks; only the last one is ragged.
-    const size_t A = action_mode == KB_ACTION_KILOBOTS ? 2 * (size_t)L.N : (size_t)L.A;
-    const bool haveAct = action && action_mode != KB_ACTION_NONE;
+  const size_t A = action_mode == KB_ACTION_KILOBOTS ? 2 * (size_t)L.N : (size_t)L.A;
+  const bool haveAct = action && action_mode != KB_ACTION_NONE;
+  // one device->host copy when the batch is stepped in one piece and the caller's buffers are laid out like the staging
+  // area (kb_get_host_layout)
+  const uint8_t* base = reinterpret_cast<const uint8_t*>(obs_kilobots);
+  const bool packed = h->hostChunks == 1 && obs_kilobots && obs_objects && obs_light && reward && done && status &&
+                      reinterpret_cast<const uint8_t*>(obs_objects) == base + h->hostOff[1] &&
+                      reinterpret_cast<const uint8_t*>(obs_light) == base + h->hostOff[2] &&
+                      reinterpret_cast<const uint8_t*>(reward) == base + h->hostOff[3] &&
+                      reinterpret_cast<const uint8_t*>(status) == base + h->hostOff[4] &&
+                      reinterpret_cast<const uint8_t*>(done) == base + h->hostOff[5];
+  // the envs [e0, e1) on stream s: H2D of their actions, the step, D2H of their outputs
+  auto stepEnvs = [&](int e0, int e1, cudaStream_t s) -> int {
+    const size_t b = (size_t)e0, n = (size_t)(e1 - e0);
+    if (haveAct)
+      CUDA_TRY(cudaMemcpyAsync(h->dAction.get() + b * A, action + b * A, sizeof(double) * n * A, cudaMemcpyHostToDevice, s));
+    const int rc = stepRange(h, haveAct ? h->dAction.get() : nullptr, action_mode, obs_kilobots ? h->dObsK : nullptr,
+                             obs_objects ? h->dObsO : nullptr, obs_light ? h->dObsL : nullptr, reward ? h->dReward : nullptr,
+                             done ? h->dDone : nullptr, status ? h->dStatus : nullptr, e0, e1 - e0, s);
+    if (rc != KB_OK) return rc;
+    if (packed) {
+      CUDA_TRY(cudaMemcpyAsync(obs_kilobots, h->dOut.get(), (size_t)h->hostTotal, cudaMemcpyDeviceToHost, s));
+      return KB_OK;
+    }
+    if (obs_kilobots && L.N > 0) CUDA_TRY(cudaMemcpyAsync(obs_kilobots + b * L.N * 3, h->dObsK + b * L.N * 3, sizeof(float) * n * L.N * 3, cudaMemcpyDeviceToHost, s));
+    if (obs_objects && L.M > 0) CUDA_TRY(cudaMemcpyAsync(obs_objects + b * L.M * 3, h->dObsO + b * L.M * 3, sizeof(float) * n * L.M * 3, cudaMemcpyDeviceToHost, s));
+    if (obs_light && L.L > 0) CUDA_TRY(cudaMemcpyAsync(obs_light + b * L.L, h->dObsL + b * L.L, sizeof(double) * n * L.L, cudaMemcpyDeviceToHost, s));
+    if (reward) CUDA_TRY(cudaMemcpyAsync(reward + b, h->dReward + b, sizeof(float) * n, cudaMemcpyDeviceToHost, s));
+    if (done) CUDA_TRY(cudaMemcpyAsync(done + b, h->dDone + b, n, cudaMemcpyDeviceToHost, s));
+    if (status) CUDA_TRY(cudaMemcpyAsync(status + b, h->dStatus + b, sizeof(int32_t) * n, cudaMemcpyDeviceToHost, s));
+    return KB_OK;
+  };
+  if (h->hostChunks == 1) {
+    if (const int rc = stepEnvs(0, h->numEnvs, st)) return rc;
+  } else {
+    // pipelined: chunk c on side stream c % 2, so that the copies of one chunk overlap the kernel of the next.  Chunks
+    // are whole blocks; only the last one is ragged.
     const int epb = h->envsPerBlock, blocks = launchGrid(h), nc = h->hostChunks;
-    CUDA_TRY(cudaEventRecord(h->evFork, st));
-    for (int i = 0; i < 2; ++i) CUDA_TRY(cudaStreamWaitEvent(h->pipe[i], h->evFork, 0));
+    CUDA_TRY(cudaEventRecord(h->evFork.get(), st));
+    for (int i = 0; i < 2; ++i) CUDA_TRY(cudaStreamWaitEvent(h->pipe[i].get(), h->evFork.get(), 0));
     for (int c = 0; c < nc; ++c) {
       const int b0 = (int)((int64_t)blocks * c / nc), b1 = (int)((int64_t)blocks * (c + 1) / nc);
       const int e0 = b0 * epb, e1 = std::min(b1 * epb, h->numEnvs);
       if (e1 <= e0) continue;
-      const size_t n = (size_t)(e1 - e0);
-      cudaStream_t s = h->pipe[c & 1];
-      if (haveAct) CUDA_TRY(cudaMemcpyAsync(h->dAction + (size_t)e0 * A, action + (size_t)e0 * A, sizeof(double) * n * A, cudaMemcpyHostToDevice, s));
-      int rc = stepRange(h, haveAct ? h->dAction : nullptr, action_mode, obs_kilobots ? h->dObsK : nullptr,
-                         obs_objects ? h->dObsO : nullptr, obs_light ? h->dObsL : nullptr, reward ? h->dReward : nullptr,
-                         done ? h->dDone : nullptr, status ? h->dStatus : nullptr, e0, e1 - e0, s);
-      if (rc != KB_OK) return rc;
-      if (obs_kilobots && L.N > 0) CUDA_TRY(cudaMemcpyAsync(obs_kilobots + (size_t)e0 * L.N * 3, h->dObsK + (size_t)e0 * L.N * 3, sizeof(float) * n * L.N * 3, cudaMemcpyDeviceToHost, s));
-      if (obs_objects && L.M > 0) CUDA_TRY(cudaMemcpyAsync(obs_objects + (size_t)e0 * L.M * 3, h->dObsO + (size_t)e0 * L.M * 3, sizeof(float) * n * L.M * 3, cudaMemcpyDeviceToHost, s));
-      if (obs_light && L.L > 0) CUDA_TRY(cudaMemcpyAsync(obs_light + (size_t)e0 * L.L, h->dObsL + (size_t)e0 * L.L, sizeof(double) * n * L.L, cudaMemcpyDeviceToHost, s));
-      if (reward) CUDA_TRY(cudaMemcpyAsync(reward + e0, h->dReward + e0, sizeof(float) * n, cudaMemcpyDeviceToHost, s));
-      if (done) CUDA_TRY(cudaMemcpyAsync(done + e0, h->dDone + e0, n, cudaMemcpyDeviceToHost, s));
-      if (status) CUDA_TRY(cudaMemcpyAsync(status + e0, h->dStatus + e0, sizeof(int32_t) * n, cudaMemcpyDeviceToHost, s));
+      if (const int rc = stepEnvs(e0, e1, h->pipe[c & 1].get())) return rc;
     }
     for (int i = 0; i < 2; ++i) {
-      CUDA_TRY(cudaEventRecord(h->evJoin[i], h->pipe[i]));
-      CUDA_TRY(cudaStreamWaitEvent(st, h->evJoin[i], 0));
-    }
-    CUDA_TRY(cudaStreamSynchronize(st));
-    return KB_OK;
-  }
-  const double* dAct = nullptr;
-  if (action && action_mode != KB_ACTION_NONE) {
-    const size_t A = action_mode == KB_ACTION_KILOBOTS ? 2 * (size_t)L.N : (size_t)L.A;
-    CUDA_TRY(cudaMemcpyAsync(h->dAction, action, sizeof(double) * E * A, cudaMemcpyHostToDevice, st));
-    dAct = h->dAction;
-  }
-  int rc = kb_step(hh, dAct, action_mode, obs_kilobots ? h->dObsK : nullptr, obs_objects ? h->dObsO : nullptr,
-                   obs_light ? h->dObsL : nullptr, reward ? h->dReward : nullptr, done ? h->dDone : nullptr,
-                   status ? h->dStatus : nullptr, stream);
-  if (rc != KB_OK) return rc;
-  {
-    // one device->host copy when the caller's buffers are laid out like the staging area (kb_get_host_layout)
-    const uint8_t* base = reinterpret_cast<const uint8_t*>(obs_kilobots);
-    const bool packed = obs_kilobots && obs_objects && obs_light && reward && done && status &&
-                        reinterpret_cast<const uint8_t*>(obs_objects) == base + h->hostOff[1] &&
-                        reinterpret_cast<const uint8_t*>(obs_light) == base + h->hostOff[2] &&
-                        reinterpret_cast<const uint8_t*>(reward) == base + h->hostOff[3] &&
-                        reinterpret_cast<const uint8_t*>(status) == base + h->hostOff[4] &&
-                        reinterpret_cast<const uint8_t*>(done) == base + h->hostOff[5];
-    if (packed) {
-      CUDA_TRY(cudaMemcpyAsync(obs_kilobots, h->dOut, (size_t)h->hostTotal, cudaMemcpyDeviceToHost, st));
-      CUDA_TRY(cudaStreamSynchronize(st));
-      return KB_OK;
+      CUDA_TRY(cudaEventRecord(h->evJoin[i].get(), h->pipe[i].get()));
+      CUDA_TRY(cudaStreamWaitEvent(st, h->evJoin[i].get(), 0));
     }
   }
-  if (obs_kilobots) CUDA_TRY(cudaMemcpyAsync(obs_kilobots, h->dObsK, sizeof(float) * E * L.N * 3, cudaMemcpyDeviceToHost, st));
-  if (obs_objects && L.M > 0) CUDA_TRY(cudaMemcpyAsync(obs_objects, h->dObsO, sizeof(float) * E * L.M * 3, cudaMemcpyDeviceToHost, st));
-  if (obs_light && L.L > 0) CUDA_TRY(cudaMemcpyAsync(obs_light, h->dObsL, sizeof(double) * E * L.L, cudaMemcpyDeviceToHost, st));
-  if (reward) CUDA_TRY(cudaMemcpyAsync(reward, h->dReward, sizeof(float) * E, cudaMemcpyDeviceToHost, st));
-  if (done) CUDA_TRY(cudaMemcpyAsync(done, h->dDone, E, cudaMemcpyDeviceToHost, st));
-  if (status) CUDA_TRY(cudaMemcpyAsync(status, h->dStatus, sizeof(int32_t) * E, cudaMemcpyDeviceToHost, st));
   CUDA_TRY(cudaStreamSynchronize(st));
   return KB_OK;
 }
 
 // ---- introspection (host pointers, synchronous) ------------------------------------------------
-static int fetchBlobs(Handle* h, std::vector<uint32_t>* buf) {
-  CUDA_TRY(cudaSetDevice(h->device));
-  CUDA_TRY(cudaDeviceSynchronize());
-  buf->resize((size_t)h->numEnvs * h->L.blobWords);
-  CUDA_TRY(cudaMemcpy(buf->data(), h->dBlobs, buf->size() * 4, cudaMemcpyDeviceToHost));
-  return KB_OK;
-}
-static inline float asf(uint32_t u) {
-  float f;
-  std::memcpy(&f, &u, 4);
-  return f;
-}
-
 int kb_get_bodies(KbHandle* hh, float* out) {
-  Handle* h = reinterpret_cast<Handle*>(hh);
-  std::vector<uint32_t> buf;
-  int rc = fetchBlobs(h, &buf);
-  if (rc) return rc;
-  const Layout& L = h->L;
-  for (int e = 0; e < h->numEnvs; ++e) {
-    const uint32_t* w = buf.data() + (size_t)e * L.blobWords;
+  const Handle* h = reinterpret_cast<Handle*>(hh);
+  return fetchBlobs(h, "kb_get_bodies", [&](int e, const uint32_t* w) {
+    const Layout& L = h->L;
     for (int b = 0; b < L.B; ++b) {
       float* o = out + ((size_t)e * L.B + b) * KB_BODY_STATE_FLOATS;
       const uint32_t* pos = w + L.oPos + 4 * b;
@@ -1495,32 +1515,25 @@ int kb_get_bodies(KbHandle* hh, float* out) {
       o[7] = (vel[3] & BF_AWAKE) ? 1.0f : 0.0f;
       o[8] = asf(xf[0]); o[9] = asf(xf[1]); o[10] = asf(xf[2]); o[11] = asf(xf[3]);
     }
-  }
-  return KB_OK;
+  });
 }
 
 int kb_set_poses_masked(KbHandle* hh, const double* body_pose, const uint8_t* body_mask) {
   Handle* h = reinterpret_cast<Handle*>(hh);
-  if (!h || !body_pose) return fail(KB_ERR_INVALID, "kb_set_poses: null");
-  CUDA_TRY(cudaSetDevice(h->device));
-  double* d = nullptr;
-  uint8_t* dm = nullptr;
+  if (const int rc = enter(h, "kb_set_poses", false)) return rc;
+  if (!body_pose) return fail(KB_ERR_INVALID, "kb_set_poses: null");
   const size_t nb = (size_t)h->numEnvs * h->L.B;
   const size_t bytes = sizeof(double) * nb * 3;
-  CUDA_TRY(cudaMalloc(&d, bytes + (body_mask ? nb : 0)));
-  CUDA_TRY(cudaMemcpy(d, body_pose, bytes, cudaMemcpyHostToDevice));
-  if (body_mask) {
-    dm = reinterpret_cast<uint8_t*>(d) + bytes;
-    CUDA_TRY(cudaMemcpy(dm, body_mask, nb, cudaMemcpyHostToDevice));
-  }
+  DevBuf<uint8_t> d;   // the poses, then the mask
+  CUDA_TRY(devAlloc(d, bytes + (body_mask ? nb : 0)));
+  CUDA_TRY(cudaMemcpy(d.get(), body_pose, bytes, cudaMemcpyHostToDevice));
+  if (body_mask) CUDA_TRY(cudaMemcpy(d.get() + bytes, body_mask, nb, cudaMemcpyHostToDevice));
   KernelArgs a;
   fillArgs(h, &a);
-  a.pose = d;
-  a.mask = dm;
-  KB_LAUNCH(kb_setpose_kernel, kb_swarm_setpose_kernel, h, (cudaStream_t)0, a);
-  cudaError_t e = cudaDeviceSynchronize();
-  cudaFree(d);
-  if (e != cudaSuccess) return fail(KB_ERR_CUDA, cudaGetErrorString(e));
+  a.pose = reinterpret_cast<const double*>(d.get());
+  a.mask = body_mask ? d.get() + bytes : nullptr;
+  if (const int rc = launch(h, tierKernels(h).setpose, a, h->numEnvs, (cudaStream_t)0)) return rc;
+  CUDA_TRY(cudaDeviceSynchronize());
   return KB_OK;
 }
 
@@ -1528,23 +1541,20 @@ int kb_set_poses(KbHandle* hh, const double* body_pose) { return kb_set_poses_ma
 
 int kb_get_status(KbHandle* hh, int32_t* out) {
   Handle* h = reinterpret_cast<Handle*>(hh);
-  if (!h || !out) return fail(KB_ERR_INVALID, "kb_get_status: null");
-  CUDA_TRY(cudaSetDevice(h->device));
-  CUDA_TRY(cudaDeviceSynchronize());
+  if (const int rc = enter(h, "kb_get_status", true)) return rc;
+  if (!out) return fail(KB_ERR_INVALID, "kb_get_status: null");
   // header word H_STATUS of every blob: one strided copy
-  CUDA_TRY(cudaMemcpy2D(out, sizeof(int32_t), h->dBlobs + h->L.oHdr + H_STATUS, (size_t)h->L.blobWords * 4, sizeof(int32_t),
-                        (size_t)h->numEnvs, cudaMemcpyDeviceToHost));
+  CUDA_TRY(cudaMemcpy2D(out, sizeof(int32_t), h->dBlobs.get() + h->L.oHdr + H_STATUS, (size_t)h->L.blobWords * 4,
+                        sizeof(int32_t), (size_t)h->numEnvs, cudaMemcpyDeviceToHost));
   return KB_OK;
 }
 
 int kb_get_body_counts(KbHandle* hh, int32_t* objects, int32_t* kilobots) {
   Handle* h = reinterpret_cast<Handle*>(hh);
-  if (!h) return fail(KB_ERR_INVALID, "kb_get_body_counts: null");
+  if (const int rc = enter(h, "kb_get_body_counts", true)) return rc;
   std::vector<int32_t> scene((size_t)h->numEnvs);
-  CUDA_TRY(cudaSetDevice(h->device));
-  CUDA_TRY(cudaDeviceSynchronize());
   // header word H_SCENE of every blob: the scene each env was last reset with
-  CUDA_TRY(cudaMemcpy2D(scene.data(), sizeof(int32_t), h->dBlobs + h->L.oHdr + H_SCENE, (size_t)h->L.blobWords * 4,
+  CUDA_TRY(cudaMemcpy2D(scene.data(), sizeof(int32_t), h->dBlobs.get() + h->L.oHdr + H_SCENE, (size_t)h->L.blobWords * 4,
                         sizeof(int32_t), (size_t)h->numEnvs, cudaMemcpyDeviceToHost));
   for (int e = 0; e < h->numEnvs; ++e) {
     const int s = scene[e] >= 0 && scene[e] < h->numScenes ? scene[e] : 0;
@@ -1555,13 +1565,9 @@ int kb_get_body_counts(KbHandle* hh, int32_t* objects, int32_t* kilobots) {
 }
 
 int kb_get_contacts(KbHandle* hh, int32_t* pairs, int32_t* count) {
-  Handle* h = reinterpret_cast<Handle*>(hh);
-  std::vector<uint32_t> buf;
-  int rc = fetchBlobs(h, &buf);
-  if (rc) return rc;
-  const Layout& L = h->L;
-  for (int e = 0; e < h->numEnvs; ++e) {
-    const uint32_t* w = buf.data() + (size_t)e * L.blobWords;
+  const Handle* h = reinterpret_cast<Handle*>(hh);
+  return fetchBlobs(h, "kb_get_contacts", [&](int e, const uint32_t* w) {
+    const Layout& L = h->L;
     const int nC = (int)w[L.oHdr + H_NC];
     count[e] = nC;
     for (int k = 0; k < nC && k < L.Cmax; ++k) {
@@ -1573,18 +1579,13 @@ int kb_get_contacts(KbHandle* hh, int32_t* pairs, int32_t* count) {
       o[2] = (info & CI_TOUCHING) ? 1 : 0;
       o[3] = (int32_t)((info & CI_PC_MASK) >> CI_PC_SHIFT);
     }
-  }
-  return KB_OK;
+  });
 }
 
 int kb_get_impulses(KbHandle* hh, float* out) {
-  Handle* h = reinterpret_cast<Handle*>(hh);
-  std::vector<uint32_t> buf;
-  int rc = fetchBlobs(h, &buf);
-  if (rc) return rc;
-  const Layout& L = h->L;
-  for (int e = 0; e < h->numEnvs; ++e) {
-    const uint32_t* w = buf.data() + (size_t)e * L.blobWords;
+  const Handle* h = reinterpret_cast<Handle*>(hh);
+  return fetchBlobs(h, "kb_get_impulses", [&](int e, const uint32_t* w) {
+    const Layout& L = h->L;
     const int nC = (int)w[L.oHdr + H_NC];
     for (int k = 0; k < nC && k < L.Cmax; ++k) {
       const int i = nC - 1 - k;
@@ -1602,67 +1603,48 @@ int kb_get_impulses(KbHandle* hh, float* out) {
       o[2] = pc > 1 ? asf(rec[MR_P1N]) : 0.0f;
       o[3] = pc > 1 ? asf(rec[MR_P1T]) : 0.0f;
     }
-  }
-  return KB_OK;
+  });
 }
 
 int kb_get_counters(KbHandle* hh, uint64_t* out) {
-  Handle* h = reinterpret_cast<Handle*>(hh);
-  std::vector<uint32_t> buf;
-  int rc = fetchBlobs(h, &buf);
-  if (rc) return rc;
-  const Layout& L = h->L;
-  for (int e = 0; e < h->numEnvs; ++e) {
-    const uint32_t* w = buf.data() + (size_t)e * L.blobWords;
-    std::memcpy(out + (size_t)e * KB_NUM_COUNTERS, w + L.oCnt, sizeof(uint64_t) * KB_NUM_COUNTERS);
-  }
-  return KB_OK;
+  const Handle* h = reinterpret_cast<Handle*>(hh);
+  return fetchBlobs(h, "kb_get_counters", [&](int e, const uint32_t* w) {
+    std::memcpy(out + (size_t)e * KB_NUM_COUNTERS, w + h->L.oCnt, sizeof(uint64_t) * KB_NUM_COUNTERS);
+  });
 }
 
 int kb_get_proxies(KbHandle* hh, float* out) {
-  Handle* h = reinterpret_cast<Handle*>(hh);
-  std::vector<uint32_t> buf;
-  int rc = fetchBlobs(h, &buf);
-  if (rc) return rc;
-  const Layout& L = h->L;
-  for (int e = 0; e < h->numEnvs; ++e) {
-    const uint32_t* w = buf.data() + (size_t)e * L.blobWords;
+  const Handle* h = reinterpret_cast<Handle*>(hh);
+  return fetchBlobs(h, "kb_get_proxies", [&](int e, const uint32_t* w) {
+    const Layout& L = h->L;
     const int np = h->hostNumProxies[w[L.oHdr + H_SCENE]];
     std::memset(out + (size_t)e * L.P * 4, 0, sizeof(float) * 4 * L.P);
     std::memcpy(out + (size_t)e * L.P * 4, w + L.oFat, sizeof(float) * 4 * np);
-  }
-  return KB_OK;
+  });
 }
 
 int kb_get_controllers(KbHandle* hh, double* ctrl, double* light) {
-  Handle* h = reinterpret_cast<Handle*>(hh);
-  std::vector<uint32_t> buf;
-  int rc = fetchBlobs(h, &buf);
-  if (rc) return rc;
-  const Layout& L = h->L;
-  for (int e = 0; e < h->numEnvs; ++e) {
-    const uint32_t* w = buf.data() + (size_t)e * L.blobWords;
+  const Handle* h = reinterpret_cast<Handle*>(hh);
+  return fetchBlobs(h, "kb_get_controllers", [&](int e, const uint32_t* w) {
+    const Layout& L = h->L;
     if (ctrl) std::memcpy(ctrl + (size_t)e * L.N * 4, w + L.oCtrl, sizeof(double) * 4 * L.N);
     if (light) std::memcpy(light + (size_t)e * L.L, w + L.oLight, sizeof(double) * L.L);
-  }
-  return KB_OK;
+  });
 }
 
 int kb_get_state(KbHandle* hh, void* out) {
   Handle* h = reinterpret_cast<Handle*>(hh);
-  if (!h || !out) return fail(KB_ERR_INVALID, "kb_get_state: null");
-  CUDA_TRY(cudaSetDevice(h->device));
-  CUDA_TRY(cudaDeviceSynchronize());
-  CUDA_TRY(cudaMemcpy(out, h->dBlobs, (size_t)h->numEnvs * h->L.blobWords * 4, cudaMemcpyDeviceToHost));
+  if (const int rc = enter(h, "kb_get_state", true)) return rc;
+  if (!out) return fail(KB_ERR_INVALID, "kb_get_state: null");
+  CUDA_TRY(cudaMemcpy(out, h->dBlobs.get(), (size_t)h->numEnvs * h->L.blobWords * 4, cudaMemcpyDeviceToHost));
   return KB_OK;
 }
 
 int kb_set_state(KbHandle* hh, const void* in) {
   Handle* h = reinterpret_cast<Handle*>(hh);
-  if (!h || !in) return fail(KB_ERR_INVALID, "kb_set_state: null");
-  CUDA_TRY(cudaSetDevice(h->device));
-  CUDA_TRY(cudaDeviceSynchronize());
-  CUDA_TRY(cudaMemcpy(h->dBlobs, in, (size_t)h->numEnvs * h->L.blobWords * 4, cudaMemcpyHostToDevice));
+  if (const int rc = enter(h, "kb_set_state", true)) return rc;
+  if (!in) return fail(KB_ERR_INVALID, "kb_set_state: null");
+  CUDA_TRY(cudaMemcpy(h->dBlobs.get(), in, (size_t)h->numEnvs * h->L.blobWords * 4, cudaMemcpyHostToDevice));
   return KB_OK;
 }
 
@@ -1670,8 +1652,9 @@ int kb_set_state(KbHandle* hh, const void* in) {
 // debug builds only: cycles per phase of the last kb_step, u64[E][KB_PROF_SLOTS]
 int kb_get_profile(KbHandle* hh, unsigned long long* out) {
   Handle* h = reinterpret_cast<Handle*>(hh);
-  CUDA_TRY(cudaDeviceSynchronize());
-  CUDA_TRY(cudaMemcpy(out, h->dProf, sizeof(unsigned long long) * KB_PROF_SLOTS * (size_t)h->numEnvs, cudaMemcpyDeviceToHost));
+  if (const int rc = enter(h, "kb_get_profile", true)) return rc;
+  CUDA_TRY(cudaMemcpy(out, h->dProf.get(), sizeof(unsigned long long) * KB_PROF_SLOTS * (size_t)h->numEnvs,
+                      cudaMemcpyDeviceToHost));
   return KB_OK;
 }
 #endif
@@ -1723,7 +1706,8 @@ int kb_get_launch_config(const KbHandle* hh, KbLaunchConfig* cfg) {
 // ---- task layer (extension beyond the reference; include/kb_b200.h "Task layer") -------------------------
 int kb_set_task(KbHandle* hh, const KbTaskDef* task, const double* target) {
   Handle* h = reinterpret_cast<Handle*>(hh);
-  if (!h || !task) return fail(KB_ERR_INVALID, "kb_set_task: null");
+  if (const int rc = enter(h, "kb_set_task", true)) return rc;
+  if (!task) return fail(KB_ERR_INVALID, "kb_set_task: null");
   if (task->mode != KB_TASK_CONST && task->mode != KB_TASK_OBJECT_TO_TARGET && task->mode != KB_TASK_SWARM_TO_TARGET)
     return fail(KB_ERR_INVALID, "kb_set_task: unknown mode");
   const int minM = *std::min_element(h->hostNumObjects.begin(), h->hostNumObjects.end());
@@ -1731,19 +1715,17 @@ int kb_set_task(KbHandle* hh, const KbTaskDef* task, const double* target) {
   if (task->mode == KB_TASK_OBJECT_TO_TARGET && (task->object < 0 || task->object >= minM))
     return fail(KB_ERR_INVALID, "kb_set_task: object index out of range (every scene of the batch must have the object)");
   if (task->mode == KB_TASK_SWARM_TO_TARGET && minN < 1) return fail(KB_ERR_INVALID, "kb_set_task: a scene without kilobots");
-  CUDA_TRY(cudaSetDevice(h->device));
-  CUDA_TRY(cudaDeviceSynchronize());
   const size_t E = (size_t)h->numEnvs;
   std::vector<double> ts(E * KB_TASK_WORDS, 0.0);
   if (!target) {  // keep the current targets
-    CUDA_TRY(cudaMemcpy(ts.data(), h->dTask, sizeof(double) * ts.size(), cudaMemcpyDeviceToHost));
+    CUDA_TRY(cudaMemcpy(ts.data(), h->dTask.get(), sizeof(double) * ts.size(), cudaMemcpyDeviceToHost));
     for (size_t e = 0; e < E; ++e)
       for (int k = 3; k < KB_TASK_WORDS; ++k) ts[e * KB_TASK_WORDS + k] = 0.0;
   } else {
     for (size_t e = 0; e < E; ++e)
       for (int k = 0; k < 3; ++k) ts[e * KB_TASK_WORDS + k] = target[e * 3 + k];
   }
-  CUDA_TRY(cudaMemcpy(h->dTask, ts.data(), sizeof(double) * ts.size(), cudaMemcpyHostToDevice));
+  CUDA_TRY(cudaMemcpy(h->dTask.get(), ts.data(), sizeof(double) * ts.size(), cudaMemcpyHostToDevice));
   TaskConst& t = h->task;
   t.mode = task->mode;
   t.object = task->object;
@@ -1760,12 +1742,11 @@ int kb_set_task(KbHandle* hh, const KbTaskDef* task, const double* target) {
 
 int kb_get_episode_stats(KbHandle* hh, double* out) {
   Handle* h = reinterpret_cast<Handle*>(hh);
-  if (!h || !out) return fail(KB_ERR_INVALID, "kb_get_episode_stats: null");
-  CUDA_TRY(cudaSetDevice(h->device));
-  CUDA_TRY(cudaDeviceSynchronize());
+  if (const int rc = enter(h, "kb_get_episode_stats", true)) return rc;
+  if (!out) return fail(KB_ERR_INVALID, "kb_get_episode_stats: null");
   const size_t E = (size_t)h->numEnvs;
   std::vector<double> ts(E * KB_TASK_WORDS);
-  CUDA_TRY(cudaMemcpy(ts.data(), h->dTask, sizeof(double) * ts.size(), cudaMemcpyDeviceToHost));
+  CUDA_TRY(cudaMemcpy(ts.data(), h->dTask.get(), sizeof(double) * ts.size(), cudaMemcpyDeviceToHost));
   for (size_t e = 0; e < E; ++e)
     for (int k = 0; k < KB_EPISODE_STATS; ++k) out[e * KB_EPISODE_STATS + k] = ts[e * KB_TASK_WORDS + 3 + k];
   return KB_OK;
@@ -1773,10 +1754,10 @@ int kb_get_episode_stats(KbHandle* hh, double* out) {
 
 int kb_reduce_episode_stats(KbHandle* hh, double* out_device, void* stream) {
   Handle* h = reinterpret_cast<Handle*>(hh);
-  if (!h || !out_device) return fail(KB_ERR_INVALID, "kb_reduce_episode_stats: null");
-  CUDA_TRY(cudaSetDevice(h->device));
-  kb_reduce_stats_kernel<<<1, 1024, 0, (cudaStream_t)stream>>>(h->dTask, h->dBlobs, h->L.blobWords, h->L.oHdr + H_STATUS,
-                                                              h->numEnvs, out_device);
+  if (const int rc = enter(h, "kb_reduce_episode_stats", false)) return rc;
+  if (!out_device) return fail(KB_ERR_INVALID, "kb_reduce_episode_stats: null");
+  kb_reduce_stats_kernel<<<1, 1024, 0, (cudaStream_t)stream>>>(h->dTask.get(), h->dBlobs.get(), h->L.blobWords,
+                                                              h->L.oHdr + H_STATUS, h->numEnvs, out_device);
   CUDA_TRY(cudaGetLastError());
   return KB_OK;
 }
@@ -1905,16 +1886,15 @@ int kb_selftest_exact_math(int32_t device, int32_t div_rounds_log2, uint64_t* mi
     return fail(KB_ERR_NO_DEVICE, "kb_selftest_exact_math: no CUDA device");
   }
   if (device >= 0) CUDA_TRY(cudaSetDevice(device));
-  unsigned long long* d = nullptr;
-  CUDA_TRY(cudaMalloc(&d, 6 * sizeof(unsigned long long)));
-  CUDA_TRY(cudaMemset(d, 0, 6 * sizeof(unsigned long long)));
-  kb_selftest_math_kernel<<<148 * 8, 256>>>(1 << div_rounds_log2, d);
+  DevBuf<unsigned long long> d;
+  CUDA_TRY(devAlloc(d, 6));
+  CUDA_TRY(cudaMemset(d.get(), 0, 6 * sizeof(unsigned long long)));
+  kb_selftest_math_kernel<<<148 * 8, 256>>>(1 << div_rounds_log2, d.get());
   CUDA_TRY(cudaGetLastError());
-  kb_selftest_pair_kernel<<<148 * 4, 256>>>(d);
+  kb_selftest_pair_kernel<<<148 * 4, 256>>>(d.get());
   CUDA_TRY(cudaGetLastError());
   CUDA_TRY(cudaDeviceSynchronize());
-  CUDA_TRY(cudaMemcpy(mismatches, d, 6 * sizeof(unsigned long long), cudaMemcpyDeviceToHost));
-  CUDA_TRY(cudaFree(d));
+  CUDA_TRY(cudaMemcpy(mismatches, d.get(), 6 * sizeof(unsigned long long), cudaMemcpyDeviceToHost));
   return KB_OK;
 }
 
@@ -1976,25 +1956,19 @@ int kb_probe_geometry(int32_t device, int32_t op, int32_t n, const KbProbeShape*
     return fail(KB_ERR_NO_DEVICE, "kb_probe_geometry: no CUDA device");
   }
   if (device >= 0) CUDA_TRY(cudaSetDevice(device));
-  ProxyConst* dPx = nullptr;
-  KbProbeCase* dCases = nullptr;
-  uint32_t* dOut = nullptr;
-  const size_t outBytes = (size_t)n * KB_PROBE_OUT_WORDS * 4;
-  cudaError_t e = cudaMalloc(&dPx, sizeof(ProxyConst) * px.size());
-  if (e == cudaSuccess) e = cudaMalloc(&dCases, sizeof(KbProbeCase) * (size_t)n);
-  if (e == cudaSuccess) e = cudaMalloc(&dOut, outBytes);
-  if (e == cudaSuccess) e = cudaMemcpy(dPx, px.data(), sizeof(ProxyConst) * px.size(), cudaMemcpyHostToDevice);
-  if (e == cudaSuccess) e = cudaMemcpy(dCases, cases, sizeof(KbProbeCase) * (size_t)n, cudaMemcpyHostToDevice);
-  if (e == cudaSuccess) e = cudaMemset(dOut, 0, outBytes);
-  if (e == cudaSuccess) {
-    e = kbLaunchProbeGeometry(op, n, dPx, dCases, dOut);
-  }
-  if (e == cudaSuccess) e = cudaDeviceSynchronize();
-  if (e == cudaSuccess) e = cudaMemcpy(out, dOut, outBytes, cudaMemcpyDeviceToHost);
-  cudaFree(dPx);
-  cudaFree(dCases);
-  cudaFree(dOut);
-  if (e != cudaSuccess) return fail(KB_ERR_CUDA, std::string("kb_probe_geometry: ") + cudaGetErrorString(e));
+  DevBuf<ProxyConst> dPx;
+  DevBuf<KbProbeCase> dCases;
+  DevBuf<uint32_t> dOut;
+  const size_t outWords = (size_t)n * KB_PROBE_OUT_WORDS;
+  CUDA_TRY(devAlloc(dPx, px.size()));
+  CUDA_TRY(devAlloc(dCases, n));
+  CUDA_TRY(devAlloc(dOut, outWords));
+  CUDA_TRY(cudaMemcpy(dPx.get(), px.data(), sizeof(ProxyConst) * px.size(), cudaMemcpyHostToDevice));
+  CUDA_TRY(cudaMemcpy(dCases.get(), cases, sizeof(KbProbeCase) * (size_t)n, cudaMemcpyHostToDevice));
+  CUDA_TRY(cudaMemset(dOut.get(), 0, outWords * 4));
+  CUDA_TRY(kbLaunchProbeGeometry(op, n, dPx.get(), dCases.get(), dOut.get()));
+  CUDA_TRY(cudaDeviceSynchronize());
+  CUDA_TRY(cudaMemcpy(out, dOut.get(), outWords * 4, cudaMemcpyDeviceToHost));
   return KB_OK;
 }
 
@@ -2002,30 +1976,29 @@ int kb_probe_geometry(int32_t device, int32_t op, int32_t n, const KbProbeShape*
 int kb_render(KbHandle* hh, const int32_t* env_ids, int32_t num_images, int32_t width, int32_t height, uint8_t* rgb,
               void* stream) {
   Handle* h = reinterpret_cast<Handle*>(hh);
-  if (!h || !env_ids || !rgb || num_images < 1 || width < 1 || height < 1)
+  if (const int rc = enter(h, "kb_render", false)) return rc;
+  if (!env_ids || !rgb || num_images < 1 || width < 1 || height < 1)
     return fail(KB_ERR_INVALID, "kb_render: invalid arguments");
   if (num_images > 65535) return fail(KB_ERR_INVALID, "kb_render: at most 65535 images per call");
   for (int i = 0; i < num_images; ++i)
     if (env_ids[i] < 0 || env_ids[i] >= h->numEnvs) return fail(KB_ERR_INVALID, "kb_render: env id out of range");
-  CUDA_TRY(cudaSetDevice(h->device));
   cudaStream_t st = (cudaStream_t)stream;
   if (num_images > h->renderIdsCap) {
     CUDA_TRY(cudaStreamSynchronize(st));
-    cudaFree(h->dRenderIds);
-    h->dRenderIds = nullptr;
-    CUDA_TRY(cudaMalloc(&h->dRenderIds, sizeof(int32_t) * (size_t)num_images));
+    h->renderIdsCap = 0;
+    CUDA_TRY(devAlloc(h->dRenderIds, num_images));
     h->renderIdsCap = num_images;
   }
-  CUDA_TRY(cudaMemcpyAsync(h->dRenderIds, env_ids, sizeof(int32_t) * (size_t)num_images, cudaMemcpyHostToDevice, st));
+  CUDA_TRY(cudaMemcpyAsync(h->dRenderIds.get(), env_ids, sizeof(int32_t) * (size_t)num_images, cudaMemcpyHostToDevice, st));
   RenderArgs a;
   a.L = h->L;
-  a.blobs = h->dBlobs;
-  a.envScene = h->dEnvScene;
-  a.proxies = h->dProxies;
-  a.bodies = h->dBodies;
-  a.scenes = h->dScenes;
-  a.lights = h->dLights;
-  a.envIds = h->dRenderIds;
+  a.blobs = h->dBlobs.get();
+  a.envScene = h->dEnvScene.get();
+  a.proxies = h->dProxies.get();
+  a.bodies = h->dBodies.get();
+  a.scenes = h->dScenes.get();
+  a.lights = h->dLights.get();
+  a.envIds = h->dRenderIds.get();
   a.numImages = num_images;
   a.width = width;
   a.height = height;
@@ -2069,14 +2042,14 @@ int kb_local_observation(KbHandle* hh, const KbLocalObsDef* def, const uint8_t* 
   if (D < 0) return D;
   if (!out) return fail(KB_ERR_INVALID, "kb_local_observation: null out");
   if (h->numEnvs == 0 || h->L.N == 0) return KB_OK;
-  CUDA_TRY(cudaSetDevice(h->device));
+  if (const int rc = enter(h, "kb_local_observation", false)) return rc;
   LocalArgs a;
   a.L = h->L;
-  a.blobs = h->dBlobs;
-  a.envScene = h->dEnvScene;
-  a.bodies = h->dBodies;
-  a.scenes = h->dScenes;
-  a.lights = h->dLights;
+  a.blobs = h->dBlobs.get();
+  a.envScene = h->dEnvScene.get();
+  a.bodies = h->dBodies.get();
+  a.scenes = h->dScenes.get();
+  a.lights = h->dLights.get();
   a.mask = mask;
   a.out = out;
   a.numEnvs = h->numEnvs;
