@@ -19,6 +19,7 @@
 #pragma once
 #include "kb_narrow.cuh"
 #include "kb_sample.cuh"
+#include "kb_solver.cuh"
 
 namespace kb {
 
@@ -290,11 +291,9 @@ struct Sim {
         const BodyConst* c = bc + b;
         bc4(b) = make_float4(__ldg(&c->invMass), __ldg(&c->invI), __ldg(&c->lcx), __ldg(&c->lcy));
         sts_u8(wa(L.sBk) + (uint32_t)b, (uint32_t)__ldg(&c->kind));
-        // b2Island::Solve damping factors (SimplePhototaxisKilobot's linearDamping = 0, lib/kilobot.py:203, is
-        // folded into the template)
+        // (SimplePhototaxisKilobot's linearDamping = 0, lib/kilobot.py:203, is folded into the template)
         const float h = L.dt, ld = __ldg(&c->linearDamping), ad = __ldg(&c->angularDamping);
-        damp(b) = L.dampingMode == 0 ? make_float2(1.0f / (1.0f + h * ld), 1.0f / (1.0f + h * ad))
-                                     : make_float2(b2clamp(1.0f - h * ld, 0.0f, 1.0f), b2clamp(1.0f - h * ad, 0.0f, 1.0f));
+        damp(b) = make_float2(kb_damping(L.dampingMode, h, ld), kb_damping(L.dampingMode, h, ad));
       } else {
         bc4(b) = make_float4(0.0f, 0.0f, 0.0f, 0.0f);
         pos4(b) = make_float4(0.0f, 0.0f, 0.0f, 0.0f);
@@ -552,46 +551,16 @@ struct Sim {
     const float radiusA = pradius(pa), radiusB = pradius(pb);
     const float4 cA4 = pos4(bA), cB4 = pos4(bB);
     const float4 kA = bc4(bA), kB = bc4(bB);
-    const float mA = kA.x, iA = kA.y, mB = kB.x, iB = kB.y;
-    const V2 cA = mk(cA4.x, cA4.y), cB = mk(cB4.x, cB4.y);
     // xf from (c, a): q == the body's current xf.q (b2Rot::Set(sweep.a) is what produced it)
-    Xf xfA, xfB;
     const float4 xa = xf4(bA), xb = xf4(bB);
-    xfA.q.s = xa.z; xfA.q.c = xa.w;
-    xfB.q.s = xb.z; xfB.q.c = xb.w;
-    xfA.p = cA - rmul(xfA.q, mk(kA.z, kA.w));
-    xfB.p = cB - rmul(xfB.q, mk(kB.z, kB.w));
-    // b2WorldManifold::Initialize
-    V2 normal, pt;
-    const V2 lp = mk(r0.z, r0.w), ln = mk(r0.x, r0.y);
-    const V2 mp0 = mk(r1.x, r1.y);
-    if (type == MANIFOLD_CIRCLES) {
-      normal = mk(1.0f, 0.0f);
-      V2 pointA = xmul(xfA, lp);
-      V2 pointB = xmul(xfB, mp0);
-      if (distsq(pointA, pointB) > KB_EPS * KB_EPS) {
-        normal = pointB - pointA;
-        normalize(normal);
-      }
-      V2 a = pointA + radiusA * normal;
-      V2 b = pointB - radiusB * normal;
-      pt = 0.5f * (a + b);
-    } else {
-      normal = rmul(xfA.q, ln);
-      V2 planePoint = xmul(xfA, lp);
-      V2 clipPoint = xmul(xfB, mp0);
-      V2 a = clipPoint + (radiusA - dot(clipPoint - planePoint, normal)) * normal;
-      V2 b = clipPoint - radiusB * normal;
-      pt = 0.5f * (a + b);
-    }
-    const V2 rA = pt - cA;
-    const V2 rB = pt - cB;
-    const float rnA = cross(rA, normal);
-    const float rnB = cross(rB, normal);
-    const float kNormal = mA + mB + iA * rnA * rnA + iB * rnB * rnB;
-    const float nMass = kNormal > 0.0f ? 1.0f / kNormal : 0.0f;
-    rec4(2 * e) = make_float4(normal.x, normal.y, nMass, r1.z);  // warm start: dtRatio (== 1) * normalImpulse
-    rec4(2 * e + 1) = make_float4(rA.x, rA.y, rB.x, rB.y);
+    Rot qA, qB;
+    qA.s = xa.z; qA.c = xa.w;
+    qB.s = xb.z; qB.c = xb.w;
+    float4 v0, v1;   // warm start with r1.z: dtRatio (== 1) * normalImpulse
+    kb_init_simple(mk(cA4.x, cA4.y), mk(cB4.x, cB4.y), qA, qB, mk(kA.z, kA.w), mk(kB.z, kB.w), r0, mk(r1.x, r1.y), type, radiusA,
+                   radiusB, kA.x, kA.y, kB.x, kB.y, r1.z, v0, v1);
+    rec4(2 * e) = v0;
+    rec4(2 * e + 1) = v1;
   }
 
   // b2ContactSolver::WarmStart
@@ -600,84 +569,21 @@ struct Sim {
     const float4 r0 = rec4(2 * e), r1 = rec4(2 * e + 1);
     const float4 kA = bc4(bA), kB = bc4(bB);
     float4 vA = vel4(bA), vB = vel4(bB);
-    const V2 normal = mk(r0.x, r0.y);
-    const V2 tangent = cross(normal, 1.0f);
-    const V2 rA = mk(r1.x, r1.y), rB = mk(r1.z, r1.w);
-    const V2 P = r0.w * normal + 0.0f * tangent;
-    vA.z -= kA.y * cross(rA, P);
-    vA.x = vA.x - kA.x * P.x;
-    vA.y = vA.y - kA.x * P.y;
-    vB.z += kB.y * cross(rB, P);
-    vB.x = vB.x + kB.x * P.x;
-    vB.y = vB.y + kB.x * P.y;
+    kb_warm_start_simple(vA, vB, r0, r1, kA.x, kA.y, kB.x, kB.y);
     vel4(bA) = vA;  // the static slot receives +0 velocities (invMass = invI = 0): harmless
     vel4(bB) = vB;
   }
 
-  // b2ContactSolver::SolveVelocityConstraints (the tangent row contributes exactly zero: friction == 0)
+  // b2ContactSolver::SolveVelocityConstraints
   __device__ __forceinline__ void solveVelocitySimple(int e, uint32_t item) {
     const int bA = IT_BA(item), bB = IT_BB(item);
     const float4 r0 = rec4(2 * e), r1 = rec4(2 * e + 1);
     const float4 kA = bc4(bA), kB = bc4(bB);
     float4 a4 = vel4(bA), b4 = vel4(bB);
-    const V2 normal = mk(r0.x, r0.y);
-    const V2 rA0 = mk(r1.x, r1.y), rB0 = mk(r1.z, r1.w);
-    const V2 Av = mk(a4.x, a4.y), Bv = mk(b4.x, b4.y);
-    V2 dv = Bv + cross(b4.z, rB0) - Av - cross(a4.z, rA0);
-    float vn = dot(dv, normal);
-    float ni = r0.w;
-    float lambda = -r0.z * (vn - 0.0f);
-    float newImpulse = b2max(ni + lambda, 0.0f);
-    lambda = newImpulse - ni;
-    V2 P = lambda * normal;
-    const V2 Av2 = Av - kA.x * P;
-    a4.z -= kA.y * cross(rA0, P);
-    const V2 Bv2 = Bv + kB.x * P;
-    b4.z += kB.y * cross(rB0, P);
-    a4.x = Av2.x; a4.y = Av2.y;
-    b4.x = Bv2.x; b4.y = Bv2.y;
+    const float newImpulse = kb_solve_velocity_simple(a4, b4, r0, r1, kA.x, kA.y, kB.x, kB.y);
     vel4(bA) = a4;
     vel4(bB) = b4;
     rec4(2 * e).set(3, newImpulse);
-  }
-
-  // the same two with the entry's records (r0, r1), inverse masses kk = (mA, iA, mB, iB) and body rows in registers
-  __device__ __forceinline__ void warmStartCached(SF4 rowA, SF4 rowB, const float4& r0, const float4& r1, const float4& kk) {
-    float4 vA = rowA, vB = rowB;
-    const V2 normal = mk(r0.x, r0.y);
-    const V2 tangent = cross(normal, 1.0f);
-    const V2 rA = mk(r1.x, r1.y), rB = mk(r1.z, r1.w);
-    const V2 P = r0.w * normal + 0.0f * tangent;
-    vA.z -= kk.y * cross(rA, P);
-    vA.x = vA.x - kk.x * P.x;
-    vA.y = vA.y - kk.x * P.y;
-    vB.z += kk.w * cross(rB, P);
-    vB.x = vB.x + kk.z * P.x;
-    vB.y = vB.y + kk.z * P.y;
-    rowA = vA;
-    rowB = vB;
-  }
-  __device__ __forceinline__ float solveVelocityCached(SF4 rowA, SF4 rowB, const float4& r0, const float4& r1, const float4& kk) {
-    float4 a4 = rowA, b4 = rowB;
-    const V2 normal = mk(r0.x, r0.y);
-    const V2 rA0 = mk(r1.x, r1.y), rB0 = mk(r1.z, r1.w);
-    const V2 Av = mk(a4.x, a4.y), Bv = mk(b4.x, b4.y);
-    V2 dv = Bv + cross(b4.z, rB0) - Av - cross(a4.z, rA0);
-    float vn = dot(dv, normal);
-    float ni = r0.w;
-    float lambda = -r0.z * (vn - 0.0f);
-    float newImpulse = b2max(ni + lambda, 0.0f);
-    lambda = newImpulse - ni;
-    V2 P = lambda * normal;
-    const V2 Av2 = Av - kk.x * P;
-    a4.z -= kk.y * cross(rA0, P);
-    const V2 Bv2 = Bv + kk.z * P;
-    b4.z += kk.w * cross(rB0, P);
-    a4.x = Av2.x; a4.y = Av2.y;
-    b4.x = Bv2.x; b4.y = Bv2.y;
-    rowA = a4;
-    rowB = b4;
-    return newImpulse;
   }
 
   // b2ContactSolver::StoreImpulses, then re-purpose the records for the position solver
@@ -690,7 +596,8 @@ struct Sim {
     rec4(2 * e) = r0;
     rec4(2 * e + 1) = make_float4(pradius(CW_PA(w)), pradius(CW_PB(w)), u2f(tp & 0xFFu), 0.0f);
     // the position sweeps decide once per solve, not once per row-step, whether this entry is the
-    // kilobot-against-kilobot case of solvePositionSimple (the predicate is copied from there)
+    // kilobot-against-kilobot case: a circle manifold for which solvePositionSimple would rotate neither body (the
+    // predicates are copied from there).  solvePositionFast takes those entries, solvePositionSimple the others.
     const int bA = IT_BA(item), bB = IT_BB(item);
     const float4 kA = bc4(bA), kB = bc4(bB);
     const bool trigA = bA != S && ((int)(tp & 0xFFu) != MANIFOLD_CIRCLES || r0.z != 0.0f || r0.w != 0.0f ||
@@ -726,75 +633,23 @@ struct Sim {
     const int bA = IT_BA(item), bB = IT_BB(item);
     const float4 r0 = rec4(2 * e), r1 = rec4(2 * e + 1);
     const float4 kA = bc4(bA), kB = bc4(bB);
-    const float mA = kA.x, iA = kA.y, mB = kB.x, iB = kB.y;
-    const V2 lcA = mk(kA.z, kA.w), lcB = mk(kB.z, kB.w);
-    float4 pA4 = pos4(bA), pB4 = pos4(bB);
-    V2 cA = mk(pA4.x, pA4.y), cB = mk(pB4.x, pB4.y);
-    float aA = pA4.z, aB = pB4.z;
-    const V2 ln = mk(r0.x, r0.y);
-    const V2 lp = mk(r0.z, r0.w);
-    const float radiusA = r1.x, radiusB = r1.y;
+    const float4 pA4 = pos4(bA), pB4 = pos4(bB);
     const int type = (int)f2u(r1.z);
     // a rotation is only needed where it multiplies something non-zero (0 * finite == 0 exactly)
-    const bool trigA = bA != S && (type != MANIFOLD_CIRCLES || lp.x != 0.0f || lp.y != 0.0f || lcA.x != 0.0f ||
-                                   lcA.y != 0.0f);
-    const bool trigB = bB != S && (lcB.x != 0.0f || lcB.y != 0.0f);
-    const V2 mpj = mk(0.0f, 0.0f);
-    V2 normal, point;
-    float separation;
-    if (type == MANIFOLD_CIRCLES && bA != S && !trigA && !trigB) {
-      // kilobot against kilobot: local centres and local points are all zero, so xf.p == c and
-      // b2Mul(xf, 0) == c exactly (up to the sign of a zero, which no later operation can observe).
-      // (bA == S with e_circles is a chain-vertex contact: its local point is the vertex, not zero.)
-      normal = cB - cA;
-      normalize(normal);
-      point = 0.5f * (cA + cB);
-      separation = dot(cB - cA, normal) - radiusA - radiusB;
-    } else {
-      Xf xfA, xfB;
-      if (trigA) xfA.q = rot_set(aA);
-      else { xfA.q.s = 0.0f; xfA.q.c = 1.0f; }
-      if (trigB) xfB.q = rot_set(aB);
-      else { xfB.q.s = 0.0f; xfB.q.c = 1.0f; }
-      xfA.p = cA - rmul(xfA.q, lcA);
-      xfB.p = cB - rmul(xfB.q, lcB);
-      if (type == MANIFOLD_CIRCLES) {
-        V2 pointA = xmul(xfA, lp);
-        V2 pointB = xmul(xfB, mpj);
-        normal = pointB - pointA;
-        normalize(normal);
-        point = 0.5f * (pointA + pointB);
-        separation = dot(pointB - pointA, normal) - radiusA - radiusB;
-      } else {
-        normal = rmul(xfA.q, ln);
-        V2 planePoint = xmul(xfA, lp);
-        V2 clipPoint = xmul(xfB, mpj);
-        separation = dot(clipPoint - planePoint, normal) - radiusA - radiusB;
-        point = clipPoint;
-      }
-    }
-    const bool ok = separation >= -3.0f * KB_LINEAR_SLOP;
-    const float C = b2clamp(KB_BAUMGARTE * (separation + KB_LINEAR_SLOP), -KB_MAX_LINEAR_CORRECTION, 0.0f);
-    // C == 0 (not penetrating beyond the slop): the impulse is -0 / K and moves nothing
-    if (C == 0.0f) return ok;
-    const V2 rA = point - cA;
-    const V2 rB = point - cB;
-    const float rnA = cross(rA, normal);
-    const float rnB = cross(rB, normal);
-    const float K = mA + mB + iA * rnA * rnA + iB * rnB * rnB;
-    const float impulse = K > 0.0f ? -C / K : 0.0f;
-    const V2 P = impulse * normal;
-    cA = cA - mA * P;
-    aA -= iA * cross(rA, P);
-    cB = cB + mB * P;
-    aB += iB * cross(rB, P);
-    if (bA != S) {
-      pA4.x = cA.x; pA4.y = cA.y; pA4.z = aA;
-      pos4(bA) = pA4;
-    }
-    if (bB != S) {
-      pB4.x = cB.x; pB4.y = cB.y; pB4.z = aB;
-      pos4(bB) = pB4;
+    const bool trigA = bA != S && (type != MANIFOLD_CIRCLES || r0.z != 0.0f || r0.w != 0.0f || kA.z != 0.0f || kA.w != 0.0f);
+    const bool trigB = bB != S && (kB.z != 0.0f || kB.w != 0.0f);
+    Rot qA, qB;
+    if (trigA) qA = rot_set(pA4.z);
+    else { qA.s = 0.0f; qA.c = 1.0f; }
+    if (trigB) qB = rot_set(pB4.z);
+    else { qB.s = 0.0f; qB.c = 1.0f; }
+    float4 a1, b1;
+    bool moved;
+    const bool ok = kb_position_simple(pA4, pB4, qA, qB, mk(kA.z, kA.w), mk(kB.z, kB.w), r0, type, r1.x, r1.y, kA.x, kA.y, kB.x, kB.y,
+                                       KB_BAUMGARTE, -3.0f * KB_LINEAR_SLOP, true, a1, b1, moved);
+    if (moved) {
+      if (bA != S) pos4(bA) = a1;
+      if (bB != S) pos4(bB) = b1;
     }
     return ok;
   }
@@ -1456,7 +1311,10 @@ struct Sim {
         uint32_t item = k < nOrd ? ent(k) : IT_NONE;
         for (int r = 0; r < nRowsU; ++r) {
           if (r == row0) {
-            warmStartCached(vA, vB, q0, q1, kk);
+            float4 a4 = vA, b4 = vB;
+            kb_warm_start_simple(a4, b4, q0, q1, kk.x, kk.y, kk.z, kk.w);
+            vA = a4;
+            vB = b4;
           } else if (IT_ROW(item) == r) {
             const uint32_t cur = item;
             const int kc = k;
@@ -1473,7 +1331,10 @@ struct Sim {
         uint32_t item = k < nOrd ? ent(k) : IT_NONE;
         for (int r = 0; r < nRowsU; ++r) {
           if (r == row0) {
-            q0.w = solveVelocityCached(vA, vB, q0, q1, kk);
+            float4 a4 = vA, b4 = vB;
+            q0.w = kb_solve_velocity_simple(a4, b4, q0, q1, kk.x, kk.y, kk.z, kk.w);
+            vA = a4;
+            vB = b4;
           } else if (IT_ROW(item) == r) {
             const uint32_t cur = item;
             const int kc = k;
@@ -1499,20 +1360,7 @@ struct Sim {
       if (isl(b) < 0) continue;
       float4 p = pos4(b);
       float4 v = vel4(b);
-      V2 translation = h * mk(v.x, v.y);
-      if (dot(translation, translation) > KB_MAX_TRANSLATION_SQ) {
-        float ratio = KB_MAX_TRANSLATION / length(translation);
-        v.x *= ratio;
-        v.y *= ratio;
-      }
-      float rotation = h * v.z;
-      if (rotation * rotation > KB_MAX_ROTATION_SQ) {
-        float ratio = KB_MAX_ROTATION / b2abs(rotation);
-        v.z *= ratio;
-      }
-      p.x += h * v.x;
-      p.y += h * v.y;
-      p.z += h * v.z;
+      kb_integrate_position(p, v, h);
       pos4(b) = p;
       vel4(b) = v;
     }
@@ -1568,15 +1416,7 @@ struct Sim {
       V2 o = mk(p.x, p.y) - rmul(q, mk(k.z, k.w));
       xf4(b) = make_float4(o.x, o.y, q.s, q.c);
       if (L.enableSleep) {
-        const float4 v = vel4(b);
-        const float linTolSqr = KB_LIN_SLEEP_TOL * KB_LIN_SLEEP_TOL;
-        const float angTolSqr = KB_ANG_SLEEP_TOL * KB_ANG_SLEEP_TOL;
-        float st;
-        if (v.z * v.z > angTolSqr || dot(mk(v.x, v.y), mk(v.x, v.y)) > linTolSqr) {
-          st = 0.0f;
-        } else {
-          st = p.w + h;
-        }
+        const float st = kb_sleep_time(vel4(b), p.w, h);
         pos4(b).set(3, st);
         if (!(st >= KB_TIME_TO_SLEEP)) islflag(island).atomOr(4u);  // minSleepTime < timeToSleep
       }

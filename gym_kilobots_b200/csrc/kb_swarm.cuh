@@ -26,9 +26,9 @@
 //     turns before it run, hand-over on named barriers (see "relay" below and DESIGN.md section 6).
 // Scope of this tier (checked by kb_create): every dynamic body is a kilobot (one circle fixture at the body origin,
 // friction 0, restitution 0), no pushable objects (M = 0); the table's chain edges are the only other proxies.
-// All constraints are therefore "simple" (one manifold point, frictionless, no restitution): kb_step.cuh's
-// initSimple / warmStartSimple / solveVelocitySimple / solvePositionSimple arithmetic, restated here on the swarm
-// layout; continuous collision (b2World::SolveTOI) is the table-edge-against-circle case of kb_toi.cuh.
+// All constraints are therefore "simple" (one manifold point, frictionless, no restitution): the arithmetic of
+// kb_solver.cuh, shared with the lane-group tier, on the swarm layout; continuous collision (b2World::SolveTOI) is the
+// table-edge-against-circle case of kb_toi.cuh.
 #pragma once
 #include "kb_toi.cuh"
 
@@ -415,90 +415,25 @@ struct Swarm {
     const float4 cA4 = pos4(bA), cB4 = pos4(bB);
     const float2 kA = massOf(bA), kB = massOf(bB);
     const float mA = kA.x, iA = kA.y, mB = kB.x, iB = kB.y;
-    const V2 cA = mk(cA4.x, cA4.y), cB = mk(cB4.x, cB4.y);
-    Xf xfA, xfB;
     const float2 qa = q2(bA), qb = q2(bB);
-    xfA.q.s = qa.x; xfA.q.c = qa.y;
-    xfB.q.s = qb.x; xfB.q.c = qb.y;
-    xfA.p = cA - rmul(xfA.q, mk(0.0f, 0.0f));
-    xfB.p = cB - rmul(xfB.q, mk(0.0f, 0.0f));
-    V2 normal, pt;
-    const V2 lp = mk(r0.z, r0.w), ln = mk(r0.x, r0.y);
-    const V2 mp0 = mk(0.0f, 0.0f);
-    if (type == MANIFOLD_CIRCLES) {
-      normal = mk(1.0f, 0.0f);
-      V2 pointA = xmul(xfA, lp);
-      V2 pointB = xmul(xfB, mp0);
-      if (distsq(pointA, pointB) > KB_EPS * KB_EPS) {
-        normal = pointB - pointA;
-        normalize(normal);
-      }
-      V2 a = pointA + radiusA * normal;
-      V2 b = pointB - radiusB * normal;
-      pt = 0.5f * (a + b);
-    } else {
-      normal = rmul(xfA.q, ln);
-      V2 planePoint = xmul(xfA, lp);
-      V2 clipPoint = xmul(xfB, mp0);
-      V2 a = clipPoint + (radiusA - dot(clipPoint - planePoint, normal)) * normal;
-      V2 b = clipPoint - radiusB * normal;
-      pt = 0.5f * (a + b);
-    }
-    const V2 rA = pt - cA;
-    const V2 rB = pt - cB;
-    const float rnA = cross(rA, normal);
-    const float rnB = cross(rB, normal);
-    const float kNormal = mA + mB + iA * rnA * rnA + iB * rnB * rnB;
-    const float nMass = kNormal > 0.0f ? 1.0f / kNormal : 0.0f;
-    rec4(3 * e) = make_float4(normal.x, normal.y, nMass, r1.x);
-    rec4(3 * e + 1) = make_float4(rA.x, rA.y, rB.x, rB.y);
+    Rot qA, qB;
+    qA.s = qa.x; qA.c = qa.y;
+    qB.s = qb.x; qB.c = qb.y;
+    float4 v0, v1;
+    kb_init_simple(mk(cA4.x, cA4.y), mk(cB4.x, cB4.y), qA, qB, mk(0.0f, 0.0f), mk(0.0f, 0.0f), r0, mk(0.0f, 0.0f), type, radiusA,
+                   radiusB, mA, iA, mB, iB, r1.x, v0, v1);
+    rec4(3 * e) = v0;
+    rec4(3 * e + 1) = v1;
     rec4(3 * e + 2) = make_float4(mA, iA, mB, iB);
   }
   // The *Core forms take the schedule entry and the records as values: the relay (below) fetches them from L2 ahead of
   // the warp's turn, so that only the shared-memory traffic on the bodies and the arithmetic are on the critical path.
   // (sA / sB: the two bodies' vel4 or pos4 rows; wA / wB: where the results go -- the same rows, or the dummy row when body A
   //  is the table or when the lane only keeps step with its warp)
-  __device__ __forceinline__ void warmStartCore(SF4 sA, SF4 sB, SF4 wA, SF4 wB, const float4& r0, const float4& r1, const float4& r2) const {
-    const float2 kA = make_float2(r2.x, r2.y), kB = make_float2(r2.z, r2.w);
-    float4 vA = sA, vB = sB;
-    const V2 normal = mk(r0.x, r0.y);
-    const V2 tangent = cross(normal, 1.0f);
-    const V2 rA = mk(r1.x, r1.y), rB = mk(r1.z, r1.w);
-    const V2 P = r0.w * normal + 0.0f * tangent;
-    vA.z -= kA.y * cross(rA, P);
-    vA.x = vA.x - kA.x * P.x;
-    vA.y = vA.y - kA.x * P.y;
-    vB.z += kB.y * cross(rB, P);
-    vB.x = vB.x + kB.x * P.x;
-    vB.y = vB.y + kB.x * P.y;
-    wA = vA;
-    wB = vB;
-  }
-  __device__ __forceinline__ void warmStartSimple(int e) const {
-    const uint32_t bb = ent0(e);
-    const SF4 sA = vel4((int)(bb & 0xFFFFu)), sB = vel4((int)(bb >> 16));
-    warmStartCore(sA, sB, (int)(bb & 0xFFFFu) != S ? sA : dummy4(), sB, rec4(3 * e), rec4(3 * e + 1), rec4(3 * e + 2));
-  }
   // returns the accumulated normal impulse (the caller keeps it in rec4(3e).w)
   __device__ __forceinline__ float solveVelocityCore(SF4 sA, SF4 sB, SF4 wA, SF4 wB, const float4& r0, const float4& r1, const float4& r2) const {
-    const float2 kA = make_float2(r2.x, r2.y), kB = make_float2(r2.z, r2.w);
     float4 a4 = sA, b4 = sB;
-    const V2 normal = mk(r0.x, r0.y);
-    const V2 rA0 = mk(r1.x, r1.y), rB0 = mk(r1.z, r1.w);
-    const V2 Av = mk(a4.x, a4.y), Bv = mk(b4.x, b4.y);
-    V2 dv = Bv + cross(b4.z, rB0) - Av - cross(a4.z, rA0);
-    float vn = dot(dv, normal);
-    float ni = r0.w;
-    float lambda = -r0.z * (vn - 0.0f);
-    float newImpulse = b2max(ni + lambda, 0.0f);
-    lambda = newImpulse - ni;
-    V2 P = lambda * normal;
-    const V2 Av2 = Av - kA.x * P;
-    a4.z -= kA.y * cross(rA0, P);
-    const V2 Bv2 = Bv + kB.x * P;
-    b4.z += kB.y * cross(rB0, P);
-    a4.x = Av2.x; a4.y = Av2.y;
-    b4.x = Bv2.x; b4.y = Bv2.y;
+    const float newImpulse = kb_solve_velocity_simple(a4, b4, r0, r1, r2.x, r2.y, r2.z, r2.w);
     wA = a4;
     wB = b4;
     return newImpulse;
@@ -550,52 +485,18 @@ struct Swarm {
       }
       return okf;
     }
-    V2 cA = mk(pA4.x, pA4.y), cB = mk(pB4.x, pB4.y);
-    V2 normal, point;
-    float separation;
-    {
-      const V2 ln = mk(r0.x, r0.y), lp = mk(r0.z, r0.w);
-      const int type = (int)f2u(r1.z);
-      // no body of this tier has a local centre or a local manifold point on B: rotations multiply exact zeros
-      Xf xfA, xfB;
-      xfA.q.s = 0.0f; xfA.q.c = 1.0f;
-      xfB.q.s = 0.0f; xfB.q.c = 1.0f;
-      xfA.p = cA - rmul(xfA.q, mk(0.0f, 0.0f));
-      xfB.p = cB - rmul(xfB.q, mk(0.0f, 0.0f));
-      const V2 mpj = mk(0.0f, 0.0f);
-      if (type == MANIFOLD_CIRCLES) {
-        V2 pointA = xmul(xfA, lp);
-        V2 pointB = xmul(xfB, mpj);
-        normal = pointB - pointA;
-        normalize(normal);
-        point = 0.5f * (pointA + pointB);
-        separation = dot(pointB - pointA, normal) - r1.x - r1.y;
-      } else {
-        normal = rmul(xfA.q, ln);
-        V2 planePoint = xmul(xfA, lp);
-        V2 clipPoint = xmul(xfB, mpj);
-        separation = dot(clipPoint - planePoint, normal) - r1.x - r1.y;
-        point = clipPoint;
-      }
+    // no body of this tier has a local centre or a local manifold point on B: rotations multiply exact zeros
+    Rot qA, qB;
+    qA.s = 0.0f; qA.c = 1.0f;
+    qB.s = 0.0f; qB.c = 1.0f;
+    float4 a1, b1;
+    bool moved;
+    const bool ok = kb_position_simple(pA4, pB4, qA, qB, mk(0.0f, 0.0f), mk(0.0f, 0.0f), r0, (int)f2u(r1.z), r1.x, r1.y, mA, iA, mB, iB,
+                                       baumgarte, limit, skipZero, a1, b1, moved);
+    if (moved) {
+      wA = a1;
+      wB = b1;
     }
-    const bool ok = separation >= limit;
-    const float C = b2clamp(baumgarte * (separation + KB_LINEAR_SLOP), -KB_MAX_LINEAR_CORRECTION, 0.0f);
-    if (skipZero && C == 0.0f) return ok;   // the impulse is -0 / K and moves nothing
-    const V2 rA = point - cA;
-    const V2 rB = point - cB;
-    const float rnA = cross(rA, normal);
-    const float rnB = cross(rB, normal);
-    const float K = mA + mB + iA * rnA * rnA + iB * rnB * rnB;
-    const float impulse = K > 0.0f ? -C / K : 0.0f;
-    const V2 P = impulse * normal;
-    cA = cA - mA * P;
-    pA4.z -= iA * cross(rA, P);
-    cB = cB + mB * P;
-    pB4.z += iB * cross(rB, P);
-    pA4.x = cA.x; pA4.y = cA.y;
-    wA = pA4;
-    pB4.x = cB.x; pB4.y = cB.y;
-    wB = pB4;
     return ok;
   }
 
@@ -879,8 +780,7 @@ struct Swarm {
       sweepp()[b] = make_float4(p.x, p.y, p.z, 0.0f);
       float4 v = vel4(b);
       const float ld = __ldg(&bc[b].linearDamping), ad = __ldg(&bc[b].angularDamping);
-      const float dl = L.dampingMode == 0 ? 1.0f / (1.0f + h * ld) : b2clamp(1.0f - h * ld, 0.0f, 1.0f);
-      const float da = L.dampingMode == 0 ? 1.0f / (1.0f + h * ad) : b2clamp(1.0f - h * ad, 0.0f, 1.0f);
+      const float dl = kb_damping(L.dampingMode, h, ld), da = kb_damping(L.dampingMode, h, ad);
       v.x *= dl;
       v.y *= dl;
       v.z *= da;
@@ -941,7 +841,10 @@ struct Swarm {
             if (pass == 0) {   // (one uniform branch per turn, not per step)
 #pragma unroll
               for (int gg = 0; gg < RG; ++gg) {
-                warmStartCore(SF4{aS[gg]}, SF4{bS[gg]}, SF4{cS[gg]}, SF4{bS[gg]}, r0, r1, r2);
+                float4 vA = SF4{aS[gg]}, vB = SF4{bS[gg]};
+                kb_warm_start_simple(vA, vB, r0, r1, r2.x, r2.y, r2.z, r2.w);
+                SF4{cS[gg]} = vA;
+                SF4{bS[gg]} = vB;
                 __syncwarp();
               }
             } else {
@@ -968,20 +871,7 @@ struct Swarm {
       if ((uint32_t)isl(b) == SW_NOISLAND) continue;
       float4 p = pos4(b);
       float4 v = vel4(b);
-      V2 translation = h * mk(v.x, v.y);
-      if (dot(translation, translation) > KB_MAX_TRANSLATION_SQ) {
-        float ratio = KB_MAX_TRANSLATION / length(translation);
-        v.x *= ratio;
-        v.y *= ratio;
-      }
-      float rotation = h * v.z;
-      if (rotation * rotation > KB_MAX_ROTATION_SQ) {
-        float ratio = KB_MAX_ROTATION / b2abs(rotation);
-        v.z *= ratio;
-      }
-      p.x += h * v.x;
-      p.y += h * v.y;
-      p.z += h * v.z;
+      kb_integrate_position(p, v, h);
       pos4(b) = p;
       vel4(b) = v;
     }
@@ -1081,12 +971,7 @@ struct Swarm {
       const Rot q = rot_set(p.z);
       q2(b) = make_float2(q.s, q.c);
       if (L.enableSleep) {
-        const float4 v = vel4(b);
-        const float linTolSqr = KB_LIN_SLEEP_TOL * KB_LIN_SLEEP_TOL;
-        const float angTolSqr = KB_ANG_SLEEP_TOL * KB_ANG_SLEEP_TOL;
-        float st;
-        if (v.z * v.z > angTolSqr || dot(mk(v.x, v.y), mk(v.x, v.y)) > linTolSqr) st = 0.0f;
-        else st = p.w + h;
+        const float st = kb_sleep_time(vel4(b), p.w, h);
         pos4(b).set(3, st);
         if (!(st >= KB_TIME_TO_SLEEP)) {
           if (island == SW_LONELY) isl(b) = SW_LONELY - 1u;   // lonely and not ready: marked "stay awake" (0xFFFD)
@@ -1507,12 +1392,7 @@ struct Swarm {
         if (!awake(bd)) continue;
         float4 sw = sweepp()[bd];
         if (sw.w < tableAlpha0) {
-          const float4 p = pos4(bd);
-          const float beta = (tableAlpha0 - sw.w) / (1.0f - sw.w);
-          sw.x += beta * (p.x - sw.x);
-          sw.y += beta * (p.y - sw.y);
-          sw.z += beta * (p.z - sw.z);
-          sw.w = tableAlpha0;
+          kb_sweep_advance(sw, pos4(bd), tableAlpha0);
           sweepp()[bd] = sw;   // several contacts of one body write identical values
         }
       }
@@ -1587,11 +1467,7 @@ struct Swarm {
         {
           float4 sw = backupSweep;
           float4 p = backupPos;
-          const float beta = (minAlpha - sw.w) / (1.0f - sw.w);
-          sw.x += beta * (p.x - sw.x);
-          sw.y += beta * (p.y - sw.y);
-          sw.z += beta * (p.z - sw.z);
-          sw.w = minAlpha;
+          kb_sweep_advance(sw, p, minAlpha);
           p.x = sw.x; p.y = sw.y; p.z = sw.z;
           sweepp()[bd] = sw;
           pos4(bd) = p;
@@ -1668,20 +1544,7 @@ struct Swarm {
             const float h = (1.0f - minAlpha) * L.dt;
             float4 p = pos4(bd);
             float4 v = vel4(bd);
-            V2 translation = h * mk(v.x, v.y);
-            if (dot(translation, translation) > KB_MAX_TRANSLATION_SQ) {
-              float ratio = KB_MAX_TRANSLATION / length(translation);
-              v.x *= ratio;
-              v.y *= ratio;
-            }
-            float rotation = h * v.z;
-            if (rotation * rotation > KB_MAX_ROTATION_SQ) {
-              float ratio = KB_MAX_ROTATION / b2abs(rotation);
-              v.z *= ratio;
-            }
-            p.x += h * v.x;
-            p.y += h * v.y;
-            p.z += h * v.z;
+            kb_integrate_position(p, v, h);
             pos4(bd) = p;
             vel4(bd) = v;
             const Rot q = rot_set(p.z);

@@ -522,13 +522,7 @@ __device__ __forceinline__ void Sim<LPE, UNI, LT>::solveTOI() {
       if (need) {
         float4 sw = sweep4(bd);
         if (sw.w < tableAlpha0) {
-          // b2Sweep::Advance(alpha0)
-          const float4 p = pos4(bd);
-          float beta = (tableAlpha0 - sw.w) / (1.0f - sw.w);
-          sw.x += beta * (p.x - sw.x);
-          sw.y += beta * (p.y - sw.y);
-          sw.z += beta * (p.z - sw.z);
-          sw.w = tableAlpha0;
+          kb_sweep_advance(sw, pos4(bd), tableAlpha0);
           sweep4(bd) = sw;
         }
       }
@@ -597,11 +591,7 @@ __device__ __forceinline__ void Sim<LPE, UNI, LT>::solveTOI() {
       float4 sw = sweep4(bd);
       float4 p = pos4(bd);
       const float4 k = bc4(bd);
-      float beta = (minAlpha - sw.w) / (1.0f - sw.w);
-      sw.x += beta * (p.x - sw.x);
-      sw.y += beta * (p.y - sw.y);
-      sw.z += beta * (p.z - sw.z);
-      sw.w = minAlpha;
+      kb_sweep_advance(sw, p, minAlpha);
       p.x = sw.x; p.y = sw.y; p.z = sw.z;
       sweep4(bd) = sw;
       pos4(bd) = p;
@@ -690,20 +680,7 @@ __device__ __forceinline__ void Sim<LPE, UNI, LT>::solveTOI() {
         float4 p = pos4(bd);
         float4 v = vel4(bd);
         const float4 kk = bc4(bd);
-        V2 translation = h * mk(v.x, v.y);
-        if (dot(translation, translation) > KB_MAX_TRANSLATION_SQ) {
-          float ratio = KB_MAX_TRANSLATION / length(translation);
-          v.x *= ratio;
-          v.y *= ratio;
-        }
-        float rotation = h * v.z;
-        if (rotation * rotation > KB_MAX_ROTATION_SQ) {
-          float ratio = KB_MAX_ROTATION / b2abs(rotation);
-          v.z *= ratio;
-        }
-        p.x += h * v.x;
-        p.y += h * v.y;
-        p.z += h * v.z;
+        kb_integrate_position(p, v, h);
         pos4(bd) = p;
         vel4(bd) = v;
         Rot q = rot_set(p.z);
