@@ -165,6 +165,22 @@ class KbSampleSpec(C.Structure):
     ]
 
 
+# actuation model (extension, include/kb_b200.h kb_set_actuation)
+class KbActuationDef(C.Structure):
+    _fields_ = [
+        ("seed", C.c_uint64),
+        ("env_id_base", C.c_int64),
+        ("gain_v_lo", C.c_double),
+        ("gain_v_hi", C.c_double),
+        ("gain_w_lo", C.c_double),
+        ("gain_w_hi", C.c_double),
+        ("drift_w", C.c_double),
+        ("noise_v", C.c_double),
+        ("noise_w", C.c_double),
+        ("p_dead", C.c_double),
+    ]
+
+
 # test-only geometry probe (include/kb_b200.h kb_probe_geometry)
 KB_PROBE_SHAPE, KB_PROBE_COLLIDE, KB_PROBE_DISTANCE, KB_PROBE_TOI = 0, 1, 2, 3
 KB_PROBE_OUT_WORDS = 40
@@ -214,7 +230,7 @@ class KbLaunchConfig(C.Structure):
     _fields_ = [("lanes_per_env", C.c_int32), ("block_threads", C.c_int32), ("grid_blocks", C.c_int32),
                 ("smem_bytes_per_block", C.c_int32), ("state_words_per_env", C.c_int32),
                 ("smem_words_per_env", C.c_int32), ("specialised", C.c_int32), ("jit_ms", C.c_float),
-                ("jit_reason", C.c_char * 256)]
+                ("jit_reason", C.c_char * 256), ("actuation", C.c_int32)]
 
 
 PRODUCT_ONLY = {
@@ -234,6 +250,9 @@ PRODUCT_ONLY = {
     "selftest_exact_math": (C.c_int, [C.c_int32, C.c_int32, C.POINTER(C.c_uint64)]),
     "local_observation_dim": (C.c_int, [_VP, C.POINTER(KbLocalObsDef)]),
     "local_observation": (C.c_int, [_VP, C.POINTER(KbLocalObsDef), _VP, _VP, _VP]),
+    # actuation model (also exported, kbo_-prefixed, by the test oracle tests/kbo_actuation.cpp)
+    "set_actuation": (C.c_int, [_VP, C.POINTER(KbActuationDef)]),
+    "get_actuation": (C.c_int, [_VP, _VP, _VP, C.POINTER(C.c_uint64)]),
 }
 
 

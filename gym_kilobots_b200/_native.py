@@ -354,6 +354,24 @@ class NativeBatch:
         self._keep_local = m
         return out
 
+    # ---- actuation model (extension: per-kilobot motor gains, drift, noise and failures; csrc/kb_env.cuh)
+    def set_actuation(self, spec):
+        """spec: scene.ActuationSpec, or None to detach.  Draws episode 0 of every env; every later reset draws the reset
+        envs' next episode."""
+        if spec is None:
+            _check(_fn["set_actuation"](self.h, None), "kb_set_actuation")
+            return
+        d = spec.to_def()
+        _check(_fn["set_actuation"](self.h, C.byref(d)), "kb_set_actuation")
+
+    def actuation(self):
+        """(draws [E,N,4] float32 = (g_v, g_w, d_w, alive), actuation episodes [E] uint32, step count) on the host."""
+        draws = np.zeros((self.E, self.N, 4), np.float32)
+        ep = np.zeros(self.E, np.uint32)
+        step = C.c_uint64()
+        _check(_fn["get_actuation"](self.h, _hptr(draws), _hptr(ep), C.byref(step)), "kb_get_actuation")
+        return draws, ep, int(step.value)
+
     def render(self, env_ids=(0,), width=1200, height=900):
         """uint8 CUDA tensor [len(env_ids), height, width, 3]: the picture KilobotsEnv.render would draw
         (kilobots_env.py:221-275; default size = screen_size :22), rasterised on the device."""
@@ -373,8 +391,9 @@ class NativeBatch:
     def launch_config(self):
         cfg = abi.KbLaunchConfig()
         _check(_fn["get_launch_config"](self.h, C.byref(cfg)), "kb_get_launch_config")
-        out = {k: int(getattr(cfg, k)) for k, _ in cfg._fields_ if k not in ("specialised", "jit_ms", "jit_reason")}
+        out = {k: int(getattr(cfg, k)) for k, _ in cfg._fields_ if k not in ("specialised", "jit_ms", "jit_reason", "actuation")}
         out["specialised"] = bool(cfg.specialised)
+        out["actuation"] = bool(cfg.actuation)
         out["jit_ms"] = round(float(cfg.jit_ms), 1)
         out["jit_reason"] = cfg.jit_reason.decode()
         out["kernel"] = ("kb_swarm_step_kernel (one CTA per env)" if out["lanes_per_env"] > 32

@@ -33,6 +33,39 @@ template <int LPE>
 __global__ void __launch_bounds__(KB_STEP_BOUNDS(LPE)) kb_step_kernel(const __grid_constant__ KernelArgs a) {
   stepKernelBody<LPE>(a, a.L);
 }
+// the same with the actuation model (kb_set_actuation)
+template <int LPE>
+__global__ void __launch_bounds__(KB_STEP_BOUNDS(LPE)) kb_step_kernel_act(const __grid_constant__ KernelArgs a) {
+  stepKernelBody<LPE, Layout, true>(a, a.L);
+}
+
+// The per-episode actuation draws of the (masked) envs, one block per env (include/kb_b200.h kb_set_actuation):
+// advance = 1 starts the env's next episode, 0 draws its current one.  Every padded kilobot slot is drawn, present or
+// not, from two Philox4x32-10 blocks (draw indices 2k, 2k + 1 of stream KS_ACTUATION, keyed like the scene sampler's
+// draws by seed, global env id and the env's actuation episode).
+__global__ void __launch_bounds__(32) kb_actuation_draw_kernel(const KbActuationDef d, const uint8_t* __restrict__ mask,
+                                                               uint32_t* episode, float4* draws, int N, int advance) {
+  const int env = blockIdx.x;
+  if (mask && !mask[env]) return;
+  const uint32_t ep = episode[env] + (uint32_t)advance;
+  __syncthreads();
+  if (threadIdx.x == 0) episode[env] = ep;
+  const unsigned long long g = (unsigned long long)(d.env_id_base + env);
+  EnvRng r;
+  r.k0 = (uint32_t)(d.seed & 0xFFFFFFFFull);
+  r.k1 = (uint32_t)(d.seed >> 32);
+  r.e0 = (uint32_t)(g & 0xFFFFFFFFull);
+  r.e1 = (uint32_t)(g >> 32);
+  r.ep = ep;
+  for (int k = threadIdx.x; k < N; k += blockDim.x) {
+    double u0, u1, u2, u3;
+    r.uniform2(KS_ACTUATION, 2u * (uint32_t)k, &u0, &u1);
+    r.uniform2(KS_ACTUATION, 2u * (uint32_t)k + 1u, &u2, &u3);
+    draws[(size_t)env * N + k] = make_float4((float)(d.gain_v_lo + (d.gain_v_hi - d.gain_v_lo) * u0),
+                                             (float)(d.gain_w_lo + (d.gain_w_hi - d.gain_w_lo) * u1),
+                                             (float)(d.drift_w * (2.0 * u2 - 1.0)), u3 < d.p_dead ? 0.0f : 1.0f);
+  }
+}
 
 template <int LPE>
 __global__ void __launch_bounds__(KB_BLOCK_OF(LPE)) kb_reset_kernel(const __grid_constant__ KernelArgs a) {
@@ -292,6 +325,16 @@ struct Handle {
   cudaKernel_t stepJit = nullptr;
   float jitMs = 0.0f;          // its compile time in kb_create (0: from a cache)
   std::string jitReason;       // why the generic kernel runs instead
+  // actuation model (kb_set_actuation): while actOn, kb_step launches stepAct, the actuation-on variant of its kernel
+  bool actOn = false;
+  KbActuationDef act = {};
+  uint64_t actStep = 0;        // kb_step / kb_step_host calls since kb_set_actuation
+  DevBuf<float4> dActDraws;    // [E][N] (g_v, g_w, d_w, alive)
+  DevBuf<uint32_t> dActEpisode;
+  const void* stepAct = nullptr;
+  bool actSpecialised = false;
+  float actJitMs = 0.0f;
+  std::string actReason;       // why the generic actuation-on kernel runs
 #ifdef KB_PROFILE
   DevBuf<unsigned long long> dProf;
 #endif
@@ -326,15 +369,18 @@ static void withTierWidth(const Handle* h, F&& f) {
 // the generic step, reset and set-pose kernels of the batch's tier and width
 struct TierKernels {
   const void *step = nullptr, *reset = nullptr, *setpose = nullptr;
+  const void* stepAct = nullptr;   // the step kernel with the actuation model
 };
 static TierKernels tierKernels(const Handle* h) {
   TierKernels k;
   withTierWidth(h, [&](auto swarm, auto width) {
     constexpr int W = decltype(width)::value;
     if constexpr (decltype(swarm)::value)
-      k = {(const void*)kb_swarm_step_kernel<W>, (const void*)kb_swarm_reset_kernel<W>, (const void*)kb_swarm_setpose_kernel<W>};
+      k = {(const void*)kb_swarm_step_kernel<W>, (const void*)kb_swarm_reset_kernel<W>,
+           (const void*)kb_swarm_setpose_kernel<W>, (const void*)kb_swarm_step_kernel_act<W>};
     else
-      k = {(const void*)kb_step_kernel<W>, (const void*)kb_reset_kernel<W>, (const void*)kb_setpose_kernel<W>};
+      k = {(const void*)kb_step_kernel<W>, (const void*)kb_reset_kernel<W>, (const void*)kb_setpose_kernel<W>,
+           (const void*)kb_step_kernel_act<W>};
   });
   return k;
 }
@@ -685,6 +731,16 @@ static void fillArgs(const Handle* h, KernelArgs* a) {
 #ifdef KB_PROFILE
   a->prof = h->dProf.get();
 #endif
+}
+
+// the per-episode actuation draws of the envs in `mask` (device u8[E] or null = all) on `stream`, after the reset kernel
+// (advance = 1) or for the episode the envs are in (0); nothing without an actuation model
+static int drawActuation(const Handle* h, const uint8_t* mask, int advance, cudaStream_t stream) {
+  if (!h->actOn) return KB_OK;
+  kb_actuation_draw_kernel<<<h->numEnvs, 32, 0, stream>>>(h->act, mask, h->dActEpisode.get(), h->dActDraws.get(), h->L.N,
+                                                          advance);
+  CUDA_TRY(cudaGetLastError());
+  return KB_OK;
 }
 
 // The batch's layout (h->L, h->W), tier, lane width and shared-memory size from its scenes.  Needs no device: `prop`
@@ -1127,7 +1183,7 @@ int kb_create(const KbSceneDesc* scenes, int32_t num_scenes, const int32_t* env_
       h->jitReason = "KB_JIT=0";
     } else {
       double ms = 0.0;
-      h->stepJit = jitStepKernel(L, &ms, &h->jitReason);
+      h->stepJit = jitStepKernel(L, false, &ms, &h->jitReason);
       h->jitMs = (float)ms;
       if (h->stepJit) {
         const cudaError_t e = raiseSmemLimit((const void*)h->stepJit, h->smemBytes);
@@ -1200,7 +1256,8 @@ int kb_reset(KbHandle* hh, const uint8_t* mask, const double* body_pose, const d
   a.lightInit = light_state;
   a.kbVel = kb_velocity;
   a.status = h->dStatus;
-  return launch(h, tierKernels(h).reset, a, h->numEnvs, (cudaStream_t)stream);
+  if (const int rc = launch(h, tierKernels(h).reset, a, h->numEnvs, (cudaStream_t)stream)) return rc;
+  return drawActuation(h, mask, 1, (cudaStream_t)stream);
 }
 
 // ---- on-device scene sampling (include/kb_b200.h "Reset with on-device scene sampling") ------------------------
@@ -1377,7 +1434,8 @@ int kb_reset_sampled(KbHandle* hh, const uint8_t* mask, void* stream) {
   a.sceneConfig = h->dSceneConfig.get();
   a.configCdf = h->weighted ? h->dConfigCdf.get() : nullptr;
   a.numConfigs = h->numConfigs;
-  return launch(h, tierKernels(h).reset, a, h->numEnvs, (cudaStream_t)stream);
+  if (const int rc = launch(h, tierKernels(h).reset, a, h->numEnvs, (cudaStream_t)stream)) return rc;
+  return drawActuation(h, mask, 1, (cudaStream_t)stream);
 }
 
 int kb_get_sampled(KbHandle* hh, double* body_pose, double* light_state, int32_t* env_scene, uint32_t* episodes) {
@@ -1421,6 +1479,18 @@ static int stepRange(Handle* h, const double* action, int32_t action_mode, float
   a.status = status;
   a.obsFlat = h->obsFlat;
   a.envOffset = envBegin;
+  if (h->actOn) {
+    a.actDraws = h->dActDraws.get();
+    a.actNoiseV = h->act.noise_v;
+    a.actNoiseW = h->act.noise_w;
+    a.actEnvIdBase = h->act.env_id_base;
+    a.actSeedLo = (uint32_t)(h->act.seed & 0xFFFFFFFFull);
+    a.actSeedHi = (uint32_t)(h->act.seed >> 32);
+    a.actStep = (uint32_t)h->actStep;
+    a.actNoise = h->act.noise_v > 0.0 || h->act.noise_w > 0.0;
+    a.actDrift = h->act.drift_w > 0.0;
+    return launch(h, h->stepAct, a, envCount, stream);
+  }
   return launch(h, h->stepJit ? (const void*)h->stepJit : tierKernels(h).step, a, envCount, stream);
 }
 
@@ -1433,8 +1503,10 @@ int kb_step(KbHandle* hh, const double* action, int32_t action_mode, float* obs_
   Handle* h = reinterpret_cast<Handle*>(hh);
   if (const int rc = enter(h, "kb_step", false)) return rc;
   if (badActionMode(action_mode)) return fail(KB_ERR_INVALID, "kb_step: bad action_mode");
-  return stepRange(h, action, action_mode, obs_kilobots, obs_objects, obs_light, reward, done, status, 0, h->numEnvs,
-                   (cudaStream_t)stream);
+  const int rc = stepRange(h, action, action_mode, obs_kilobots, obs_objects, obs_light, reward, done, status, 0,
+                           h->numEnvs, (cudaStream_t)stream);
+  if (rc == KB_OK) ++h->actStep;
+  return rc;
 }
 
 int kb_step_host(KbHandle* hh, const double* action, int32_t action_mode, float* obs_kilobots, float* obs_objects,
@@ -1495,6 +1567,7 @@ int kb_step_host(KbHandle* hh, const double* action, int32_t action_mode, float*
       CUDA_TRY(cudaStreamWaitEvent(st, h->evJoin[i].get(), 0));
     }
   }
+  ++h->actStep;   // every chunk stepped with the same count
   CUDA_TRY(cudaStreamSynchronize(st));
   return KB_OK;
 }
@@ -1697,9 +1770,84 @@ int kb_get_launch_config(const KbHandle* hh, KbLaunchConfig* cfg) {
   cfg->smem_bytes_per_block = (int32_t)h->smemBytes;
   cfg->state_words_per_env = h->L.stateWords;
   cfg->smem_words_per_env = h->L.smemWords;
-  cfg->specialised = h->stepJit != nullptr;
-  cfg->jit_ms = h->jitMs;
-  std::snprintf(cfg->jit_reason, sizeof(cfg->jit_reason), "%s", h->jitReason.c_str());
+  cfg->specialised = h->actOn ? h->actSpecialised : h->stepJit != nullptr;
+  cfg->actuation = h->actOn ? 1 : 0;
+  cfg->jit_ms = h->actOn ? h->actJitMs : h->jitMs;
+  std::snprintf(cfg->jit_reason, sizeof(cfg->jit_reason), "%s", (h->actOn ? h->actReason : h->jitReason).c_str());
+  return KB_OK;
+}
+
+// ---- actuation model (include/kb_b200.h kb_set_actuation) ------------------------------------------------------
+int kb_set_actuation(KbHandle* hh, const KbActuationDef* def) {
+  Handle* h = reinterpret_cast<Handle*>(hh);
+  if (const int rc = enter(h, "kb_set_actuation", true)) return rc;   // no launch in flight reads the old draws
+  if (!def) {
+    h->actOn = false;
+    return KB_OK;
+  }
+  const KbActuationDef& d = *def;
+  const struct {
+    const char* name;
+    double v;
+  } fields[] = {{"gain_v_lo", d.gain_v_lo}, {"gain_v_hi", d.gain_v_hi}, {"gain_w_lo", d.gain_w_lo}, {"gain_w_hi", d.gain_w_hi},
+                {"drift_w", d.drift_w},     {"noise_v", d.noise_v},     {"noise_w", d.noise_w},     {"p_dead", d.p_dead}};
+  for (const auto& f : fields) {
+    if (!std::isfinite(f.v)) return fail(KB_ERR_INVALID, std::string("kb_set_actuation: ") + f.name + " is not finite");
+    if (f.v < 0.0) return fail(KB_ERR_INVALID, std::string("kb_set_actuation: ") + f.name + " is negative");
+  }
+  if (d.gain_v_lo > d.gain_v_hi) return fail(KB_ERR_INVALID, "kb_set_actuation: gain_v_lo > gain_v_hi");
+  if (d.gain_w_lo > d.gain_w_hi) return fail(KB_ERR_INVALID, "kb_set_actuation: gain_w_lo > gain_w_hi");
+  if (d.p_dead > 1.0) return fail(KB_ERR_INVALID, "kb_set_actuation: p_dead is outside [0, 1]");
+  // the actuation-on step kernel: the specialised one when the batch runs a specialised kernel, else the generic one
+  const TierKernels tk = tierKernels(h);
+  const void* kernel = tk.stepAct;
+  bool specialised = false;
+  double ms = 0.0;
+  std::string reason = h->jitReason;
+  if (h->stepJit) {
+    reason.clear();
+    cudaKernel_t jit = jitStepKernel(h->L, true, &ms, &reason);
+    if (jit) {
+      const cudaError_t e = raiseSmemLimit((const void*)jit, h->smemBytes);
+      if (e == cudaSuccess) {
+        kernel = (const void*)jit;
+        specialised = true;
+      } else {
+        cudaGetLastError();
+        reason = std::string("load error: ") + cudaGetErrorString(e);
+      }
+    }
+    const char* ev = getenv("KB_JIT");
+    if (!specialised && ev && atoi(ev) == 1)
+      return fail(KB_ERR_CUDA, "kb_set_actuation: KB_JIT=1 but the specialised step kernel is not available: " + reason);
+  }
+  if (!specialised) CUDA_TRY(raiseSmemLimit(kernel, h->smemBytes));
+  if (!h->dActDraws) {
+    CUDA_TRY(devAlloc(h->dActDraws, (size_t)h->numEnvs * std::max(h->L.N, 1)));
+    CUDA_TRY(devAlloc(h->dActEpisode, (size_t)h->numEnvs));
+  }
+  CUDA_TRY(cudaMemset(h->dActEpisode.get(), 0, sizeof(uint32_t) * (size_t)h->numEnvs));
+  h->act = d;
+  h->actOn = true;
+  h->actStep = 0;
+  h->stepAct = kernel;
+  h->actSpecialised = specialised;
+  h->actJitMs = (float)ms;
+  h->actReason = specialised ? std::string() : reason;
+  if (const int rc = drawActuation(h, nullptr, 0, nullptr)) return rc;   // episode 0 of every env
+  CUDA_TRY(cudaDeviceSynchronize());
+  return KB_OK;
+}
+
+int kb_get_actuation(KbHandle* hh, float* draws, uint32_t* episodes, uint64_t* step) {
+  Handle* h = reinterpret_cast<Handle*>(hh);
+  if (const int rc = enter(h, "kb_get_actuation", true)) return rc;
+  if (!h->actOn) return fail(KB_ERR_INVALID, "kb_get_actuation: no actuation model (kb_set_actuation)");
+  const size_t E = (size_t)h->numEnvs;
+  if (draws && h->L.N > 0)
+    CUDA_TRY(cudaMemcpy(draws, h->dActDraws.get(), sizeof(float4) * E * h->L.N, cudaMemcpyDeviceToHost));
+  if (episodes) CUDA_TRY(cudaMemcpy(episodes, h->dActEpisode.get(), sizeof(uint32_t) * E, cudaMemcpyDeviceToHost));
+  if (step) *step = h->actStep;
   return KB_OK;
 }
 

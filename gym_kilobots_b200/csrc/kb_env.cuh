@@ -152,10 +152,60 @@ __device__ __forceinline__ void setKilobotActions(T& s, const double* action, in
   }
 }
 
+// ------------------------------------------------------------------------------------------------- actuation model
+// (include/kb_b200.h kb_set_actuation; gym_kilobots_b200/actuation.py evaluates the same draws in numpy).  Kilobot k of an
+// env has per-episode draws (g_v, g_w, d_w, alive) in a.actDraws and, with noise, per-sub-step factors f_v, f_w from one
+// Philox4x32-10 block with counter (k | sub-step << 16, step count, global env id low word, KS_ACTUATION_NOISE | high
+// word << 8).  A controller's velocity v and turn rate w become (v * g_v) * f_v and (w * g_w) * f_w (+ d_w with drift),
+// float32; a dead kilobot's controller runs but sets no velocity.
+struct KilobotActuation {
+  float gv, gw, dw, fv, fw;
+  bool alive;
+};
+
+__device__ __forceinline__ KilobotActuation kilobotActuation(const KernelArgs& a, int envIn, int k, int substep) {
+  const float4 d = a.actDraws[(size_t)envIn * a.L.N + k];
+  KilobotActuation ka;
+  ka.gv = d.x;
+  ka.gw = d.y;
+  ka.dw = d.z;
+  ka.alive = d.w != 0.0f;
+  ka.fv = 1.0f;
+  ka.fw = 1.0f;
+  if (a.actNoise && ka.alive) {
+    const unsigned long long g = (unsigned long long)(a.actEnvIdBase + envIn);
+    const Philox4 r = philox4x32((uint32_t)k | ((uint32_t)substep << 16), a.actStep, (uint32_t)(g & 0xFFFFFFFFull),
+                                 KS_ACTUATION_NOISE | ((uint32_t)(g >> 32) << 8), a.actSeedLo, a.actSeedHi);
+    ka.fv = (float)(1.0 + a.actNoiseV * (2.0 * u53(r.x, r.y) - 1.0));
+    ka.fw = (float)(1.0 + a.actNoiseW * (2.0 * u53(r.z, r.w) - 1.0));
+  }
+  return ka;
+}
+
+// a controller's SetLinearVelocity / SetAngularVelocity through the actuation model (ACT) or directly
+template <bool ACT, class T>
+__device__ __forceinline__ void driveLinear(T& s, int b, V2 v, const KilobotActuation& ka) {
+  if constexpr (ACT) {
+    if (!ka.alive) return;
+    v = mk((v.x * ka.gv) * ka.fv, (v.y * ka.gv) * ka.fv);
+  }
+  setLinearVelocity(s, b, v);
+}
+template <bool ACT, class T>
+__device__ __forceinline__ void driveAngular(T& s, int b, float w, const KilobotActuation& ka, int drift) {
+  if constexpr (ACT) {
+    if (!ka.alive) return;
+    w = (w * ka.gw) * ka.fw;
+    if (drift) w = w + ka.dw;   // only with drift: the identity model adds nothing, not even -0.0 + 0.0
+  }
+  setAngularVelocity(s, b, w);
+}
+
 // every kilobot senses the light and runs its controller, which sets its velocity (an absent kilobot neither senses nor
-// runs a controller: KB_BODY_ABSENT needs no light and takes the default case)
-template <class T>
-__device__ __forceinline__ void senseControl(T& s, int first, int stride) {
+// runs a controller: KB_BODY_ABSENT needs no light and takes the default case).  ACT: through the actuation model of
+// env envIn at sub-step `substep` (a, envIn and substep are not read without it).
+template <bool ACT = false, class T>
+__device__ __forceinline__ void senseControl(T& s, int first, int stride, const KernelArgs& a, int envIn, int substep) {
   const auto& L = s.L;
   const SF64Arr ls = s.lightState();
 #pragma unroll 1
@@ -164,6 +214,10 @@ __device__ __forceinline__ void senseControl(T& s, int first, int stride) {
     const int kind = s.bkind(b);
     const Xf xf = s.bodyXf(b);
     double* c = s.ctrl(k);
+    KilobotActuation ka;
+    if constexpr (ACT) {
+      if (kind >= KB_KILOBOT_PHOTOTAXIS && kind <= KB_KILOBOT_ACCELERATION) ka = kilobotActuation(a, envIn, k, substep);
+    }
     double value = 0.0, gx = 0.0, gy = 0.0;
     // the light is only looked at where its value can reach the controller: a PhototaxisKilobot samples
     // on every 6th call (lib/kilobot.py:328-333), velocity / acceleration control never
@@ -226,8 +280,8 @@ __device__ __forceinline__ void senseControl(T& s, int first, int stride) {
         V2 lv = mk(wv.x / 25.0f, wv.y / 25.0f);
         lv = mk(lv.x / L.dt, lv.y / L.dt);
         lv = mk(lv.x * 25.0f, lv.y * 25.0f);
-        setAngularVelocity(s, b, w);
-        setLinearVelocity(s, b, lv);
+        driveAngular<ACT>(s, b, w, ka, a.actDrift);
+        driveLinear<ACT>(s, b, lv, ka);
       } break;
       case KB_KILOBOT_SIMPLE_PHOTOTAXIS: {
         double mx = gx, my = gy;
@@ -238,7 +292,7 @@ __device__ __forceinline__ void senseControl(T& s, int first, int stride) {
         }
         mx *= 25.0;
         my *= 25.0;
-        setLinearVelocity(s, b, mk((float)mx, (float)my));
+        driveLinear<ACT>(s, b, mk((float)mx, (float)my), ka);
         // linearDamping = 0: kept as a per-kind constant of the solver's damping
       } break;
       case KB_KILOBOT_ACCELERATION: {
@@ -257,8 +311,8 @@ __device__ __forceinline__ void senseControl(T& s, int first, int stride) {
         double lx = sc.y, ly = sc.x;
         lx *= c[0] * 25.0;
         ly *= c[0] * 25.0;
-        setLinearVelocity(s, b, mk((float)lx, (float)ly));
-        setAngularVelocity(s, b, (float)c[1]);
+        driveLinear<ACT>(s, b, mk((float)lx, (float)ly), ka);
+        driveAngular<ACT>(s, b, (float)c[1], ka, a.actDrift);
       } break;
       default: break;
     }

@@ -33,6 +33,8 @@ namespace kb {
 #define KS_SWARM 5
 #define KS_SHUFFLE 6
 #define KS_CONFIG 8
+#define KS_ACTUATION 9         // per-episode actuation draws (kb_env.cuh)
+#define KS_ACTUATION_NOISE 10  // per-sub-step actuation noise (kb_env.cuh)
 
 struct SamplerConst {
   uint32_t seedLo, seedHi;

@@ -75,6 +75,15 @@ struct KernelArgs {
   const int32_t* sceneConfig;   // [S], -1 = no configuration
   const double* configCdf;
   int32_t numConfigs;
+  // actuation model (kb_set_actuation, kb_env.cuh): read only by the step kernels compiled with it switched on.
+  // actDraws [E][N] = (g_v, g_w, d_w, alive) of the env's current episode; actStep: the handle's kb_step count.
+  const float4* actDraws;
+  double actNoiseV, actNoiseW;
+  int64_t actEnvIdBase;
+  uint32_t actSeedLo, actSeedHi;
+  uint32_t actStep;
+  int32_t actNoise;   // noise_v > 0 || noise_w > 0: draw the per-sub-step factors
+  int32_t actDrift;   // drift_w > 0: add d_w to the turn rate
 };
 
 }  // namespace kb

@@ -39,8 +39,9 @@ namespace kb {
 // The batch is padded to a whole number of blocks (numEnvs <= grid * EPB): every lane of the step kernel owns
 // a real environment, so the groups of a warp can run in lock step.  Padding envs replicate the inputs of the
 // last real env and never write outputs.  Everything the layout covers is read through s.L, so that a compile-time
-// layout turns offsets, counts and constants into immediates.
-template <int LPE, class LT>
+// layout turns offsets, counts and constants into immediates.  ACT: the controllers drive through the actuation model
+// (kb_env.cuh); the kernels without it are compiled from exactly the code they had before the model existed.
+template <int LPE, class LT, bool ACT = false>
 __device__ __forceinline__ void stepKernelBody(const KernelArgs& a, const LT& layout) {
   constexpr int EPB = KB_BLOCK_OF(LPE) / LPE;
   const int slot = threadIdx.x / LPE;
@@ -78,7 +79,7 @@ __device__ __forceinline__ void stepKernelBody(const KernelArgs& a, const LT& la
       if (s.g.lane == 0) lightStep(s, act);
       s.g.usync();
     }
-    senseControl(s, s.g.lane, LPE);
+    senseControl<ACT>(s, s.g.lane, LPE, a, envIn, step);
     s.g.usync();
     s.g.usync();
     s.worldStep();

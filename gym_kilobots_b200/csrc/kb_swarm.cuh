@@ -1629,8 +1629,9 @@ __device__ __forceinline__ void swarmBind(Swarm<NT>& s, const KernelArgs& a, int
   s.nP = __ldg(&a.scenes[scene].numProxies);
 }
 
-template <int NT>
-__global__ void __launch_bounds__(NT, NT >= 512 ? 1 : (NT >= 256 ? 2 : 4)) kb_swarm_step_kernel(const __grid_constant__ KernelArgs a) {
+// the step of one env per CTA.  ACT: the controllers drive through the actuation model (kb_env.cuh)
+template <int NT, bool ACT>
+__device__ __forceinline__ void swarmStepBody(const KernelArgs& a) {
   const int env = a.envOffset + blockIdx.x;
   Swarm<NT> s(a.L, a.W);
   const int scene = swarmSceneOf(a, env);
@@ -1649,7 +1650,7 @@ __global__ void __launch_bounds__(NT, NT >= 512 ? 1 : (NT >= 256 ? 2 : 4)) kb_sw
       if (s.tid == 0) lightStep(s, act);
       __syncthreads();
     }
-    senseControl(s, s.tid, NT);
+    senseControl<ACT>(s, s.tid, NT, a, env, step);
     __syncthreads();
     s.worldStep();
   }
@@ -1660,6 +1661,15 @@ __global__ void __launch_bounds__(NT, NT >= 512 ? 1 : (NT >= 256 ? 2 : 4)) kb_sw
   if (a.prof && s.tid == 0)
     for (int i = 0; i < KB_PROF_SLOTS; ++i) a.prof[(size_t)env * KB_PROF_SLOTS + i] = (unsigned long long)s.tp[i];
 #endif
+}
+
+template <int NT>
+__global__ void __launch_bounds__(NT, NT >= 512 ? 1 : (NT >= 256 ? 2 : 4)) kb_swarm_step_kernel(const __grid_constant__ KernelArgs a) {
+  swarmStepBody<NT, false>(a);
+}
+template <int NT>
+__global__ void __launch_bounds__(NT, NT >= 512 ? 1 : (NT >= 256 ? 2 : 4)) kb_swarm_step_kernel_act(const __grid_constant__ KernelArgs a) {
+  swarmStepBody<NT, true>(a);
 }
 
 template <int NT>

@@ -8,6 +8,8 @@ The envs of one batch may differ in their numbers of objects and kilobots: N and
 `kilobot_mask` / `object_mask` say which rows an env populates, and the rows it does not are NaN.
 With `local_observation=scene.LocalObsSpec(...)` the observation also holds obs['local'] [E, N, D]: what each kilobot
 senses in its own frame (neighbours, objects, light), computed on the device after every step and reset.
+With `actuation=scene.ActuationSpec(...)` the kilobots' motors differ per robot and episode (gains, drift, failures) and
+are noisy per sub-step, drawn on the device.
 """
 import numpy as np
 
@@ -23,11 +25,12 @@ class KilobotsVecEnv:
     """
 
     def __init__(self, scenario, device=0, action_mode=abi.KB_ACTION_LIGHT, task=None, targets=None,
-                 flat_observation=False, allow_status_flags=False, local_observation=None):
+                 flat_observation=False, allow_status_flags=False, local_observation=None, actuation=None):
         """task / targets: optional `scene.TaskSpec` and per-env target poses [E,3] -- on-device reward, done and
         episode statistics (an extension: the reference's hooks are abstract and its in-tree envs return constants).
         flat_observation: also emit obs['flat'], the vector YamlKilobotsEnv.observation_space describes.
-        local_observation: a `scene.LocalObsSpec`; also emit obs['local'], each kilobot's local observation."""
+        local_observation: a `scene.LocalObsSpec`; also emit obs['local'], each kilobot's local observation.
+        actuation: a `scene.ActuationSpec`; the kilobots drive through that actuation model (`set_actuation`)."""
         self.scenario = scenario
         # KB_STATUS_* bits (contact / solver capacity overflow, non-finite pose) raise KbStatusError in step() and
         # check_status() unless explicitly allowed: a dropped pair is silently different physics
@@ -48,6 +51,8 @@ class KilobotsVecEnv:
         self._init_masks()
         if task is not None:
             self.set_task(task, targets)
+        if actuation is not None:
+            self.set_actuation(actuation)
 
     def _init_masks(self):
         """kilobot_mask [E,N] / object_mask [E,M]: bool CUDA tensors, True where the env's current scene has that
@@ -140,6 +145,17 @@ class KilobotsVecEnv:
     # -- task layer (extension) -----------------------------------------------------------------
     def set_task(self, task, targets=None):
         self.batch.set_task(task, targets)
+
+    # -- actuation model (extension) --------------------------------------------------------------
+    def set_actuation(self, spec):
+        """Attach a `scene.ActuationSpec` (None detaches it).  Draws episode 0 of every env now; every reset then draws the
+        reset envs' next episode on the device."""
+        self.batch.set_actuation(spec)
+
+    def actuation_draws(self):
+        """float32 [E, N, 4] host array: every kilobot slot's (speed gain, turn-rate gain, turn-rate drift rad/s, alive)
+        in the env's current episode -- for logging or a privileged critic."""
+        return self.batch.actuation()[0]
 
     def episode_stats(self):
         """dict of [E] float64 arrays: return, length, position_error, orientation_error, success, done_count."""

@@ -139,6 +139,32 @@ class LocalObsSpec:
         return d
 
 
+@dataclass(frozen=True)
+class ActuationSpec:
+    """Actuation model (include/kb_b200.h kb_set_actuation): kilobots whose motors differ, drift and fail.  Per episode and
+    kilobot: a gain on the linear speed in [gain_v_lo, gain_v_hi], a gain on the turn rate in [gain_w_lo, gain_w_hi], an
+    additive turn rate in [-drift_w, drift_w] rad/s, and with probability p_dead motors that stay off; per sub-step the
+    speed and turn rate are scaled by 1 + noise_v * xi and 1 + noise_w * xi, xi uniform in [-1, 1).  The defaults are the
+    identity: exactly the physics without a model.  env_id_base: global id of the batch's env 0 (rank * envs per rank)."""
+    seed: int = 0
+    env_id_base: int = 0
+    gain_v_lo: float = 1.0
+    gain_v_hi: float = 1.0
+    gain_w_lo: float = 1.0
+    gain_w_hi: float = 1.0
+    drift_w: float = 0.0
+    noise_v: float = 0.0
+    noise_w: float = 0.0
+    p_dead: float = 0.0
+
+    def to_def(self):
+        d = abi.KbActuationDef()
+        d.seed, d.env_id_base = int(self.seed) & 0xFFFFFFFFFFFFFFFF, int(self.env_id_base)
+        for name in ("gain_v_lo", "gain_v_hi", "gain_w_lo", "gain_w_hi", "drift_w", "noise_v", "noise_w", "p_dead"):
+            setattr(d, name, float(getattr(self, name)))
+        return d
+
+
 @dataclass
 class SceneSpec:
     bodies: List[BodySpec] = field(default_factory=list)   # objects first, then kilobots

@@ -326,6 +326,8 @@ typedef struct KbLaunchConfig {
   int32_t specialised;
   float jit_ms;                  /* its compile time in kb_create, ms (0: taken from a cache) */
   char jit_reason[256];          /* why the generic kernel runs ("" when specialised) */
+  int32_t actuation;             /* 1: the step kernel drives the controllers through the actuation model (kb_set_actuation):
+                                    specialised / jit_ms / jit_reason then describe that variant */
 } KbLaunchConfig;
 int kb_get_launch_config(const KbHandle* h, KbLaunchConfig* cfg);
 /* Needs no GPU: the source kb_create generates for the specialised step kernel of a lane-group batch of `scenes`
@@ -417,6 +419,46 @@ int kb_local_observation_dim(const KbHandle* h, const KbLocalObsDef* def);
 /* out: device f32[E, Nmax, D]; mask: device u8[E] or NULL = every env (rows of unmasked envs are not written).
    Asynchronous on `stream`: no allocation, no host synchronisation. */
 int kb_local_observation(KbHandle* h, const KbLocalObsDef* def, const uint8_t* mask, float* out, void* stream);
+
+/*
+ * Actuation model -- an EXTENSION beyond the reference: kilobots whose motors differ from robot to robot and from moment
+ * to moment, the way real kilobots do (hand-calibrated vibration motors; some fail), so that policies trained here do not
+ * rely on identical, noiseless robots.  NULL detaches the model.  Per episode, per padded kilobot slot k (present or not,
+ * so that presence does not change a draw), float32 in a device array [E, Nmax, 4]:
+ *   g_v = (float)(gain_v_lo + (gain_v_hi - gain_v_lo) * u0)   gain on the linear speed
+ *   g_w = (float)(gain_w_lo + (gain_w_hi - gain_w_lo) * u1)   gain on the turn rate
+ *   d_w = (float)(drift_w * (2 * u2 - 1))                      additive turn rate, rad/s
+ *   alive = u3 < p_dead ? 0 : 1                                 a dead kilobot's motors are off for the whole episode
+ * u0, u1 / u2, u3: the two 53-bit uniforms of the Philox4x32-10 blocks with draw index 2k / 2k + 1 of stream 9, keyed like
+ * kb_set_sampler's draws by (seed, global env id = env_id_base + env, the env's actuation episode).  kb_set_actuation draws
+ * episode 0 of every env; every kb_reset / kb_reset_sampled then advances the reset envs' episode and redraws their rows.
+ * With noise_v or noise_w > 0, every sub-step draws xi_v, xi_w = 2 u - 1 in [-1, 1) per kilobot from the Philox block
+ * with counter (k | sub-step << 16, step, global env id low word, 10 | high word << 8), where step counts the kb_step /
+ * kb_step_host calls since kb_set_actuation (modulo 2^32; kb_step_host's chunks share it).  Where a controller sets a
+ * velocity v (b2 units) or turn rate w, float32 in this order:
+ *   v' = (v * g_v) * f_v,  f_v = (float)(1 + noise_v * xi_v)
+ *   w' = (w * g_w) * f_w,  f_w = (float)(1 + noise_w * xi_w),  then w' + d_w only when drift_w > 0
+ * A dead kilobot's controller runs and keeps its state, but sets no velocity: the body is passive and can be pushed.
+ * SimplePhototaxisKilobot sets no turn rate, so it gets no angular transform; KB_ACTION_KILOBOTS is transformed too.
+ * Gains [1, 1], no noise, no drift and p_dead = 0 give exactly the physics without a model.
+ * KB_ERR_INVALID (message naming the field): a non-finite or negative value, lo > hi, p_dead > 1.
+ * The model's draws and counters are not part of kb_get_state / kb_set_state: restoring a checkpoint does not restore
+ * the actuation stream.  gym_kilobots_b200/actuation.py evaluates the same draws in numpy.  oracle/libkbo.so, the
+ * reference's restatement, has no kbo_set_actuation: the tests build the oracle with the model from tests/kbo_actuation.cpp.
+ */
+typedef struct KbActuationDef {
+  uint64_t seed;
+  int64_t env_id_base;             /* global id of this handle's env 0 (rank * envs per rank) */
+  double gain_v_lo, gain_v_hi;
+  double gain_w_lo, gain_w_hi;
+  double drift_w;                  /* rad/s */
+  double noise_v, noise_w;         /* relative amplitudes per sub-step */
+  double p_dead;
+} KbActuationDef;
+int kb_set_actuation(KbHandle* h, const KbActuationDef* def);
+/* host f32[E, Nmax, 4] (g_v, g_w, d_w, alive), u32[E] actuation episodes, the step count (any may be NULL); synchronises.
+   KB_ERR_INVALID without a model. */
+int kb_get_actuation(KbHandle* h, float* draws, uint32_t* episodes, uint64_t* step);
 
 /* Off-screen rasteriser (SURVEY.md 8(f) n4): the picture KilobotsEnv.render draws through
  * kb_rendering.KilobotsViewer (kilobots_env.py:221-275) -- table, objects, kilobots, light -- for num_images
